@@ -2,6 +2,7 @@
 """Benchmark of the Locator training hot path (BASELINE.json metric: train samples/s per model).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg3|fixture]
+                    [--dump-outputs DIR]
 
 A "step" is one optimizer step of one model (batch 32) on BASELINE config[1]: 1,000 samples x
 100,000 SNPs (810 train / 90 validation rows), nlayers=10, width=256.  The timed region runs exactly
@@ -11,7 +12,10 @@ of an epoch, that epoch's validation pass, callbacks and checkpoint are inside t
 in the reference's model.fit) on data already resident in HBM.  N > 1: every rank trains its own
 model on its own GPU (replicates are independent; no collective on the training path) -> weak scaling.
 
-Printed JSON line: see the task contract.  Extra objects:
+--dump-outputs DIR: after the timed steps, rank 0 writes what they left in its model as float32 DIR/<name>.npy (see
+dump_outputs).  The inputs depend only on the arguments (fixed seeds), so two builds can be compared output for output.
+
+Printed JSON line (rank 0): the metric (`value`, samples/s), the run's settings and clocks, and extra objects:
   e2e          the public API end to end: LocatorModel(...) creation + init + fit() for >= 20 epochs on
                PAGEABLE host numpy matrices (H2D, 2-bit pack, epochs incl. validation, history D2H)
   roofline     the first-layer backward + Adam kernel (24*K*H bytes per launch) timed alone, CUDA events
@@ -168,6 +172,30 @@ def workload_string(workload):
             f"nlayers {L}, width {H}")
 
 
+W1_SAMPLE_ROWS = 16384  # W1 is K x 256 float32 (100 MB at cfg2): a fixed sample of its SNP rows is dumped
+
+
+def dump_outputs(m, out_dir):
+    """What a caller of the timed loc_train_steps calls receives from the model after the last step, as float32
+    .npy files: every weight array in Keras order and the last step's loss.  Every array's shape depends on the
+    workload only (the per-epoch history is left out: it is empty when the run ends inside its first epoch).  W1 is
+    cut to W1_SAMPLE_ROWS rows drawn with default_rng(0), so that the whole dump stays below 64 MB at every workload."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"last_loss": np.array([m.state().last_loss], np.float32)}
+    for i, w in enumerate(m.get_weights()):
+        if i < 4:
+            name = ("bn_gamma", "bn_beta", "bn_moving_mean", "bn_moving_var")[i]
+        else:
+            d, isb = divmod(i - 4, 2)
+            name = f"dense{d + 1:02d}_{'bias' if isb else 'kernel'}"
+        if i == 4:
+            rows = np.sort(np.random.default_rng(0).choice(m.K, min(m.K, W1_SAMPLE_ROWS), replace=False))
+            w, name = w[rows], name + "_sampled_rows"
+        out[f"w{i:02d}_{name}"] = w
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def run_reference(args, workload):
     """--impl reference: the reference's algorithm on the host CPU (oracle port; TF/Keras cannot be
     installed on this image -- no wheel, no network), all host threads, bounded sample."""
@@ -307,7 +335,12 @@ def main():
     ap.add_argument("--no-large-batch", action="store_true", help="skip the --batch_size 64 / 256 side measurement")
     ap.add_argument("--e2e-epochs", type=int, default=20)
     ap.add_argument("--group", type=int, default=4, help="replicates per GPU for the group / work-queue measurements (0/1 = skip the group leg)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed model's outputs after its last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the CUDA model of --impl b200")
     workload = args.workload
     if args.impl == "reference":
         run_reference(args, workload)
@@ -387,6 +420,8 @@ def main():
     assert st.t == warm + steps, (st.t, warm, steps)
     assert st.nonfinite == 0 and np.isfinite(st.last_loss), "non-finite loss during the timed region"
     value = aggregate_value(world, steps, B, ms)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(m, args.dump_outputs)  # before the roofline launches below change the model
 
     # ---- roofline: first-layer backward + Adam alone, CUDA events on the launching stream ----
     rows_dev = torch.as_tensor(rng.permutation(ntr)[:B].astype(np.int32)).cuda()

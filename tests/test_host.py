@@ -29,7 +29,11 @@ def test_cabi_exports_every_declared_symbol():
         assert hasattr(_cabi.lib, name)
     assert _cabi.lib.loc_abi_version() == 1
     assert _cabi.lib.loc_l1_impl() in (b"tcgen05", b"simt")
-    assert _cabi.lib.loc_launch_count() == 0  # nothing has been launched: no compute without a GPU
+    # loading the library launches nothing; counted in a fresh process, since the counter is per process and GPU
+    # tests that ran before this one in the same session have launched kernels
+    r = subprocess.run([sys.executable, "-c", "from locator_b200 import _cabi; print(_cabi.lib.loc_launch_count())"],
+                       cwd=ROOT, capture_output=True, text=True, check=True)
+    assert int(r.stdout) == 0
 
 
 def test_product_package_never_imports_the_oracle():
