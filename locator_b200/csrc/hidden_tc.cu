@@ -137,13 +137,13 @@ __device__ __forceinline__ void hidden_tc_body(const HidArgs& a) {
                  "l"(src), "r"((uint32_t)kSlot), "r"(smem_u32(&wbar[u & 1]))
                  : "memory");
   };
-  // Launched with programmatic stream serialization behind this model's small-layer update (train_step's chain):
-  // its results -- the weight-slice images and biases read below -- are complete after this wait.  A no-op for
-  // plain launches.
-  // (A chained single-model step names both producers explicitly -- wait_upd for the update, wait_bwd for the backward's
-  // tiles, each published behind a fence -- and skips the grid-level wait: that one also covers the backward's
-  // completion as a GRID, several microseconds after its last CTA has signed off.  LOC_GDC_WAIT=1 restores it.)
-  if (!(a.wait_bwd != 0 && a.wait_upd != 0 && a.skip_grid_wait)) asm volatile("griddepcontrol.wait;" ::: "memory");
+  // Launched with programmatic stream serialization (train_step's chain, the replicate rings): the results of the
+  // kernels in front of it in the stream are complete after this wait.  A no-op for plain launches.
+  // It is left out when both producers are named by flags -- wait_upd for the small-layer update (the weight-slice
+  // images and biases read below), wait_bwd for the backward's Z1 tiles, each published behind a fence -- as in a
+  // chained single-model step: the grid-level wait also covers the backward's completion as a GRID, several
+  // microseconds after its last CTA has signed off.
+  if (!(a.wait_bwd != 0 && a.wait_upd != 0)) asm volatile("griddepcontrol.wait;" ::: "memory");
   __shared__ int s_dz_done;  // lowest layer whose dz this CTA has written completely (backward chain)
   if (a.wait_upd != 0) {  // the small-layer update of the previous step ran under that step's hidden stack
     if (tid == 0) wait_counter(&a.st->upd_cnt, a.wait_upd, &a.st->chain_timeout, 20u);

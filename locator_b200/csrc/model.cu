@@ -221,8 +221,6 @@ static unsigned long long* timeline_buffer() {
   return g_tl;
 }
 
-static int g_fuse_debug = 0;  // loc_debug_stage: LOC_FUSE_DEBUG bits (timing experiments only)
-
 static L1Args l1_args(loc_model* m, const uint32_t* packed, int64_t row_words, const RowSrc& src, int training,
                       int gated) {
   L1Args a;
@@ -235,13 +233,6 @@ static L1Args l1_args(loc_model* m, const uint32_t* packed, int64_t row_words, c
   a.src = src;
   a.src_next = src;
   a.fuse_next = 0;
-  static const int alternate = getenv("LOC_NO_ALTERNATE") ? 0 : 1;
-  a.alternate = alternate;
-  // the chunks stream through L2 once per step: evict_first on both directions measured 7% faster
-  // (B200, cfg2) than the default policy; LOC_STREAM_HINT overrides for A/B runs
-  static const int stream_hint = getenv("LOC_STREAM_HINT") ? atoi(getenv("LOC_STREAM_HINT")) : 3;
-  a.stream_hint = stream_hint;
-  a.dbg_flags = g_fuse_debug;
   a.rev = (int)(m->h_steps & 1);  // steps launched so far (training hidden stacks): odd steps walk downwards
   a.wait_hid = 0u;
   a.wait_bwd = 0u;
@@ -308,7 +299,6 @@ static HidArgs hid_args(loc_model* m, const RowSrc& src, int training, int gated
   h.partial_stride = (int64_t)kMaxB * m->H;
   h.partial_row0 = 0;
   h.val_slot = nullptr;
-  h.skip_grid_wait = 0;
   h.loss_rows = 0;
   h.row_base = 0;
   h.mask_rows = 0;
@@ -503,8 +493,8 @@ static int train_step_big(loc_model* m, const RowSrc& src, int gated, cudaStream
 // first-layer forward on the W1 chunks it has just updated (they are still in shared memory), so the
 // following step is called with have_fwd = true and skips its own forward launch.
 //
-// Chained steps (chain_capable): the step's kernels go into ONE stream as  H -> B -> U  (hidden stack on its
-// 16-SM cluster, first-layer backward + Adam (+ next forward), small-layer update), every one of them launched
+// Chained steps (chain_capable): the step's kernels go into ONE stream as  H -> U -> B  (hidden stack on its
+// 16-SM cluster, small-layer update, first-layer backward + Adam (+ next forward)), every one of them launched
 // with programmatic stream serialization, i.e. scheduled as soon as its predecessor's CTAs are all running instead
 // of after it has drained, and handing over through two device flags instead of kernel boundaries:
 //   B's CTAs take the 132 SMs H does not use while H still runs: barriers, TMEM and the first ring stages of
@@ -512,10 +502,10 @@ static int train_step_big(loc_model* m, const RowSrc& src, int gated, cudaStream
 //     touches dZ1.  Its last 16 CTAs get H's SMs when H exits; they hold the smaller tile shares (tile_range in
 //     l1_tc.cu), so they still finish with the others.  (With fewer first-layer CTAs than SMs --
 //     loc_model_set_l1_ctas, replicate rings -- all of B is resident early.)
-//   U is placed wherever SMs free up (H's SMs at once when B leaves them alone, else B's first finishers) and
-//     waits for the same flag;
-//   the NEXT step's H is queued behind U -- griddepcontrol.wait covers U's results -- and waits for
-//     DevState::bwd_cnt (one count per finished CTA of B) before it reads the Z1 tiles B's fused forward left.
+//   U's blocks take SMs H leaves idle and wait for the same flag (per layer: DevState::dz_cnt, below);
+//   the NEXT step's H is queued behind B and waits for DevState::upd_cnt (every finished block of U) and
+//     DevState::bwd_cnt (one count per finished CTA of B) before it reads the small weights and the Z1 tiles B's
+//     fused forward left -- not for B's completion as a grid (griddepcontrol.wait), which comes microseconds later.
 // Kernel boundaries (drain + launch + ramp: 6-15 us each on this part, `scripts/timeline.py`) disappear from the
 // step's critical path; what remains is H + B plus the flags' latency.
 static int train_step(loc_model* m, const RowSrc& src, int gated, cudaStream_t s, int stage_mask = 15,
@@ -538,27 +528,21 @@ static int train_step(loc_model* m, const RowSrc& src, int gated, cudaStream_t s
     begin_training_hidden(m, h);
     if (h_overlaps) h.wait_bwd = m->h_bwd_cnt;  // every CTA of the previous step's backward has signed off
     if (chain) h.wait_upd = m->h_upd_cnt;       // ... and every block of the small-layer updates so far
-    h.skip_grid_wait = h_overlaps && getenv("LOC_GDC_WAIT") == nullptr;
     if (m->hid_tc ? hidden_tc_launch(h, s, h_overlaps) : hidden_launch(h, m->cluster, s)) return 1;
   }
   if (chain) {
     // U goes in FRONT of B: its blocks land on the SMs that idle under the hidden stack and update layer i as soon
     // as the stack's backward chain has produced dz_i (DevState::dz_cnt), so the update is finished a couple of
     // microseconds after H instead of occupying the SMs between B's end and the next H.  B's CTAs take the SMs the
-    // update's blocks leave (LOC_CHAIN_ORDER=hbu: the update behind the backward, as in the replicate rings).
-    const char* order = getenv("LOC_CHAIN_ORDER");
-    const bool u_first = order == nullptr || strcmp(order, "hbu") != 0;
+    // update's blocks leave.
     UpdArgs u = upd_args(m, src.nb, gated);
     u.wait_hid = h.hid_seq;
-    if (u_first) {
-      u.wait_dz = 16u * h.hid_seq;  // 16 CTAs of every training hidden stack so far
-      u.wait_upd = m->h_upd_cnt;    // every block of the updates launched so far
-      if (update_launch(m, u, s, true)) return 1;
-    }
+    u.wait_dz = 16u * h.hid_seq;  // 16 CTAs of every training hidden stack so far
+    u.wait_upd = m->h_upd_cnt;    // every block of the updates launched so far
+    if (update_launch(m, u, s, true)) return 1;
     a.wait_hid = h.hid_seq;
     a.wait_bwd = m->h_bwd_cnt;  // every backward launched so far for this model
     if (backward_tc(m, a, s, true)) return 1;
-    if (!u_first && update_launch(m, u, s, true)) return 1;
     m->chain_open = 1;
     m->chain_stream = s;
     return 0;
@@ -1157,7 +1141,7 @@ int loc_train_step(loc_model* m, const int32_t* d_rows, int32_t nb, void* stream
 
 int loc_debug_stage(loc_model* m, int32_t stage, const int32_t* d_rows, int32_t nb, void* stream) {
   LOC_CHECK(m != nullptr && m->train_packed != nullptr, "loc_debug_stage: no training data bound");
-  LOC_CHECK(stage >= 0 && stage < 6 && d_rows != nullptr && nb >= 1 && nb <= m->B, "loc_debug_stage: bad arguments");
+  LOC_CHECK(stage >= 0 && stage < 5 && d_rows != nullptr && nb >= 1 && nb <= m->B, "loc_debug_stage: bad arguments");
   LOC_CHECK(m->B <= kMaxB, "loc_debug_stage: single stages are only available for batch_size <= 32");
   m->span_perm = nullptr;
   RowSrc src;
@@ -1166,20 +1150,7 @@ int loc_debug_stage(loc_model* m, int32_t stage, const int32_t* d_rows, int32_t 
   src.offset = 0;
   src.row0 = 0;
   src.nb = nb;
-  if (stage == 4) {  // backward + fused next forward
-    const char* e = getenv("LOC_FUSE_DEBUG");
-    g_fuse_debug = e != nullptr ? atoi(e) : 0;
-    const int rc = train_step(m, src, 0, (cudaStream_t)stream, 4, &src);
-    g_fuse_debug = 0;
-    return rc;
-  }
-  if (stage == 5) {  // L2 prefetch of the next backward's head: LOC_PREFETCH="skip,count" chunks per CTA
-    LOC_CHECK(m->use_tc, "loc_debug_stage: stage 5 needs the tcgen05 first layer");
-    int skip = 0, cnt = 16;
-    if (const char* e = getenv("LOC_PREFETCH")) sscanf(e, "%d,%d", &skip, &cnt);
-    L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 0);
-    return l1_prefetch_tc(a, m->n_bwd_blocks, skip, cnt, 0, (cudaStream_t)stream);
-  }
+  if (stage == 4) return train_step(m, src, 0, (cudaStream_t)stream, 4, &src);  // backward + fused next forward
   return train_step(m, src, 0, (cudaStream_t)stream, 1 << stage);
 }
 
@@ -1385,7 +1356,7 @@ int64_t loc_debug_read(loc_model* m, int32_t which, float* h_dst, int64_t max_n,
 // after the span are.
 static int run_span(loc_model* m, const int32_t* perm, int64_t epoch_stride, int64_t step0, int64_t nsteps, int gated,
                     bool* have_fwd, cudaStream_t s) {
-  const bool fuse = m->use_tc && m->B <= kMaxB && getenv("LOC_NO_FUSE") == nullptr;
+  const bool fuse = m->use_tc && m->B <= kMaxB;
   auto step_rows = [&](int64_t off) {
     RowSrc src;
     src.rows = perm;

@@ -65,16 +65,14 @@ struct L1Args {
   RowSrc src;
   RowSrc src_next;  // rows of the following step (fused forward of the tcgen05 backward kernel)
   int fuse_next;
-  int alternate;  // tcgen05 backward: walk the CTA's tiles downwards on odd steps (the tail of the previous
-                  // step's updates is still in L2: those reads hit and their dirty lines are overwritten in place)
-  int stream_hint;  // tcgen05 backward: L2 evict_first on the W1/m/v chunk loads (bit 0) / stores (bit 1)
-  int rev;          // tcgen05 backward: walk the tiles downwards (host-side step parity; see `alternate`)
+  int rev;  // tcgen05 backward: walk the CTA's tiles downwards -- odd steps (host-side step parity), so that a walk starts
+            // on the tail of the previous step's updates, still in L2: those reads hit and their dirty lines are
+            // overwritten in place
   unsigned wait_hid;  // != 0: launched ahead of this step's hidden stack -- wait for DevState::hid_seq >= wait_hid before dZ1 is read
   unsigned wait_bwd;  // with wait_hid: the previous backward of this model may still be running on other SMs when this
                       // CTA starts -- no chunk is loaded before DevState::bwd_cnt >= wait_bwd (all its CTAs are done)
   unsigned long long* tl;  // kernel timeline buffer (diagnostics) or nullptr
   int tl_id;
-  int dbg_flags;    // timing experiments on the fused forward (loc_debug_stage + LOC_FUSE_DEBUG); 0 in production
   float *gamma, *beta, *mmean, *mvar;
   float* W1;
   float *m_gamma, *v_gamma, *m_beta, *v_beta, *mW1, *vW1;
@@ -119,7 +117,6 @@ struct HidArgs {
   unsigned hid_seq;   // training launches: value to publish in DevState::hid_seq when everything is written
   unsigned wait_upd;  // != 0: wait for DevState::upd_cnt >= wait_upd before the small weights are read (the update ran
                       // under the previous hidden stack, not directly in front of this launch)
-  int skip_grid_wait;  // chained step: wait_bwd and wait_upd cover every producer, griddepcontrol.wait is left out
   unsigned long long* tl;  // kernel timeline buffer (diagnostics) or nullptr
   int tl_id;
   // Batches of more than 32 rows (bigbatch.cu): the step's rows go through the stack in 32-row chunks, one launch each.
@@ -179,9 +176,6 @@ int l1_backward_tc(const L1Args& a, int nblocks, cudaStream_t s, bool overlap_pr
 int l1_tc_partials(int64_t K);
 // inference forward of up to 256 rows in one pass over W1: out [n_partials][32 * ceil(nrows / 32)][256]
 int l1_forward_wide_tc(const L1Args& a, int n_partials, int nrows, float* out, cudaStream_t s);
-// L2 prefetch of the head of the next backward's walk (chunks [skip, skip + n) of every CTA; t_ahead: optimizer
-// steps between now and that backward -- decides the walk direction)
-int l1_prefetch_tc(const L1Args& a, int nblocks, int skip_chunks, int n_chunks, int t_ahead, cudaStream_t s);
 
 }  // namespace loc
 
