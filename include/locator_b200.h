@@ -70,7 +70,8 @@ typedef struct loc_state {
 
 int loc_abi_version(void);
 const char* loc_last_error(void);
-/* Name of the first-layer kernel family in use ("simt" or "tcgen05"). */
+/* Name of the first-layer kernel family a width-256 model runs on the sm_100a device the library is
+ * built for: "tcgen05".  loc_model_impl gives the family a particular model uses. */
 const char* loc_l1_impl(void);
 
 /* ---------------- genotype ingest (K1/K2) ---------------- */

@@ -661,10 +661,7 @@ static int w1_download(loc_model* m, const float* d_tiled, float* h_dst, cudaStr
 
 extern "C" {
 
-const char* loc_l1_impl(void) {
-  const char* e = getenv("LOC_L1_IMPL");
-  return (e != nullptr && strcmp(e, "simt") == 0) ? "simt" : "tcgen05";
-}
+const char* loc_l1_impl(void) { return "tcgen05"; }
 
 }  // extern "C"
 
@@ -795,13 +792,8 @@ int loc_model_create(loc_model** out, int64_t K, int32_t width, int32_t nlayers,
   LOC_CHECK(ndev > 0, "loc_model_create: no CUDA device (this library has no CPU fallback)");
   int dev = 0;
   LOC_CUDA(cudaGetDevice(&dev));
-  int hid_tc, use_tc;
-  {
-    const char* himpl = getenv("LOC_HIDDEN_IMPL");
-    hid_tc = (himpl == nullptr || strcmp(himpl, "simt") != 0) && hidden_tc_supported(width, nlayers);
-    const char* impl = getenv("LOC_L1_IMPL");
-    use_tc = (impl == nullptr || strcmp(impl, "simt") != 0) && l1_tc_supported(K, width);
-  }
+  const int hid_tc = hidden_tc_supported(width, nlayers);
+  const int use_tc = l1_tc_supported(K, width);
   const bool want_dbg = getenv("LOC_HID_TRACE") != nullptr;
   if (loc_model* r = pool_limit() > 0 ? pool_take(dev, K, width, nlayers, use_tc, hid_tc, max_epochs, want_dbg, chunks) : nullptr) {
     // a recycled handle: same buffers, new shape and settings, nothing bound

@@ -1,8 +1,9 @@
 """GPU parity: the CUDA training / prediction path (through the C ABI) vs the CPU oracle.
 
-Tolerances.  The CUDA-core kernels (LOC_L1_IMPL=simt / LOC_HIDDEN_IMPL=simt, other widths) are
-plain fp32 (differences = summation order only); the tcgen05 first layer and hidden stack multiply
-in TF32 (10-bit mantissa, as TensorFlow does by default on Ampere+ GPUs), fp32 accumulate.
+Tolerances.  The CUDA-core kernels (widths other than 256, hidden stacks too deep for the
+tcgen05 kernel) are plain fp32 (differences = summation order only); the tcgen05 first layer
+and hidden stack multiply in TF32 (10-bit mantissa, as TensorFlow does by default on Ampere+
+GPUs), fp32 accumulate.
 Stated tolerances:
   forward / predict      |dy| <= 2e-3 * (1 + |y|)      (tf32) ; 2e-5 (fp32)
   per-step loss          rel 2e-3 (tf32) ; 1e-4 (fp32)
