@@ -172,7 +172,7 @@ int loc_np_legacy_permutation(uint32_t* mt_key, int32_t* mt_pos, int64_t n, int6
  * -> Dense(2) -> Dense(2); Adam(1e-3, .9, .999, 1e-7).  batch_size <= LOC_MAX_BATCH_SIZE
  * (locator.py:69,371; steps of more than LOC_MAX_BATCH rows: batch statistics over the whole step,
  * 32-row chunks through the hidden stack, one pass over W1 | m | v -- csrc/bigbatch.cu; such models
- * cannot be grouped or sharded), nlayers >= 2.  Allocates parameters, Adam state, best-weights snapshot and
+ * cannot be sharded), nlayers >= 2.  Allocates parameters, Adam state, best-weights snapshot and
  * workspaces on the current device. */
 int loc_model_create(loc_model** out, int64_t K, int32_t width, int32_t nlayers, int32_t batch_size,
                      float dropout_prop, int32_t max_epochs);
@@ -294,7 +294,11 @@ int loc_train_steps(loc_model* m, const int32_t* d_perm, int32_t step0, int32_t 
  *            previous model of its ring (programmatic dependent launch inside one stream);
  *   lockstep (otherwise): the hidden stacks of all models share one launch (one cluster per model), the
  *            first-layer kernels run back to back.
- * Environment LOC_GROUP_SCHEDULE=ring|lockstep overrides the choice by size. */
+ * Environment LOC_GROUP_SCHEDULE=ring|lockstep overrides the choice by size.
+ * Models of batch_size > 32 have a third schedule, whatever LOC_GROUP_SCHEDULE says: per step, the batch
+ * statistics of all models in one launch, each model's wide first-layer forward, the 32-row chunks of whole
+ * models packed into shared hidden-stack launches (floor(8 / chunks) models per launch), one step end for
+ * all models, then the first-layer backwards back to back while the small-layer updates run on side streams. */
 int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* const* d_perms, int32_t n_epochs,
                            void* stream);
 

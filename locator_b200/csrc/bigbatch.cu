@@ -37,7 +37,10 @@ __device__ __forceinline__ void bb_moments(int n1, int n2, int nb, float& mean, 
 
 // Genotype counts over the step's rows -> batch statistics.  256 threads = 32 packed words (16 SNPs each) x 8 row
 // slices; the slices' counts meet in shared memory (integer atomics: order-free), then one thread per SNP finishes.
-__global__ void __launch_bounds__(256) k_bb_stats(BigArgs a) {
+// blockIdx.y: model of a replicate group (the grid covers the largest K of the group).
+__global__ void __launch_bounds__(256) k_bb_stats(BigGroupArgs ga) {
+  const BigArgs& a = ga.a[blockIdx.y];
+  if ((int64_t)blockIdx.x * 32 * 16 >= a.K) return;
   if (a.gated && a.st->stopped) return;
   __shared__ int64_t s_rows[LOC_MAX_BATCH_SIZE];
   __shared__ unsigned cnt[32][2][16];
@@ -508,9 +511,12 @@ __global__ void __launch_bounds__(1024) k_bb_hidden_update(BigArgs a) {
   }
 }
 
-// End of a large step whose chunks ran through the hidden stack side by side (one grouped launch): per-chunk loss sums
-// added in chunk order (same bits as chunk-by-chunk launches), then the optimizer bookkeeping of the step.
-__global__ void k_bb_step_end(DevState* st, const float* slots, int nc, int loss_rows, int gated) {
+// End of a large step whose chunks ran through the hidden stack side by side (grouped launches): per-chunk loss sums
+// added in chunk order (same bits as chunk-by-chunk launches), then the optimizer bookkeeping of the step.  One block
+// per model of a replicate group.
+__global__ void k_bb_step_end(BigEndArgs e, int nc, int loss_rows, int gated) {
+  DevState* st = e.st[blockIdx.x];
+  const float* slots = e.slots[blockIdx.x];
   if (gated && st->stopped) return;
   float acc = 0.f;
   for (int c = 0; c < nc; ++c) {
@@ -530,8 +536,9 @@ __global__ void k_bb_step_end(DevState* st, const float* slots, int nc, int loss
   st->alpha = st->lr * sqrtf(1.f - b2p) / (1.f - b1p);
 }
 
-int bb_step_end_launch(DevState* st, const float* slots, int nc, int loss_rows, int gated, cudaStream_t s) {
-  k_bb_step_end<<<1, 1, 0, s>>>(st, slots, nc, loss_rows, gated);
+int bb_step_end_launch(const BigEndArgs& e, int nc, int loss_rows, int gated, cudaStream_t s) {
+  LOC_CHECK(e.n >= 1 && e.n <= kMaxGroup, "step end (large batch): bad group size");
+  k_bb_step_end<<<(unsigned)e.n, 1, 0, s>>>(e, nc, loss_rows, gated);
   LOC_LAUNCHED();
   return 0;
 }
@@ -547,10 +554,14 @@ static int bb_sms() {
   return n;
 }
 
-int bb_stats_launch(const BigArgs& a, cudaStream_t s) {
-  LOC_CHECK(a.nb >= 1 && a.nb <= LOC_MAX_BATCH_SIZE, "batch statistics: a step holds 1..256 rows");
-  const int64_t nwords = cdiv(a.K, 16);
-  k_bb_stats<<<(unsigned)cdiv(nwords, 32), 256, 0, s>>>(a);
+int bb_stats_launch(const BigGroupArgs& g, cudaStream_t s) {
+  LOC_CHECK(g.n >= 1 && g.n <= kMaxGroup, "batch statistics: bad group size");
+  int64_t kmax = 0;
+  for (int i = 0; i < g.n; ++i) {
+    LOC_CHECK(g.a[i].nb >= 1 && g.a[i].nb <= LOC_MAX_BATCH_SIZE, "batch statistics: a step holds 1..256 rows");
+    if (g.a[i].K > kmax) kmax = g.a[i].K;
+  }
+  k_bb_stats<<<dim3((unsigned)cdiv(cdiv(kmax, 16), 32), (unsigned)g.n), 256, 0, s>>>(g);
   LOC_LAUNCHED();
   return 0;
 }

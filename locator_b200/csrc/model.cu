@@ -385,23 +385,14 @@ static bool chain_capable(const loc_model* m) {
   return !off && m->use_tc && m->hid_tc && m->exchange == nullptr && m->tp == nullptr;
 }
 
-// One optimizer step of a model created with batch_size > 32 (bigbatch.cu): batch statistics over all rows of the
-// step, first-layer forward with those statistics (one wide pass over W1 on the tcgen05 path), the step's 32-row
-// chunks through the hidden stack, then one pass over W1 | m | v (dW1 over all rows + Adam) and the small-layer update
-// over the chunks.  Plain launches on one stream.
-static int train_step_big(loc_model* m, const RowSrc& src, int gated, cudaStream_t s) {
-  m->chain_open = 0;
-  m->span_perm = nullptr;
-  const int nb = src.nb, nc = (nb + kMaxB - 1) / kMaxB;
-  LOC_CHECK(nb >= 1 && nc <= m->cap_chunks && m->bb_mean != nullptr, "training step: more rows than the model's batch_size");
-  LOC_CHECK(m->exchange == nullptr && m->tp == nullptr, "sharded models train with batch_size <= 32");
+static BigArgs big_args(loc_model* m, const RowSrc& src, int gated) {
   BigArgs g;
   g.K = m->K;
   g.H = m->H;
   g.L = m->L;
   g.gated = gated;
   g.tiled = m->use_tc;
-  g.nb = nb;
+  g.nb = src.nb;
   g.packed = m->train_packed;
   g.row_words = m->train_row_words;
   g.src = src;
@@ -429,63 +420,124 @@ static int train_step_big(loc_model* m, const RowSrc& src, int gated, cudaStream
   g.Hc = m->H / m->cluster;
   g.slice_mode = m->hid_tc;
   g.st = m->st;
-  if (bb_stats_launch(g, s)) return 1;
-  const bool wide = m->wide != nullptr && m->use_tc && m->hid_tc && getenv("LOC_NO_WIDE") == nullptr;
-  if (wide) {
-    L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 0, gated);
-    a.mmean = m->bb_mean;  // "inference" forward with the step's batch statistics
-    a.mvar = m->bb_var;
-    if (l1_forward_wide_tc(a, m->n_partials, nb, m->wide, s)) return 1;
+  return g;
+}
+
+// One optimizer step of n models created with batch_size > 32 (bigbatch.cu), the same number of rows each (a
+// single model, or a replicate group of loc_group_train_epochs):
+//   batch statistics over all rows of every model's step (one launch for the group),
+//   first-layer forward with those statistics (one wide pass over W1 per model on the tcgen05 path),
+//   the step's 32-row chunks through the hidden stack -- tcgen05: side by side, one cluster per chunk, whole models
+//     per grouped launch (floor(8 / chunks) models each), then the step end of all models in one launch,
+//   one pass over W1 | m | v per model (dW1 over all rows + Adam), back to back,
+//   the small-layer update over the chunks: after the backward for a single model; in a group on the model's side
+//     stream, forked after the hidden launch that holds its chunks (it runs under the other models' backwards) and
+//     joined before the next step.
+// Every model's launches are the ones it gets alone, with the same arguments, so the group gives the same bits.
+static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int gated, cudaStream_t s) {
+  const int nb = srcs[0].nb, nc = (nb + kMaxB - 1) / kMaxB;
+  LOC_CHECK(n >= 1 && n <= kMaxGroup, "training step (large batch): bad group size");
+  BigGroupArgs bg;
+  bg.n = n;
+  for (int g = 0; g < n; ++g) {
+    loc_model* m = ms[g];
+    m->chain_open = 0;
+    m->span_perm = nullptr;
+    LOC_CHECK(srcs[g].nb == nb, "training step (large batch): the models of a group step the same number of rows");
+    LOC_CHECK(nb >= 1 && nc <= m->cap_chunks && m->bb_mean != nullptr, "training step: more rows than the model's batch_size");
+    LOC_CHECK(m->exchange == nullptr && m->tp == nullptr, "sharded models train with batch_size <= 32");
+    bg.a[g] = big_args(m, srcs[g], gated);
   }
-  const int64_t chunk_stride = (int64_t)m->L * kMaxB * m->H;
-  // tcgen05 hidden stack: the chunks run side by side, one cluster each (k_hidden_tc_group); their loss sums and the
-  // step's optimizer bookkeeping follow in k_bb_step_end.  LOC_BB_SERIAL=1 (tests): one launch per chunk.
-  const bool side_by_side = wide && nc > 1 && getenv("LOC_BB_SERIAL") == nullptr;
-  HidGroupArgs hg;
-  hg.n = nc;
-  for (int c = 0; c < nc; ++c) {
-    RowSrc sc = src;
-    if (src.rows != nullptr)
-      sc.offset = src.offset + (int64_t)kMaxB * c;
-    else
-      sc.row0 = src.row0 + kMaxB * c;
-    sc.nb = nb - kMaxB * c < kMaxB ? nb - kMaxB * c : kMaxB;
-    if (!wide) {
-      L1Args a = l1_args(m, m->train_packed, m->train_row_words, sc, 0, gated);
-      a.mmean = m->bb_mean;
+  if (bb_stats_launch(bg, s)) return 1;
+  const bool no_wide = getenv("LOC_NO_WIDE") != nullptr;
+  const bool wide = ms[0]->wide != nullptr && ms[0]->use_tc && ms[0]->hid_tc && !no_wide;
+  if (wide) {
+    for (int g = 0; g < n; ++g) {
+      loc_model* m = ms[g];
+      L1Args a = l1_args(m, m->train_packed, m->train_row_words, srcs[g], 0, gated);
+      a.mmean = m->bb_mean;  // "inference" forward with the step's batch statistics
       a.mvar = m->bb_var;
-      if (forward_l1(m, a, s)) return 1;
+      if (l1_forward_wide_tc(a, m->n_partials, nb, m->wide, s)) return 1;
     }
-    HidArgs h = hid_args(m, sc, 1, gated, m->train_locs, nullptr);
-    if (wide) {
-      h.partials = m->wide;
-      h.n_partials = m->n_partials;
-      h.partial_stride = (int64_t)nc * kMaxB * m->H;
-      h.partial_row0 = kMaxB * c;
+  }
+  // tcgen05 hidden stack: the chunks run side by side, one cluster each (k_hidden_tc_group); their loss sums and the
+  // step's optimizer bookkeeping follow in k_bb_step_end.  LOC_BB_SERIAL=1 (tests): one launch per chunk.  A model's
+  // chunks never straddle two launches: each publishes DevState::hid_seq once all of the model's chunks are done.
+  const bool side_by_side = wide && nc > 1 && getenv("LOC_BB_SERIAL") == nullptr;
+  const int per_launch = side_by_side ? kMaxGroup / nc : 1;
+  const bool fork = n > 1;
+  for (int g0 = 0; g0 < n; g0 += per_launch) {
+    const int g1 = g0 + per_launch < n ? g0 + per_launch : n;
+    HidGroupArgs hg;
+    hg.n = 0;
+    for (int g = g0; g < g1; ++g) {
+      loc_model* m = ms[g];
+      const RowSrc& src = srcs[g];
+      const int64_t chunk_stride = (int64_t)m->L * kMaxB * m->H;
+      const int first = hg.n;
+      for (int c = 0; c < nc; ++c) {
+        RowSrc sc = src;
+        if (src.rows != nullptr)
+          sc.offset = src.offset + (int64_t)kMaxB * c;
+        else
+          sc.row0 = src.row0 + kMaxB * c;
+        sc.nb = nb - kMaxB * c < kMaxB ? nb - kMaxB * c : kMaxB;
+        if (!wide) {
+          L1Args a = l1_args(m, m->train_packed, m->train_row_words, sc, 0, gated);
+          a.mmean = m->bb_mean;
+          a.mvar = m->bb_var;
+          if (forward_l1(m, a, s)) return 1;
+        }
+        HidArgs h = hid_args(m, sc, 1, gated, m->train_locs, nullptr);
+        if (wide) {
+          h.partials = m->wide;
+          h.n_partials = m->n_partials;
+          h.partial_stride = (int64_t)nc * kMaxB * m->H;
+          h.partial_row0 = kMaxB * c;
+        }
+        h.acts = m->acts + c * chunk_stride;
+        h.dzs = m->dzs + c * chunk_stride;
+        h.outs = m->outs + c * 256;
+        h.loss_rows = nb;
+        h.row_base = kMaxB * c;
+        h.mask_rows = kMaxB * m->cap_chunks;
+        h.chunk_flags = (c > 0 ? 1 : 0) | (c < nc - 1 ? 2 : 0);
+        begin_training_hidden(m, h);
+        if (side_by_side) {
+          h.chunk_flags = 2;  // nobody bumps the step counters inside the launch
+          h.val_slot = m->val_slots + 2 * c;
+          hg.a[hg.n++] = h;
+          continue;
+        }
+        if (m->hid_tc ? hidden_tc_launch(h, s) : hidden_launch(h, m->cluster, s)) return 1;
+      }
+      for (int i = first; i < hg.n; ++i) hg.a[i].hid_seq = m->h_hid_seq;  // published concurrently: the same (final) value
     }
-    h.acts = m->acts + c * chunk_stride;
-    h.dzs = m->dzs + c * chunk_stride;
-    h.outs = m->outs + c * 256;
-    h.loss_rows = nb;
-    h.row_base = kMaxB * c;
-    h.mask_rows = kMaxB * m->cap_chunks;
-    h.chunk_flags = (c > 0 ? 1 : 0) | (c < nc - 1 ? 2 : 0);
-    begin_training_hidden(m, h);
-    if (side_by_side) {
-      h.chunk_flags = 2;  // nobody bumps the step counters inside the launch
-      h.val_slot = m->val_slots + 2 * c;
-      hg.a[c] = h;
-      continue;
+    if (side_by_side && hidden_tc_group_launch(hg, s)) return 1;
+    if (fork) {
+      LOC_CUDA(cudaEventRecord(ms[g0]->ev_hid, s));
+      for (int g = g0; g < g1; ++g) {
+        loc_model* m = ms[g];
+        LOC_CUDA(cudaStreamWaitEvent(m->side, ms[g0]->ev_hid, 0));
+        if (bb_hidden_update_launch(bg.a[g], m->side)) return 1;
+        LOC_CUDA(cudaEventRecord(m->ev_upd, m->side));
+      }
     }
-    if (m->hid_tc ? hidden_tc_launch(h, s) : hidden_launch(h, m->cluster, s)) return 1;
   }
   if (side_by_side) {
-    for (int c = 0; c < nc; ++c) hg.a[c].hid_seq = m->h_hid_seq;  // published concurrently: the same (final) value
-    if (hidden_tc_group_launch(hg, s)) return 1;
-    if (bb_step_end_launch(m->st, m->val_slots, nc, nb, gated, s)) return 1;
+    BigEndArgs e;
+    e.n = n;
+    for (int g = 0; g < n; ++g) {
+      e.st[g] = ms[g]->st;
+      e.slots[g] = ms[g]->val_slots;
+    }
+    if (bb_step_end_launch(e, nc, nb, gated, s)) return 1;
   }
-  if (bb_l1_backward_launch(g, m->bb_pq, s)) return 1;
-  return bb_hidden_update_launch(g, s);
+  for (int g = 0; g < n; ++g)
+    if (bb_l1_backward_launch(bg.a[g], ms[g]->bb_pq, s)) return 1;
+  if (!fork) return bb_hidden_update_launch(bg.a[0], s);
+  for (int g = 0; g < n; ++g) LOC_CUDA(cudaStreamWaitEvent(s, ms[g]->ev_upd, 0));
+  return 0;
 }
 
 // One optimizer step: 3-4 launches (stage_mask selects a subset for profiling / tests).
@@ -512,7 +564,7 @@ static int train_step(loc_model* m, const RowSrc& src, int gated, cudaStream_t s
                       const RowSrc* next = nullptr, bool have_fwd = false) {
   if (m->B > kMaxB) {
     LOC_CHECK(stage_mask == 15, "single stages of a step are only available for batch_size <= 32");
-    return train_step_big(m, src, gated, s);
+    return train_step_big(&m, &src, 1, gated, s);
   }
   L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, gated);
   if (next != nullptr && m->use_tc) {
@@ -1160,7 +1212,6 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
               "loc_group_train_epochs: every model needs bound training / validation data and a batch order");
     LOC_CHECK(m->hid_tc && m->use_tc, "loc_group_train_epochs: grouped replicates need the tcgen05 kernels (width 256)");
     LOC_CHECK(m->exchange == nullptr && m->tp == nullptr, "loc_group_train_epochs: sharded models cannot be grouped");
-    LOC_CHECK(m->B <= kMaxB, "loc_group_train_epochs: grouped replicates train with batch_size <= 32");
     LOC_CHECK(m->L == m0->L && m->B == m0->B && m->n_train == m0->n_train,
               "loc_group_train_epochs: replicates of a group must share nlayers, batch size and training-set size");
   }
@@ -1190,8 +1241,12 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
   // max(B, H) instead of B + H / G -- a gain only when the weight stream outlasts the hidden stack, hence
   // K >= kRingMinK.  "lockstep" (small K, models on all SMs, or LOC_GROUP_SCHEDULE=lockstep): all hidden
   // stacks in one launch, then the backwards back to back, updates on side streams.
+  // Models of more than 32 rows a step ("large batch", LOC_GROUP_SCHEDULE does not apply): train_step_big with the
+  // whole group, a lockstep of its own -- one statistics launch, hidden stacks packed whole models per launch, one
+  // step end, the backwards back to back, updates on side streams.
+  const bool big = m0->B > kMaxB;
   const char* sched = getenv("LOC_GROUP_SCHEDULE");  // "ring" / "lockstep" override the choice by K (tests, A/B)
-  bool ring = n_models >= 2 && (m0->K >= kRingMinK || (sched != nullptr && strcmp(sched, "ring") == 0));
+  bool ring = !big && n_models >= 2 && (m0->K >= kRingMinK || (sched != nullptr && strcmp(sched, "ring") == 0));
   for (int g = 0; g < n_models; ++g) ring = ring && models[g]->n_bwd_blocks <= sm_count() - 16;
   if (sched != nullptr && strcmp(sched, "lockstep") == 0) ring = false;
   struct Pending {
@@ -1251,8 +1306,13 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
         g0 = g1;
       }
     }
+    for (int64_t off = 0; big && off < m0->n_train; off += m0->B) {
+      RowSrc srcs[kMaxGroup];
+      for (int g = 0; g < n_models; ++g) srcs[g] = step_rows(g, off);
+      if (train_step_big(models, srcs, n_models, 1, s)) return 1;
+    }
     bool have_fwd = false;
-    for (int64_t off = 0; !ring && off < m0->n_train; off += m0->B) {
+    for (int64_t off = 0; !ring && !big && off < m0->n_train; off += m0->B) {
       const bool has_next = off + m0->B < m0->n_train;
       HidGroupArgs hg;
       hg.n = n_models;

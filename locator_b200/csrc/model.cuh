@@ -226,11 +226,22 @@ struct BigArgs {
   int Hc, slice_mode;
   DevState* st;
 };
-int bb_stats_launch(const BigArgs& a, cudaStream_t s);
+// The same step of up to kMaxGroup models (replicate groups: same row count per step, K may differ)
+struct BigGroupArgs {
+  int n;
+  BigArgs a[kMaxGroup];
+};
+// Step end of the models of a group whose chunks ran side by side: model g's per-chunk loss sums are slots[g]
+struct BigEndArgs {
+  int n;
+  DevState* st[kMaxGroup];
+  const float* slots[kMaxGroup];
+};
+int bb_stats_launch(const BigGroupArgs& g, cudaStream_t s);
 int bb_l1_backward_launch(const BigArgs& a, float* pq_part, cudaStream_t s);
 int64_t bb_pq_floats(int64_t K, int H);  // scratch of the backward: per column group partial sums for gamma / beta
 int bb_hidden_update_launch(const BigArgs& a, cudaStream_t s);
-int bb_step_end_launch(DevState* st, const float* slots, int nc, int loss_rows, int gated, cudaStream_t s);
+int bb_step_end_launch(const BigEndArgs& e, int nc, int loss_rows, int gated, cudaStream_t s);
 constexpr int kMaxChunks = LOC_MAX_BATCH_SIZE / LOC_MAX_BATCH;
 
 int tp_exchange(loc_tp* tp, const float* partials, int n_partials, cudaStream_t s);

@@ -372,9 +372,11 @@ def fit_group(models, xs, ys, validation_datas, epochs=None, patience=100, verbo
     """Train up to 8 independent models (replicates) side by side on one GPU.
 
     Same semantics per model as ``LocatorModel.fit`` (each model keeps its own shuffle stream,
-    callbacks state and history); the steps are issued in lockstep through
-    ``loc_group_train_epochs`` so the models' latency-bound hidden stacks share one launch.  Models
-    must have the same nlayers / batch size / number of training rows (replicates of one run do).
+    callbacks state and history, and ends bit-identical to the same model trained alone); the steps
+    are issued in lockstep through ``loc_group_train_epochs`` so the models' latency-bound hidden
+    stacks share launches.  Any batch size: above 32 rows the models' batch statistics and step ends
+    share one launch each, and their 32-row chunks share hidden-stack launches.  Models must have the
+    same nlayers / batch size / number of training rows (replicates of one run do) and width 256.
     Returns the list of History objects.
     """
     G = len(models)

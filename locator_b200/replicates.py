@@ -94,8 +94,8 @@ def _run_items(L, items, base, reps=None):
     """Train + predict a list of replicates inside the current process / on the current device.
 
     One replicate: the reference's sequence (load_network, train_network, predict_locs).  Several:
-    the models are trained side by side as one lockstep group (model.fit_group; results are
-    bit-identical to training them one after the other), then predicted one by one.
+    the models are trained side by side as one lockstep group (model.fit_group, at any batch size;
+    results are bit-identical to training them one after the other), then predicted one by one.
     ``reps``: the items' matrices when a Prefetcher has already prepared them.
     """
     from .model import fit_group
@@ -116,7 +116,7 @@ def _run_items(L, items, base, reps=None):
             args.out = original_out
     _tick(f"{len(models)} models created")
     same = len({(r["traingen"].n, m.nlayers, m.batch_size) for r, m in zip(reps, models)}) == 1
-    if len(reps) > 1 and same and all(m.impl == "tcgen05" and m.batch_size <= 32 for m in models):
+    if len(reps) > 1 and same and all(m.impl == "tcgen05" for m in models):
         start = time.time()
         histories = fit_group(models, [r["traingen"] for r in reps], [r["trainlocs"] for r in reps],
                               [(r["testgen"], r["testlocs"]) for r in reps], epochs=args.max_epochs,

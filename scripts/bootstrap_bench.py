@@ -21,6 +21,8 @@ def main():
     ap.add_argument("--epochs", type=int, default=20)
     ap.add_argument("--snps", type=int, default=100000)
     ap.add_argument("--samples", type=int, default=1000)
+    ap.add_argument("--batch_size", type=int, default=None, help="passed to the CLI (default: the CLI's own)")
+    ap.add_argument("--replicates_per_gpu", type=int, default=None, help="passed to the CLI (default: the CLI's own)")
     a = ap.parse_args()
     import bench
     from locator_b200 import io
@@ -46,6 +48,9 @@ def main():
         cmd = [sys.executable, "-m", "locator_b200", "--zarr", z, "--sample_data", "/tmp/bb/samples.txt", "--out", out,
                "--seed", "12345", "--bootstrap", "--nboots", str(a.nboots), "--max_epochs", str(a.epochs),
                "--patience", "1000", "--keras_verbose", "0", "--gpus", str(n)]
+        for flag in ("batch_size", "replicates_per_gpu"):
+            if getattr(a, flag) is not None:
+                cmd += [f"--{flag}", str(getattr(a, flag))]
         t = time.time()
         r = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True, timeout=1500)
         dt = time.time() - t
@@ -60,7 +65,8 @@ def main():
         print(n, "GPU(s):", json.dumps(res[n]), flush=True)
     same = all(outs[1] == outs[n] for n in outs)
     print(json.dumps({"workload": f"bootstrap: FULL + {a.nboots} replicates x {a.samples} samples x {a.snps} SNPs, "
-                                  f"{a.epochs} epochs each", "results": res,
+                                  f"{a.epochs} epochs each", "batch_size": a.batch_size,
+                      "replicates_per_gpu": a.replicates_per_gpu, "results": res,
                       "outputs_identical_across_gpu_counts": same}))
 
 
