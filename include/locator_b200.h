@@ -189,6 +189,14 @@ int loc_model_pool_clear(void);
 int64_t loc_debug_timeline(uint64_t* h_out, int64_t max_records);
 /* First-layer kernel family this model actually runs: "tcgen05" or "simt". */
 const char* loc_model_impl(const loc_model* m);
+/* Hidden-stack kernel family this model actually runs: "tcgen05" (width 256, nlayers up to 14) or "simt" (the
+ * CUDA-core stack: other widths, deeper width-256 stacks -- behind the tcgen05 first layer there). */
+const char* loc_model_hidden_impl(const loc_model* m);
+/* Deepest nlayers in [2, 64] that loc_model_create can build at this width: the CUDA-core hidden stack's layout
+ * (needed by every model) has at least one weight slot in shared memory at some admissible cluster size.  0: no
+ * nlayers fits (the widths above 320 except 384), or the width is not a multiple of 32 in [32, 1024].  Host arithmetic, no
+ * device needed; an upper bound -- loc_model_create also needs the device to schedule the cluster. */
+int32_t loc_hidden_max_nlayers(int32_t width);
 
 /* Philox glorot-uniform kernels, zero biases, gamma 1 / beta 0 / moving mean 0 /
  * moving var 1, zero Adam state, reset optimizer + callback state. `seed` also

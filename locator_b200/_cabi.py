@@ -67,6 +67,8 @@ SIGNATURES = {
     "loc_model_pool_clear": (C.c_int, []),
     "loc_debug_timeline": (I64, [P, I64]),
     "loc_model_impl": (C.c_char_p, [P]),
+    "loc_model_hidden_impl": (C.c_char_p, [P]),
+    "loc_hidden_max_nlayers": (I32, [I32]),
     "loc_model_init": (C.c_int, [P, C.c_uint64, P]),
     "loc_model_num_weights": (C.c_int, [P]),
     "loc_model_weight_size": (I64, [P, I32]),

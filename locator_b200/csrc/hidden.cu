@@ -730,13 +730,22 @@ static int launch_hidden_cluster(const HidArgs& a, int cluster, cudaStream_t s, 
   return 0;
 }
 
+static const int kClusterCands[5] = {16, 8, 4, 2, 1};
+
+int hidden_max_nlayers(int H) {
+  if (H < 32 || H > 1024 || H % 32 != 0) return 0;
+  // fixed shared memory grows with L, so the shapes with a slot are L = 2 .. deepest
+  for (int L = 64; L >= 2; --L)
+    for (int c : kClusterCands)
+      if (H % (4 * c) == 0 && hidden_slots(H, L, c) >= 1) return L;
+  return 0;
+}
+
 int hidden_max_cluster(int H, int L) {
   cudaFuncSetAttribute(k_hidden<256, 16>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
   cudaFuncSetAttribute(k_hidden<0, 0>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
   cudaGetLastError();
-  const int cands[5] = {16, 8, 4, 2, 1};
-  for (int ci = 0; ci < 5; ++ci) {
-    const int c = cands[ci];
+  for (int c : kClusterCands) {
     if (H % (4 * c) != 0) continue;
     if (hidden_slots(H, L, c) < 1) continue;
     const size_t smem = hidden_smem_bytes(H, L, c);

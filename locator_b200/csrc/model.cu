@@ -971,6 +971,10 @@ int loc_model_pool_clear(void) {
 
 const char* loc_model_impl(const loc_model* m) { return (m != nullptr && m->use_tc) ? "tcgen05" : "simt"; }
 
+const char* loc_model_hidden_impl(const loc_model* m) { return (m != nullptr && m->hid_tc) ? "tcgen05" : "simt"; }
+
+int32_t loc_hidden_max_nlayers(int32_t width) { return hidden_max_nlayers(width); }
+
 int loc_model_init(loc_model* m, uint64_t seed, void* stream) {
   LOC_CHECK(m != nullptr, "loc_model_init: null model");
   cudaStream_t s = (cudaStream_t)stream;
@@ -1210,7 +1214,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
     loc_model* m = models[g];
     LOC_CHECK(m != nullptr && d_perms[g] != nullptr && m->train_packed != nullptr && m->val_packed != nullptr,
               "loc_group_train_epochs: every model needs bound training / validation data and a batch order");
-    LOC_CHECK(m->hid_tc && m->use_tc, "loc_group_train_epochs: grouped replicates need the tcgen05 kernels (width 256)");
+    LOC_CHECK(m->hid_tc && m->use_tc, "loc_group_train_epochs: grouped replicates need the tcgen05 first layer and hidden stack (width 256, nlayers <= 14)");
     LOC_CHECK(m->exchange == nullptr && m->tp == nullptr, "loc_group_train_epochs: sharded models cannot be grouped");
     LOC_CHECK(m->L == m0->L && m->B == m0->B && m->n_train == m0->n_train,
               "loc_group_train_epochs: replicates of a group must share nlayers, batch size and training-set size");

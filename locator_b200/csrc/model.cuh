@@ -160,6 +160,7 @@ int hidden_launch(const HidArgs& a, int cluster, cudaStream_t s);
 int hidden_update_launch(const UpdArgs& a, cudaStream_t s, bool overlap_previous = false);
 int hidden_max_cluster(int H, int L);  // largest usable cluster size (16, 8, ...) for this device
 int hidden_slots(int H, int L, int cluster);
+int hidden_max_nlayers(int H);  // deepest L in [2, 64] with a slot at some cluster size (host arithmetic), 0 = none
 int hidden_reslice(const float* small, float* fs, float* bs, int H, int L, int cluster, cudaStream_t s);
 size_t hidden_smem_bytes(int H, int L, int cluster);
 

@@ -117,17 +117,27 @@ def set_args(namespace):
 def validate_args(ns):
     """Limits of this build, checked before any data is read (the reference accepts any value and fails -- or
     not -- inside Keras).  Documented in INTEGRATION.md as deliberate deviations of the boundary."""
-    from ._cabi import lib  # noqa: F401  (fails loudly here when the CUDA library is missing)
+    from ._cabi import lib  # fails loudly here when the CUDA library is missing
 
     problems = []
     if not 1 <= int(ns.batch_size) <= 256:
         problems.append(f"--batch_size {ns.batch_size}: must be in [1, 256] (up to 32, the reference's default, a step runs "
                         "on the fused tensor-core kernels; 33..256 rows go through the stack in 32-row chunks)")
-    if int(ns.width) < 32 or int(ns.width) > 1024 or int(ns.width) % 32:
+    width, nlayers = int(ns.width), int(ns.nlayers)
+    # every model needs the CUDA-core hidden stack's shared-memory layout to hold at least one weight slice
+    deepest = int(lib.loc_hidden_max_nlayers(width))
+    if width < 32 or width > 1024 or width % 32:
         problems.append(f"--width {ns.width}: must be a multiple of 32 in [32, 1024] (256, the default, runs on the "
                         "tensor cores; other widths on the CUDA-core kernels)")
-    if not 2 <= int(ns.nlayers) <= 64:
+    elif deepest == 0:
+        ok = ", ".join(str(w) for w in range(32, 1025, 32) if lib.loc_hidden_max_nlayers(w) > 0)
+        problems.append(f"--width {ns.width}: this build cannot hold a hidden layer of that width in shared memory at any "
+                        f"--nlayers (widths that build: {ok})")
+    if not 2 <= nlayers <= 64:
         problems.append(f"--nlayers {ns.nlayers}: must be in [2, 64]")
+    elif 0 < deepest < nlayers:
+        problems.append(f"--nlayers {ns.nlayers}: at --width {width} this build holds at most {deepest} hidden layers "
+                        "(the CUDA-core hidden stack keeps one layer's weight slice in shared memory)")
     if not 0.0 <= float(ns.dropout_prop) < 1.0:
         problems.append(f"--dropout_prop {ns.dropout_prop}: must be in [0, 1)")
     if int(ns.max_epochs) < 1:

@@ -122,7 +122,13 @@ class LocatorModel:
 
     @property
     def impl(self):
+        """First-layer kernel family: "tcgen05" or "simt" (CUDA cores)."""
         return lib.loc_model_impl(self._h).decode()
+
+    @property
+    def hidden_impl(self):
+        """Hidden-stack kernel family: "tcgen05" or "simt" (CUDA cores; width-256 stacks deeper than 14 layers)."""
+        return lib.loc_model_hidden_impl(self._h).decode()
 
     # ---- weights (Keras order) -------------------------------------------------
     def num_weights(self):
@@ -376,7 +382,8 @@ def fit_group(models, xs, ys, validation_datas, epochs=None, patience=100, verbo
     are issued in lockstep through ``loc_group_train_epochs`` so the models' latency-bound hidden
     stacks share launches.  Any batch size: above 32 rows the models' batch statistics and step ends
     share one launch each, and their 32-row chunks share hidden-stack launches.  Models must have the
-    same nlayers / batch size / number of training rows (replicates of one run do) and width 256.
+    same nlayers / batch size / number of training rows (replicates of one run do) and run the tcgen05 first layer
+    and hidden stack (width 256, nlayers up to 14: ``impl == hidden_impl == "tcgen05"``).
     Returns the list of History objects.
     """
     G = len(models)

@@ -116,7 +116,10 @@ def _run_items(L, items, base, reps=None):
             args.out = original_out
     _tick(f"{len(models)} models created")
     same = len({(r["traingen"].n, m.nlayers, m.batch_size) for r, m in zip(reps, models)}) == 1
-    if len(reps) > 1 and same and all(m.impl == "tcgen05" for m in models):
+    # groups need the tcgen05 first layer AND hidden stack: width-256 models deeper than 14 layers run their hidden
+    # stack on CUDA cores and train one after the other
+    tc = all(m.impl == "tcgen05" and m.hidden_impl == "tcgen05" for m in models)
+    if len(reps) > 1 and same and tc:
         start = time.time()
         histories = fit_group(models, [r["traingen"] for r in reps], [r["trainlocs"] for r in reps],
                               [(r["testgen"], r["testlocs"]) for r in reps], epochs=args.max_epochs,

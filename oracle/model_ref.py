@@ -83,12 +83,15 @@ class RefLocator:
 
     def __init__(self, K, width=256, nlayers=10, dropout=0.25, weights=None, seed=0, lr=1e-3, numerics="fp32",
                  l1_parts=1):
-        """numerics: "fp32" (the reference's CPU arithmetic) or "tf32" (the device's operand rounding, see
-        tf32_rna / tf32_trunc above).  l1_parts > 1: the first layer's sum over the SNPs is taken in that many
+        """numerics: "fp32" (the reference's CPU arithmetic), "tf32" (the device's operand rounding, see
+        tf32_rna / tf32_trunc above) or "tf32_l1" (tcgen05 first layer, CUDA-core hidden stack -- width-256 models
+        deeper than the tcgen05 stack holds: the first layer's forward and backward as in "tf32", the hidden and output
+        products in fp32).  l1_parts > 1: the first layer's sum over the SNPs is taken in that many
         contiguous parts (64-SNP tiles dealt out like the device's CTAs) added in order -- a different fp32
         summation order of the same products, which is all a change of the device's CTA count does."""
-        assert numerics in ("fp32", "tf32")
-        self.tf32 = numerics == "tf32"
+        assert numerics in ("fp32", "tf32", "tf32_l1")
+        self.tf32 = numerics == "tf32"  # tf32 operands in the hidden and output layers
+        self.tf32_l1 = numerics in ("tf32", "tf32_l1")  # tf32 operands in the first layer, its backward as the device's
         self.l1_parts = int(l1_parts)
         if nlayers < 2:
             raise ValueError("oracle restates nlayers >= 2 (first Dense precedes Dropout)")
@@ -141,10 +144,11 @@ class RefLocator:
         op_a = tf32_rna if self.tf32 else (lambda t: t)     # operand tiles the kernels build
         op_w = tf32_trunc if self.tf32 else (lambda t: t)   # weights as stored
         for i in range(self.L):
+            oa, ow = (tf32_rna, tf32_trunc) if i == 0 and self.tf32_l1 else (op_a, op_w)
             if i == 0 and self.l1_parts > 1:
-                z = self._l1_in_parts(op_a(acts[-1]), op_w(self.W[0])) + self.b[0]
+                z = self._l1_in_parts(oa(acts[-1]), ow(self.W[0])) + self.b[0]
             else:
-                z = op_a(acts[-1]) @ op_w(self.W[i]) + self.b[i]
+                z = oa(acts[-1]) @ ow(self.W[i]) + self.b[i]
             h = elu(z)
             zs.append(z)
             if i == self.n_before - 1:  # Dropout sits after the floor(L/2)-th Dense
@@ -204,11 +208,11 @@ class RefLocator:
             dz = torch.where(z > 0, dh, dh * torch.exp(z))  # EluGrad: (out+1)*g for out<0
             dzs[i] = dz
             gb[i] = dz.sum(0)
-            if i == 0 and self.tf32:
+            if i == 0 and self.tf32_l1:
                 break  # first layer below: the device never forms d loss / d (BN output)
             gW[i] = acts[i].T @ dz
             dh = (tf32_rna(dz) @ tf32_trunc(self.W[i]).T) if self.tf32 else (dz @ self.W[i].T)
-        if self.tf32:
+        if self.tf32_l1:
             # first-layer backward as the device computes it (csrc/l1_tc.cu): S = (x - mean)^T dz with the centred
             # genotypes rounded to tf32 (exact for a batch of 32) and dz as hi + lo parts (fp32-accurate);
             # dW1 = inv * S + beta * c0, dgamma = rs * sum_j W1 * S, dbeta = sum_j W1 * c0, c0 = column sums of dz

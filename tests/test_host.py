@@ -596,10 +596,13 @@ def test_validate_args_limits_of_this_build():
         return L.build_parser().parse_args(["--vcf", "x.vcf", "--sample_data", "s.txt", "--out", "o"] + list(extra))
 
     for ok in ([], ["--batch_size", "1"], ["--batch_size", "64"], ["--batch_size", "256"], ["--width", "96"],
-               ["--nlayers", "2"], ["--dropout_prop", "0"]):
+               ["--nlayers", "2"], ["--dropout_prop", "0"], ["--nlayers", "21"], ["--width", "320", "--nlayers", "13"]):
         L.validate_args(ns(*ok))
     for bad, word in ((["--batch_size", "0"], "batch_size"), (["--batch_size", "257"], "batch_size"),
                       (["--width", "100"], "width"), (["--nlayers", "1"], "nlayers"), (["--dropout_prop", "1.0"], "dropout_prop"),
-                      (["--max_epochs", "0"], "max_epochs"), (["--windows", "--window_size", "2e5"], "window_size")):
+                      (["--max_epochs", "0"], "max_epochs"), (["--windows", "--window_size", "2e5"], "window_size"),
+                      # deepest stack per width: the CUDA-core hidden stack's shared-memory layout (loc_hidden_max_nlayers)
+                      (["--nlayers", "22"], "at most 21"), (["--width", "512"], "width 512"),
+                      (["--width", "224", "--nlayers", "11"], "at most 10")):
         with pytest.raises(SystemExit, match=word):
             L.validate_args(ns(*bad))

@@ -141,6 +141,47 @@ def test_oracle_gradients_match_autograd(K, H, L, p, B):
     assert float(grads[0][0]) == 0.0  # d gamma of the constant column is exactly zero
 
 
+def test_oracle_tf32_l1_rounds_the_first_layer_only():
+    """numerics="tf32_l1" (tcgen05 first layer + CUDA-core hidden stack, width-256 models deeper than 14 layers):
+    the first layer's pre-activation equals the "tf32" mode's bit for bit; from that layer's output on, the hidden and
+    output layers are the "fp32" mode's arithmetic; the first-layer gradient is the device's formula (as in "tf32")."""
+    K, H, L, p, B = 70, 24, 5, 0.25, 12
+    rng = np.random.default_rng(4)
+    x = rng.integers(0, 3, size=(B, K)).astype(np.uint8)
+    y = rng.normal(size=(B, 2)).astype(np.float32)
+    ws = model_ref.init_weights(K, H, L, seed=6)
+    ws[0] = rng.uniform(0.5, 1.5, K).astype(np.float32)
+    ws[1] = rng.normal(0, 0.1, K).astype(np.float32)
+    for i in range(5, len(ws), 2):
+        ws[i] = rng.normal(0, 0.05, ws[i].shape).astype(np.float32)
+    mask = rng.uniform(size=(B, H)) >= p
+    out = {}
+    for mode in ("fp32", "tf32", "tf32_l1"):
+        ref = model_ref.RefLocator(K, H, L, dropout=p, weights=ws, numerics=mode)
+        out[mode] = (ref,) + ref.gradients(x, y, mask)
+    ref, loss, grads, c = out["tf32_l1"]
+    assert torch.equal(c["zs"][0], out["tf32"][3]["zs"][0])
+    assert not torch.equal(c["zs"][0], out["fp32"][3]["zs"][0])  # the rounding is visible at these scales
+    # the hidden and output layers in plain fp32, fed the first layer's output
+    a = c["acts"][1]
+    for i in range(1, L):
+        z = a @ ref.W[i] + ref.b[i]
+        assert torch.equal(z, c["zs"][i]), i
+        a = c["acts"][i + 1]
+    y2 = (a @ ref.W[L] + ref.b[L]) @ ref.W[L + 1] + ref.b[L + 1]
+    assert loss == float(model_ref.RefLocator.loss_per_sample(y2, torch.as_tensor(y)).mean())
+    assert loss != out["tf32"][1]
+    # hidden-layer backward in fp32: d loss / d z of layer 0 from fp32 products, then the device's first-layer formula
+    dz1, W1 = c["dzs"][1], ref.W[1]
+    dz0 = torch.where(c["zs"][0] > 0, dz1 @ W1.T, (dz1 @ W1.T) * torch.exp(c["zs"][0]))  # Dropout sits after layer 1
+    assert torch.equal(c["dzs"][0], dz0)
+    S = model_ref.tf32_rna(c["x"] - c["mean"]).T @ dz0
+    assert torch.equal(grads[2], (c["rs"] * ref.gamma)[:, None] * S + ref.beta[:, None] * dz0.sum(0)[None, :])
+    # and the whole gradient stays close to the fp32 mode's
+    for g, g32 in zip(grads, out["fp32"][2]):
+        np.testing.assert_allclose(g.numpy(), g32.numpy(), rtol=2e-2, atol=2e-3 * float(g32.abs().max()))
+
+
 def test_oracle_adam_and_callbacks_semantics():
     # Keras Adam, one step from zero state: update = -lr * sign(g) * |g| / (|g| + eps*...) ~ -lr * sign(g)
     ref = model_ref.RefLocator(10, 8, 2, dropout=0.0, seed=1)
