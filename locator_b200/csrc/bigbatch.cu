@@ -543,17 +543,6 @@ int bb_step_end_launch(const BigEndArgs& e, int nc, int loss_rows, int gated, cu
   return 0;
 }
 
-static int bb_sms() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    if (n <= 0) n = 148;
-  }
-  return n;
-}
-
 int bb_stats_launch(const BigGroupArgs& g, cudaStream_t s) {
   LOC_CHECK(g.n >= 1 && g.n <= kMaxGroup, "batch statistics: bad group size");
   int64_t kmax = 0;
@@ -577,7 +566,7 @@ static int bb_l1_backward_cw(const BigArgs& a, float* pq_part, cudaStream_t s) {
                       (size_t)(2 * 4 * kBbThreads + CW) * sizeof(float);
   LOC_CUDA(cudaFuncSetAttribute(k_bb_l1_bwd<CW, TILED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int64_t niter = cdiv(cdiv(a.K, kBbT), kBbWordsPerIter);
-  int64_t by = cdiv((int64_t)bb_sms(), ncg);  // one 512-thread block per SM
+  int64_t by = cdiv((int64_t)sm_count(), ncg);  // one 512-thread block per SM
   if (by > niter) by = niter;
   if (by < 1) by = 1;
   k_bb_l1_bwd<CW, TILED><<<dim3((unsigned)ncg, (unsigned)by), kBbThreads, smem, s>>>(a, pq_part);

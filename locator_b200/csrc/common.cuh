@@ -46,6 +46,17 @@ inline int fail(const char* what, const char* file, int line) {
 
 inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// SMs of the device current at the first call (148 on a B200); launch geometry everywhere derives from this one value.
+inline int sm_count() {
+  static const int n = [] {
+    int dev = 0, v = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
+    return v > 0 ? v : 148;
+  }();
+  return n;
+}
+
 // ---- Keras constants (SURVEY.md Appendix A) ----
 constexpr float kBnEps = 1e-3f;
 constexpr float kBnMom = 0.99f;

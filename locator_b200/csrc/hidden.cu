@@ -777,9 +777,11 @@ int hidden_reslice(const float* small, float* fs, float* bs, int H, int L, int c
   return 0;
 }
 
+int hidden_update_blocks(int H, int L) { return (L - 1) * (H / kUpdRows) + 1; }
+
 int hidden_update_launch(const UpdArgs& a, cudaStream_t s, bool overlap_previous) {
   LOC_CHECK(a.H % kUpdRows == 0 && a.H >= 32 && a.H <= 1024, "hidden update: bad width");
-  const int nblk = (a.L - 1) * (a.H / kUpdRows) + 1;
+  const int nblk = hidden_update_blocks(a.H, a.L);
   // overlap_previous: programmatic dependent launch (see l1_backward_tc) -- the update of a model whose hidden
   // stack finished a slot earlier runs next to another model's first-layer backward
   cudaLaunchConfig_t cfg = {};

@@ -22,7 +22,7 @@
 namespace loc {
 namespace htc {
 
-constexpr int kH = 256, kC = 16, kRB = 8, kCW = 64;
+constexpr int kH = 256, kC = kHidTcCtas, kRB = 8, kCW = 64;
 constexpr int kThreads = 512;
 constexpr int kSlot = kH * kCW * 4;    // 64 KB weight-slice image
 constexpr int kGath = kRB * kH * 4;    // 8 KB gathered B operand: [8 k-atoms][8 rows][128 B]

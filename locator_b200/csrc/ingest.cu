@@ -506,11 +506,9 @@ int loc_site_stats(const int8_t* d_gt, int64_t nvar, int64_t nsamp, int32_t min_
   int64_t blocks = cdiv(nvar, warps_per_block);
   static int wave = 0;  // one resident wave of blocks; the warps loop over the sites
   if (wave == 0) {
-    int dev = 0, sms = 148, per_sm = 4;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    int per_sm = 4;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_site_stats, 256, 0);
-    wave = sms * (per_sm > 0 ? per_sm : 1);
+    wave = sm_count() * (per_sm > 0 ? per_sm : 1);
   }
   if (blocks > wave) blocks = wave;
   k_site_stats<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(d_gt, nvar, nsamp, min_mac, d_n_alleles,

@@ -1130,17 +1130,6 @@ __global__ void __launch_bounds__(B_THREADS, 1) k_l1_bwd_tc(L1Args a, int64_t nt
 // ---------------------------------------------------------------------------------------------
 // Host side
 // ---------------------------------------------------------------------------------------------
-static int g_tc_sms = 0;
-static int tc_sm_count() {
-  if (!g_tc_sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&g_tc_sms, cudaDevAttrMultiProcessorCount, dev);
-    if (g_tc_sms <= 0) g_tc_sms = 148;
-  }
-  return g_tc_sms;
-}
-
 bool l1_tc_supported(int64_t K, int H) {
   if (H != tc::kH || K < 1) return false;
   int dev = 0, major = 0;
@@ -1151,7 +1140,7 @@ bool l1_tc_supported(int64_t K, int H) {
 
 int l1_tc_partials(int64_t K) {
   const int64_t ntiles = cdiv(K, tc::B_NT);
-  return (int)(ntiles < tc_sm_count() ? ntiles : tc_sm_count());
+  return (int)(ntiles < sm_count() ? ntiles : sm_count());
 }
 
 int l1_forward_tc(const L1Args& a, int n_partials, cudaStream_t s) {
@@ -1186,13 +1175,15 @@ int l1_backward_tc(const L1Args& a, int nblocks, cudaStream_t s, bool overlap_pr
     attr_set = true;
   }
   const int64_t ntiles = cdiv(a.K, tc::B_NT);
-  int64_t grid = ntiles < tc_sm_count() ? ntiles : tc_sm_count();
-  if (nblocks > 0 && nblocks < grid) grid = nblocks;  // loc_model_set_l1_ctas: leave SMs to a concurrent hidden stack
+  // exactly nblocks CTAs: the caller's mirror of DevState::bwd_cnt counts them (fewer than SMs: loc_model_set_l1_ctas
+  // leaves SMs to a concurrent hidden stack)
+  LOC_CHECK(nblocks >= 1 && nblocks <= ntiles && nblocks <= sm_count(),
+            "first-layer backward: CTA count must be in [1, min(tiles, SMs)]");
   // overlap_previous: programmatic dependent launch -- the kernel starts once every CTA of the previous
   // kernel in the stream is running (it never waits for that kernel's results: the ring schedule puts
   // another model's hidden stack there), instead of after its completion
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
+  cfg.gridDim = dim3((unsigned)nblocks);
   cfg.blockDim = dim3(tc::B_THREADS);
   cfg.dynamicSmemBytes = tc::B_SMEM;
   cfg.stream = s;

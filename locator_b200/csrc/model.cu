@@ -162,17 +162,6 @@ __global__ void __launch_bounds__(256) k_copy_segs(CopySegs cs, const int* cond)
   }
 }
 
-static int g_sm_count = 0;
-static int sm_count() {
-  if (!g_sm_count) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&g_sm_count, cudaDevAttrMultiProcessorCount, dev);
-    if (g_sm_count <= 0) g_sm_count = 148;
-  }
-  return g_sm_count;
-}
-
 static int fill(float* p, int64_t n, float v, cudaStream_t s) {
   if (n <= 0) return 0;
   int64_t blocks = cdiv(n, 256 * 8);
@@ -356,6 +345,40 @@ static UpdArgs upd_args(loc_model* m, int nb, int gated) {
   return u;
 }
 
+// Rows [off, off + nb) of a batch order.  epoch_stride != 0: the order holds one such row per epoch and the
+// device-side epoch counter picks it (row_of).
+static RowSrc order_rows(const int32_t* order, int64_t epoch_stride, int64_t off, int64_t nb) {
+  return RowSrc{order, epoch_stride, off, 0, (int32_t)nb};
+}
+
+// Rows row0 .. row0 + nb - 1 of the bound matrix (validation / predict).
+static RowSrc consecutive_rows(int64_t row0, int64_t nb) { return RowSrc{nullptr, 0, 0, (int32_t)row0, (int32_t)nb}; }
+
+// The training step that starts at row `off` of a batch order: batch_size rows, fewer at the end of the epoch.
+static RowSrc step_rows(const loc_model* m, const int32_t* order, int64_t epoch_stride, int64_t off) {
+  return order_rows(order, epoch_stride, off, m->n_train - off < m->B ? m->n_train - off : m->B);
+}
+
+// 32-row chunk c of a step or of a wide inference pass.
+static RowSrc chunk_rows(RowSrc src, int c) {
+  if (src.rows != nullptr)
+    src.offset += (int64_t)kMaxB * c;
+  else
+    src.row0 += kMaxB * c;
+  src.nb = src.nb - kMaxB * c < kMaxB ? src.nb - kMaxB * c : kMaxB;
+  return src;
+}
+
+// Chunk c of the nc chunks of a wide pass: its Z1 rows start at row 32 c of the pass's split-K tiles in m->wide, and
+// its outputs go to the chunk's block of m->outs.
+static void wide_chunk(const loc_model* m, HidArgs& h, int nc, int c) {
+  h.partials = m->wide;
+  h.n_partials = m->n_partials;
+  h.partial_stride = (int64_t)nc * kMaxB * m->H;
+  h.partial_row0 = kMaxB * c;
+  h.outs = m->outs + c * 256;
+}
+
 // A training launch of the hidden stack advances the step parity (tile walk direction of the backward) and the
 // hand-over flag it publishes when it is done; call right before the launch.
 static void begin_training_hidden(loc_model* m, HidArgs& h) {
@@ -363,8 +386,15 @@ static void begin_training_hidden(loc_model* m, HidArgs& h) {
   h.hid_seq = ++m->h_hid_seq;
 }
 
-// First-layer backward of the tcgen05 path + the host mirror of the counter its CTAs bump when they are done.
-static int backward_tc(loc_model* m, L1Args& a, cudaStream_t s, bool overlap_previous = false) {
+// One model's hidden stack on its family's kernel.  overlap_previous (tcgen05 only): programmatic dependent launch.
+static int hidden_stack(const loc_model* m, const HidArgs& h, cudaStream_t s, bool overlap_previous = false) {
+  return m->hid_tc ? hidden_tc_launch(h, s, overlap_previous) : hidden_launch(h, m->cluster, s);
+}
+
+// First-layer backward + Adam; on the tcgen05 path also the host mirror of the counter its CTAs bump when they are
+// done (l1_backward_tc launches exactly n_bwd_blocks of them).
+static int backward_l1(loc_model* m, L1Args& a, cudaStream_t s, bool overlap_previous = false) {
+  if (!m->use_tc) return l1_backward_simt(a, m->n_bwd_blocks, s);
   a.rev = (int)(m->h_steps & 1);
   if (l1_backward_tc(a, m->n_bwd_blocks, s, overlap_previous)) return 1;
   m->h_bwd_cnt += (unsigned)m->n_bwd_blocks;
@@ -374,7 +404,25 @@ static int backward_tc(loc_model* m, L1Args& a, cudaStream_t s, bool overlap_pre
 // Small-layer update + the host mirror of the counter its blocks bump when they are done.
 static int update_launch(loc_model* m, const UpdArgs& u, cudaStream_t s, bool overlap_previous = false) {
   if (hidden_update_launch(u, s, overlap_previous)) return 1;
-  m->h_upd_cnt += (unsigned)((m->L - 1) * (m->H / 16) + 1);
+  m->h_upd_cnt += (unsigned)hidden_update_blocks(m->H, m->L);
+  return 0;
+}
+
+// The small-layer updates of models ms[0..n) beside their first-layer backwards: each on its model's side stream,
+// behind the event ms[0]->ev_hid records now on `s` (after the hidden-stack launch that holds the n models).
+// update(i, stream) launches model i's update; join_updates makes `s` wait for all of them.
+template <class Update>
+static int fork_updates(loc_model* const* ms, int n, cudaStream_t s, Update update) {
+  LOC_CUDA(cudaEventRecord(ms[0]->ev_hid, s));
+  for (int i = 0; i < n; ++i) {
+    LOC_CUDA(cudaStreamWaitEvent(ms[i]->side, ms[0]->ev_hid, 0));
+    if (update(i, ms[i]->side)) return 1;
+    LOC_CUDA(cudaEventRecord(ms[i]->ev_upd, ms[i]->side));
+  }
+  return 0;
+}
+static int join_updates(loc_model* const* ms, int n, cudaStream_t s) {
+  for (int i = 0; i < n; ++i) LOC_CUDA(cudaStreamWaitEvent(s, ms[i]->ev_upd, 0));
   return 0;
 }
 
@@ -472,16 +520,10 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
     hg.n = 0;
     for (int g = g0; g < g1; ++g) {
       loc_model* m = ms[g];
-      const RowSrc& src = srcs[g];
       const int64_t chunk_stride = (int64_t)m->L * kMaxB * m->H;
       const int first = hg.n;
       for (int c = 0; c < nc; ++c) {
-        RowSrc sc = src;
-        if (src.rows != nullptr)
-          sc.offset = src.offset + (int64_t)kMaxB * c;
-        else
-          sc.row0 = src.row0 + kMaxB * c;
-        sc.nb = nb - kMaxB * c < kMaxB ? nb - kMaxB * c : kMaxB;
+        const RowSrc sc = chunk_rows(srcs[g], c);
         if (!wide) {
           L1Args a = l1_args(m, m->train_packed, m->train_row_words, sc, 0, gated);
           a.mmean = m->bb_mean;
@@ -489,15 +531,12 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
           if (forward_l1(m, a, s)) return 1;
         }
         HidArgs h = hid_args(m, sc, 1, gated, m->train_locs, nullptr);
-        if (wide) {
-          h.partials = m->wide;
-          h.n_partials = m->n_partials;
-          h.partial_stride = (int64_t)nc * kMaxB * m->H;
-          h.partial_row0 = kMaxB * c;
-        }
+        if (wide)
+          wide_chunk(m, h, nc, c);
+        else
+          h.outs = m->outs + c * 256;
         h.acts = m->acts + c * chunk_stride;
         h.dzs = m->dzs + c * chunk_stride;
-        h.outs = m->outs + c * 256;
         h.loss_rows = nb;
         h.row_base = kMaxB * c;
         h.mask_rows = kMaxB * m->cap_chunks;
@@ -509,20 +548,14 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
           hg.a[hg.n++] = h;
           continue;
         }
-        if (m->hid_tc ? hidden_tc_launch(h, s) : hidden_launch(h, m->cluster, s)) return 1;
+        if (hidden_stack(m, h, s)) return 1;
       }
       for (int i = first; i < hg.n; ++i) hg.a[i].hid_seq = m->h_hid_seq;  // published concurrently: the same (final) value
     }
     if (side_by_side && hidden_tc_group_launch(hg, s)) return 1;
-    if (fork) {
-      LOC_CUDA(cudaEventRecord(ms[g0]->ev_hid, s));
-      for (int g = g0; g < g1; ++g) {
-        loc_model* m = ms[g];
-        LOC_CUDA(cudaStreamWaitEvent(m->side, ms[g0]->ev_hid, 0));
-        if (bb_hidden_update_launch(bg.a[g], m->side)) return 1;
-        LOC_CUDA(cudaEventRecord(m->ev_upd, m->side));
-      }
-    }
+    if (fork && fork_updates(ms + g0, g1 - g0, s,
+                             [&](int i, cudaStream_t su) { return bb_hidden_update_launch(bg.a[g0 + i], su); }))
+      return 1;
   }
   if (side_by_side) {
     BigEndArgs e;
@@ -536,11 +569,10 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
   for (int g = 0; g < n; ++g)
     if (bb_l1_backward_launch(bg.a[g], ms[g]->bb_pq, s)) return 1;
   if (!fork) return bb_hidden_update_launch(bg.a[0], s);
-  for (int g = 0; g < n; ++g) LOC_CUDA(cudaStreamWaitEvent(s, ms[g]->ev_upd, 0));
-  return 0;
+  return join_updates(ms, n, s);
 }
 
-// One optimizer step: 3-4 launches (stage_mask selects a subset for profiling / tests).
+// One optimizer step: 3-4 launches.
 // `next` (tcgen05 path): rows of the following step -- the backward kernel then also runs that step's
 // first-layer forward on the W1 chunks it has just updated (they are still in shared memory), so the
 // following step is called with have_fwd = true and skips its own forward launch.
@@ -560,28 +592,23 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
 //     fused forward left -- not for B's completion as a grid (griddepcontrol.wait), which comes microseconds later.
 // Kernel boundaries (drain + launch + ramp: 6-15 us each on this part, `scripts/timeline.py`) disappear from the
 // step's critical path; what remains is H + B plus the flags' latency.
-static int train_step(loc_model* m, const RowSrc& src, int gated, cudaStream_t s, int stage_mask = 15,
-                      const RowSrc* next = nullptr, bool have_fwd = false) {
-  if (m->B > kMaxB) {
-    LOC_CHECK(stage_mask == 15, "single stages of a step are only available for batch_size <= 32");
-    return train_step_big(&m, &src, 1, gated, s);
-  }
+static int train_step(loc_model* m, const RowSrc& src, int gated, cudaStream_t s, const RowSrc* next = nullptr,
+                      bool have_fwd = false) {
+  if (m->B > kMaxB) return train_step_big(&m, &src, 1, gated, s);
   L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, gated);
   if (next != nullptr && m->use_tc) {
     a.src_next = *next;
     a.fuse_next = 1;
   }
-  const bool chain = stage_mask == 15 && chain_capable(m);
+  const bool chain = chain_capable(m);
   const bool h_overlaps = chain && have_fwd && m->chain_open && m->chain_stream == s;  // the stream's last kernels: this model's B, U
   m->chain_open = 0;
-  if ((stage_mask & 1) && !have_fwd && (forward_l1(m, a, s) || exchange_partials(m, s))) return 1;
+  if (!have_fwd && (forward_l1(m, a, s) || exchange_partials(m, s))) return 1;
   HidArgs h = hid_args(m, src, 1, gated, m->train_locs, nullptr);
-  if (stage_mask & 2) {
-    begin_training_hidden(m, h);
-    if (h_overlaps) h.wait_bwd = m->h_bwd_cnt;  // every CTA of the previous step's backward has signed off
-    if (chain) h.wait_upd = m->h_upd_cnt;       // ... and every block of the small-layer updates so far
-    if (m->hid_tc ? hidden_tc_launch(h, s, h_overlaps) : hidden_launch(h, m->cluster, s)) return 1;
-  }
+  begin_training_hidden(m, h);
+  if (h_overlaps) h.wait_bwd = m->h_bwd_cnt;  // every CTA of the previous step's backward has signed off
+  if (chain) h.wait_upd = m->h_upd_cnt;       // ... and every block of the small-layer updates so far
+  if (hidden_stack(m, h, s, h_overlaps)) return 1;
   if (chain) {
     // U goes in FRONT of B: its blocks land on the SMs that idle under the hidden stack and update layer i as soon
     // as the stack's backward chain has produced dz_i (DevState::dz_cnt), so the update is finished a couple of
@@ -589,38 +616,23 @@ static int train_step(loc_model* m, const RowSrc& src, int gated, cudaStream_t s
     // update's blocks leave.
     UpdArgs u = upd_args(m, src.nb, gated);
     u.wait_hid = h.hid_seq;
-    u.wait_dz = 16u * h.hid_seq;  // 16 CTAs of every training hidden stack so far
-    u.wait_upd = m->h_upd_cnt;    // every block of the updates launched so far
+    u.wait_dz = (unsigned)kHidTcCtas * h.hid_seq;  // every CTA of every training hidden stack so far
+    u.wait_upd = m->h_upd_cnt;                     // every block of the updates launched so far
     if (update_launch(m, u, s, true)) return 1;
     a.wait_hid = h.hid_seq;
     a.wait_bwd = m->h_bwd_cnt;  // every backward launched so far for this model
-    if (backward_tc(m, a, s, true)) return 1;
+    if (backward_l1(m, a, s, true)) return 1;
     m->chain_open = 1;
     m->chain_stream = s;
     return 0;
   }
   // Unchained: the small-layer update only needs the hidden kernel's outputs: it runs on a side stream next to
-  // the first-layer backward (full steps only; single-stage debug launches stay on `s`).
-  const bool fork = stage_mask == 15;
-  if (fork) {
-    LOC_CUDA(cudaEventRecord(m->ev_hid, s));
-    LOC_CUDA(cudaStreamWaitEvent(m->side, m->ev_hid, 0));
-  }
-  cudaStream_t su = fork ? m->side : s;
-  auto backward = [&]() -> int {
-    return m->use_tc ? backward_tc(m, a, s) : l1_backward_simt(a, m->n_bwd_blocks, s);
-  };
-  if (!(stage_mask & 8)) {
-    if ((stage_mask & 4) && backward()) return 1;
-    return 0;
-  }
-  UpdArgs u = upd_args(m, src.nb, gated);
-  if (update_launch(m, u, su)) return 1;
-  if (fork) LOC_CUDA(cudaEventRecord(m->ev_upd, m->side));
-  if ((stage_mask & 4) && backward()) return 1;
-  if ((stage_mask & 4) && a.fuse_next && exchange_partials(m, s)) return 1;  // the next step's tile is complete
-  if (fork) LOC_CUDA(cudaStreamWaitEvent(s, m->ev_upd, 0));
-  return 0;
+  // the first-layer backward.
+  const UpdArgs u = upd_args(m, src.nb, gated);
+  if (fork_updates(&m, 1, s, [&](int, cudaStream_t su) { return update_launch(m, u, su); })) return 1;
+  if (backward_l1(m, a, s)) return 1;
+  if (a.fuse_next && exchange_partials(m, s)) return 1;  // the next step's tile is complete
+  return join_updates(&m, 1, s);
 }
 
 // Inference-mode forward over n rows (Keras predict / evaluate at batch 32: locator.py:374,414,441).
@@ -639,26 +651,14 @@ static int infer_rows(loc_model* m, const uint32_t* packed, int64_t n, int64_t r
     for (int64_t r0 = 0; r0 < n; r0 += 256) {
       const int nrows = (int)((n - r0) < 256 ? (n - r0) : 256);
       const int nc = (nrows + 31) / 32;
-      RowSrc src;
-      src.rows = nullptr;
-      src.epoch_stride = 0;
-      src.offset = 0;
-      src.row0 = (int32_t)r0;
-      src.nb = nrows;
+      const RowSrc src = consecutive_rows(r0, nrows);
       L1Args a = l1_args(m, packed, row_words, src, 0, gated);
       if (l1_forward_wide_tc(a, m->n_partials, nrows, m->wide, s)) return 1;
       HidGroupArgs hg;
       hg.n = nc;
       for (int c = 0; c < nc; ++c) {
-        RowSrc sc = src;
-        sc.row0 = (int32_t)(r0 + 32 * c);
-        sc.nb = nrows - 32 * c < kMaxB ? nrows - 32 * c : kMaxB;
-        HidArgs h = hid_args(m, sc, 0, gated, locs, pred_out);
-        h.partials = m->wide;
-        h.n_partials = m->n_partials;
-        h.partial_stride = (int64_t)nc * 32 * m->H;
-        h.partial_row0 = 32 * c;
-        h.outs = m->outs + c * 256;
+        HidArgs h = hid_args(m, chunk_rows(src, c), 0, gated, locs, pred_out);
+        wide_chunk(m, h, nc, c);
         h.val_slot = locs != nullptr ? m->val_slots + 2 * c : nullptr;
         hg.a[c] = h;
       }
@@ -671,16 +671,10 @@ static int infer_rows(loc_model* m, const uint32_t* packed, int64_t n, int64_t r
     return 0;
   }
   for (int64_t r0 = 0; r0 < n; r0 += kMaxB) {
-    RowSrc src;
-    src.rows = nullptr;
-    src.epoch_stride = 0;
-    src.offset = 0;
-    src.row0 = (int32_t)r0;
-    src.nb = (int32_t)((n - r0) < kMaxB ? (n - r0) : kMaxB);
+    const RowSrc src = consecutive_rows(r0, (n - r0) < kMaxB ? (n - r0) : kMaxB);
     L1Args a = l1_args(m, packed, row_words, src, 0, gated);
     if (forward_l1(m, a, s) || exchange_partials(m, s)) return 1;
-    HidArgs h = hid_args(m, src, 0, gated, locs, pred_out);
-    if (m->hid_tc ? hidden_tc_launch(h, s) : hidden_launch(h, m->cluster, s)) return 1;
+    if (hidden_stack(m, hid_args(m, src, 0, gated, locs, pred_out), s)) return 1;
   }
   return 0;
 }
@@ -1178,28 +1172,44 @@ int loc_train_step(loc_model* m, const int32_t* d_rows, int32_t nb, void* stream
   LOC_CHECK(m != nullptr && m->train_packed != nullptr, "loc_train_step: no training data bound");
   LOC_CHECK(d_rows != nullptr && nb >= 1 && nb <= m->B, "loc_train_step: bad batch");
   m->span_perm = nullptr;
-  RowSrc src;
-  src.rows = d_rows;
-  src.epoch_stride = 0;
-  src.offset = 0;
-  src.row0 = 0;
-  src.nb = nb;
-  return train_step(m, src, 0, (cudaStream_t)stream);
+  return train_step(m, order_rows(d_rows, 0, 0, nb), 0, (cudaStream_t)stream);
 }
 
 int loc_debug_stage(loc_model* m, int32_t stage, const int32_t* d_rows, int32_t nb, void* stream) {
   LOC_CHECK(m != nullptr && m->train_packed != nullptr, "loc_debug_stage: no training data bound");
   LOC_CHECK(stage >= 0 && stage < 5 && d_rows != nullptr && nb >= 1 && nb <= m->B, "loc_debug_stage: bad arguments");
   LOC_CHECK(m->B <= kMaxB, "loc_debug_stage: single stages are only available for batch_size <= 32");
+  cudaStream_t s = (cudaStream_t)stream;
   m->span_perm = nullptr;
-  RowSrc src;
-  src.rows = d_rows;
-  src.epoch_stride = 0;
-  src.offset = 0;
-  src.row0 = 0;
-  src.nb = nb;
-  if (stage == 4) return train_step(m, src, 0, (cudaStream_t)stream, 4, &src);  // backward + fused next forward
-  return train_step(m, src, 0, (cudaStream_t)stream, 1 << stage);
+  m->chain_open = 0;
+  const RowSrc src = order_rows(d_rows, 0, 0, nb);
+  L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 0);
+  switch (stage) {
+    case 0:  // first-layer forward (+ the shard exchange)
+      return forward_l1(m, a, s) || exchange_partials(m, s);
+    case 1: {  // training hidden stack
+      HidArgs h = hid_args(m, src, 1, 0, m->train_locs, nullptr);
+      begin_training_hidden(m, h);
+      return hidden_stack(m, h, s);
+    }
+    case 2:  // first-layer backward + Adam
+      return backward_l1(m, a, s);
+    case 3:  // small-layer update
+      return update_launch(m, upd_args(m, nb, 0), s);
+    default:  // 4: first-layer backward + Adam with the next forward (same rows) fused in on the tcgen05 path
+      if (m->use_tc) {
+        a.src_next = src;
+        a.fuse_next = 1;
+      }
+      return backward_l1(m, a, s);
+  }
+}
+
+static int end_epoch(loc_model* m, cudaStream_t s) {
+  if (infer_rows(m, m->val_packed, m->n_val, m->val_row_words, m->val_locs, nullptr, 1, s)) return 1;
+  k_epoch_end<<<1, 1, 0, s>>>(m->st, m->hist);
+  LOC_LAUNCHED();
+  return copy_weights(m, true, &m->st->improved, s);
 }
 
 // below this many SNPs the first-layer backward is shorter than the hidden stack (42 us ~ 35k SNPs)
@@ -1226,15 +1236,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
     k_begin_call<<<1, 1, 0, s>>>(models[g]->st);
     LOC_LAUNCHED();
   }
-  auto step_rows = [&](int g, int64_t off) {
-    RowSrc src;
-    src.rows = d_perms[g];
-    src.epoch_stride = m0->n_train;
-    src.offset = off;
-    src.row0 = 0;
-    src.nb = (int32_t)((m0->n_train - off) < m0->B ? (m0->n_train - off) : m0->B);
-    return src;
-  };
+  auto rows = [&](int g, int64_t off) { return step_rows(models[g], d_perms[g], m0->n_train, off); };
   // Schedule.  "ring" (default whenever every model's first-layer kernels leave one cluster's worth of SMs
   // free, loc_model_set_l1_ctas): one stream, per slot  H(g) -> B(g-1) -> U(g-1)  where H is the 16-CTA hidden
   // stack of model g (plain launch: starts when everything before it is complete), B the first-layer backward
@@ -1251,7 +1253,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
   const bool big = m0->B > kMaxB;
   const char* sched = getenv("LOC_GROUP_SCHEDULE");  // "ring" / "lockstep" override the choice by K (tests, A/B)
   bool ring = !big && n_models >= 2 && (m0->K >= kRingMinK || (sched != nullptr && strcmp(sched, "ring") == 0));
-  for (int g = 0; g < n_models; ++g) ring = ring && models[g]->n_bwd_blocks <= sm_count() - 16;
+  for (int g = 0; g < n_models; ++g) ring = ring && models[g]->n_bwd_blocks <= sm_count() - kHidTcCtas;
   if (sched != nullptr && strcmp(sched, "lockstep") == 0) ring = false;
   struct Pending {
     loc_model* m;
@@ -1279,24 +1281,24 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
           pend.a.wait_hid = pend.hid_seq;
           pend.a.wait_bwd = pend.m->h_bwd_cnt;
           pend.u.wait_hid = pend.hid_seq;
-          if (backward_tc(pend.m, pend.a, s, overlap)) return 1;
+          if (backward_l1(pend.m, pend.a, s, overlap)) return 1;
           return update_launch(pend.m, pend.u, s, overlap);
         };
         for (int64_t off = 0; off < m0->n_train; off += m0->B) {
           const bool has_next = off + m0->B < m0->n_train;
           for (int g = g0; g < g1; ++g) {
             loc_model* m = models[g];
-            const RowSrc src = step_rows(g, off);
+            const RowSrc src = rows(g, off);
             L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 1);
             if (!have_fwd && forward_l1(m, a, s)) return 1;  // first step of the epoch: later ones are fused
             HidArgs h = hid_args(m, src, 1, 1, m->train_locs, nullptr);
             begin_training_hidden(m, h);
             const bool h_overlaps = chain2 && have_fwd;  // directly behind this model's own backward + update
             if (h_overlaps) h.wait_bwd = m->h_bwd_cnt;
-            if (hidden_tc_launch(h, s, h_overlaps)) return 1;
+            if (hidden_stack(m, h, s, h_overlaps)) return 1;
             if (pend.m != nullptr && launch_pending(true)) return 1;
             if (has_next) {
-              a.src_next = step_rows(g, off + m0->B);
+              a.src_next = rows(g, off + m0->B);
               a.fuse_next = 1;
             }
             pend.m = m;
@@ -1312,7 +1314,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
     }
     for (int64_t off = 0; big && off < m0->n_train; off += m0->B) {
       RowSrc srcs[kMaxGroup];
-      for (int g = 0; g < n_models; ++g) srcs[g] = step_rows(g, off);
+      for (int g = 0; g < n_models; ++g) srcs[g] = rows(g, off);
       if (train_step_big(models, srcs, n_models, 1, s)) return 1;
     }
     bool have_fwd = false;
@@ -1323,7 +1325,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
       // first-layer forwards (first step of the epoch only: later ones are fused into the backward)
       for (int g = 0; g < n_models; ++g) {
         loc_model* m = models[g];
-        const RowSrc src = step_rows(g, off);
+        const RowSrc src = rows(g, off);
         if (!have_fwd) {
           L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 1);
           if (forward_l1(m, a, s)) return 1;
@@ -1334,34 +1336,25 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
       // all hidden stacks in one launch: one cluster per replicate
       if (hidden_tc_group_launch(hg, s)) return 1;
       // small-layer updates on the side streams, first-layer backward (+ next forward) back to back
-      LOC_CUDA(cudaEventRecord(m0->ev_hid, s));
+      if (fork_updates(models, n_models, s, [&](int g, cudaStream_t su) {
+            return update_launch(models[g], upd_args(models[g], hg.a[g].src.nb, 1), su);
+          }))
+        return 1;
       for (int g = 0; g < n_models; ++g) {
         loc_model* m = models[g];
-        LOC_CUDA(cudaStreamWaitEvent(m->side, m0->ev_hid, 0));
-        UpdArgs u = upd_args(m, hg.a[g].src.nb, 1);
-        if (update_launch(m, u, m->side)) return 1;
-        LOC_CUDA(cudaEventRecord(m->ev_upd, m->side));
-      }
-      for (int g = 0; g < n_models; ++g) {
-        loc_model* m = models[g];
-        const RowSrc src = step_rows(g, off);
+        const RowSrc src = rows(g, off);
         L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 1);
         if (has_next) {
-          a.src_next = step_rows(g, off + m0->B);
+          a.src_next = rows(g, off + m0->B);
           a.fuse_next = 1;
         }
-        if (backward_tc(m, a, s)) return 1;
+        if (backward_l1(m, a, s)) return 1;
       }
-      for (int g = 0; g < n_models; ++g) LOC_CUDA(cudaStreamWaitEvent(s, models[g]->ev_upd, 0));
+      if (join_updates(models, n_models, s)) return 1;
       have_fwd = has_next;
     }
-    for (int g = 0; g < n_models; ++g) {
-      loc_model* m = models[g];
-      if (infer_rows(m, m->val_packed, m->n_val, m->val_row_words, m->val_locs, nullptr, 1, s)) return 1;
-      k_epoch_end<<<1, 1, 0, s>>>(m->st, m->hist);
-      LOC_LAUNCHED();
-      if (copy_weights(m, true, &m->st->improved, s)) return 1;
-    }
+    for (int g = 0; g < n_models; ++g)
+      if (end_epoch(models[g], s)) return 1;
   }
   return 0;
 }
@@ -1413,31 +1406,15 @@ int64_t loc_debug_read(loc_model* m, int32_t which, float* h_dst, int64_t max_n,
 static int run_span(loc_model* m, const int32_t* perm, int64_t epoch_stride, int64_t step0, int64_t nsteps, int gated,
                     bool* have_fwd, cudaStream_t s) {
   const bool fuse = m->use_tc && m->B <= kMaxB;
-  auto step_rows = [&](int64_t off) {
-    RowSrc src;
-    src.rows = perm;
-    src.epoch_stride = epoch_stride;
-    src.offset = off;
-    src.row0 = 0;
-    src.nb = (int32_t)((m->n_train - off) < m->B ? (m->n_train - off) : m->B);
-    return src;
-  };
   for (int64_t st = step0; st < step0 + nsteps; ++st) {
     const int64_t off = st * m->B;
-    const RowSrc src = step_rows(off);
+    const RowSrc src = step_rows(m, perm, epoch_stride, off);
     const bool has_next = fuse && off + m->B < m->n_train;  // within the epoch (the validation pass reuses the tiles)
-    const RowSrc next = has_next ? step_rows(off + m->B) : src;
-    if (train_step(m, src, gated, s, 15, has_next ? &next : nullptr, *have_fwd)) return 1;
+    const RowSrc next = has_next ? step_rows(m, perm, epoch_stride, off + m->B) : src;
+    if (train_step(m, src, gated, s, has_next ? &next : nullptr, *have_fwd)) return 1;
     *have_fwd = has_next;
   }
   return 0;
-}
-
-static int end_epoch(loc_model* m, cudaStream_t s) {
-  if (infer_rows(m, m->val_packed, m->n_val, m->val_row_words, m->val_locs, nullptr, 1, s)) return 1;
-  k_epoch_end<<<1, 1, 0, s>>>(m->st, m->hist);
-  LOC_LAUNCHED();
-  return copy_weights(m, true, &m->st->improved, s);
 }
 
 int loc_train_epochs(loc_model* m, const int32_t* d_perms, int32_t n_epochs, void* stream) {

@@ -158,13 +158,15 @@ int l1_forward_simt(const L1Args& a, int n_partials, cudaStream_t s);
 int l1_backward_simt(const L1Args& a, int nblocks, cudaStream_t s);
 int hidden_launch(const HidArgs& a, int cluster, cudaStream_t s);
 int hidden_update_launch(const UpdArgs& a, cudaStream_t s, bool overlap_previous = false);
+int hidden_update_blocks(int H, int L);  // blocks of one hidden_update_launch (each bumps DevState::upd_cnt once)
 int hidden_max_cluster(int H, int L);  // largest usable cluster size (16, 8, ...) for this device
 int hidden_slots(int H, int L, int cluster);
 int hidden_max_nlayers(int H);  // deepest L in [2, 64] with a slot at some cluster size (host arithmetic), 0 = none
 int hidden_reslice(const float* small, float* fs, float* bs, int H, int L, int cluster, cudaStream_t s);
 size_t hidden_smem_bytes(int H, int L, int cluster);
 
-// tcgen05 hidden stack (hidden_tc.cu): width 256, 16-CTA cluster
+// tcgen05 hidden stack (hidden_tc.cu): width 256, one cluster of kHidTcCtas CTAs per model (and SMs: one CTA per SM)
+constexpr int kHidTcCtas = 16;
 bool hidden_tc_supported(int H, int L);
 int hidden_tc_launch(const HidArgs& a, cudaStream_t s, bool overlap_previous = false);
 int hidden_tc_group_launch(const HidGroupArgs& g, cudaStream_t s);
