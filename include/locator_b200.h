@@ -294,19 +294,23 @@ int loc_train_steps(loc_model* m, const int32_t* d_perm, int32_t step0, int32_t 
 
 /* Replicate group (bootstrap / window models trained side by side on one GPU, locator.py:519-583 and
  * :609-681 run them one after the other): the same as loc_train_epochs for n_models <= 8 independent models.
- * Models must share nlayers, batch size and training-set size (true for the replicates of one run);
- * d_perms[g] is model g's batch order.  Every model ends bit-identical to the same model trained alone.
- * Two schedules:
- *   ring     (models of >= 32768 SNPs whose first-layer kernels leave 16 SMs free, loc_model_set_l1_ctas):
- *            the hidden stack of one model runs concurrently with the first-layer backward + Adam of the
- *            previous model of its ring (programmatic dependent launch inside one stream);
- *   lockstep (otherwise): the hidden stacks of all models share one launch (one cluster per model), the
- *            first-layer kernels run back to back.
- * Environment LOC_GROUP_SCHEDULE=ring|lockstep overrides the choice by size.
+ * Models must share width, nlayers, batch size and training-set size (true for the replicates of one run)
+ * and one kernel family: all tcgen05 (width 256, nlayers <= 14) or all CUDA-core (other widths).  Width 256
+ * with 15..21 layers (tcgen05 first layer, CUDA-core hidden stack) and groups mixing families are refused:
+ * such models train one at a time.  d_perms[g] is model g's batch order.  Every model ends bit-identical to
+ * the same model trained alone.  Two schedules:
+ *   ring     (tcgen05 models of >= 32768 SNPs whose first-layer kernels leave 16 SMs free,
+ *            loc_model_set_l1_ctas): the hidden stack of one model runs concurrently with the first-layer
+ *            backward + Adam of the previous model of its ring (programmatic dependent launch inside one stream);
+ *   lockstep (otherwise, and always for CUDA-core models): the hidden stacks of all models share one launch
+ *            (one cluster per model), the first-layer kernels run back to back.
+ * Environment LOC_GROUP_SCHEDULE=ring|lockstep overrides the choice by size for tcgen05 models.
  * Models of batch_size > 32 have a third schedule, whatever LOC_GROUP_SCHEDULE says: per step, the batch
- * statistics of all models in one launch, each model's wide first-layer forward, the 32-row chunks of whole
- * models packed into shared hidden-stack launches (floor(8 / chunks) models per launch), one step end for
- * all models, then the first-layer backwards back to back while the small-layer updates run on side streams. */
+ * statistics of all models in one launch; on tcgen05 each model's wide first-layer forward, the 32-row chunks
+ * of whole models packed into shared hidden-stack launches (floor(8 / chunks) models per launch) and one step
+ * end for all models; on CUDA cores, chunk by chunk, every model's first-layer forward and then that chunk of
+ * every model in one hidden-stack launch; then the first-layer backwards back to back while the small-layer
+ * updates run on side streams. */
 int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* const* d_perms, int32_t n_epochs,
                            void* stream);
 

@@ -34,6 +34,11 @@ __device__ __forceinline__ unsigned cluster_size() {
   asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
   return r;
 }
+__device__ __forceinline__ unsigned cluster_id() {
+  unsigned r;
+  asm volatile("mov.u32 %0, %%clusterid.x;" : "=r"(r));
+  return r;
+}
 // Release/acquire at cluster scope: (distributed) shared-memory and global writes made before it by
 // any CTA of the cluster are visible to every CTA after it.
 __device__ __forceinline__ void cluster_barrier() {
@@ -130,8 +135,13 @@ __device__ __noinline__ void slice_matmul(const float* gathered, const float* Ws
 
 // TH / THc: compile-time width and slice width (0 = take them from the arguments): the common
 // 256-wide, 16-CTA configuration gets shift-and-mask index arithmetic and fully unrolled loops.
+// One launch runs g.n independent models (a single model is a group of one): cluster c runs model c with
+// g.a[c], exactly as a launch of that model alone would.  Every model-specific location -- DevState, dropout
+// stream, masks, partial tiles, acts / dzs / outs, dbg -- comes from g.a[c], and the CTA's place
+// inside its model is its cluster rank, so clusters never touch each other's data or wait on each other.
 template <int TH, int THc>
-__global__ void __launch_bounds__(kHidThreads, 1) k_hidden(HidArgs a) {
+__global__ void __launch_bounds__(kHidThreads, 1) k_hidden(HidGroupArgs g) {
+  const HidArgs& a = g.a[cluster_id()];
   if (a.gated && a.st->stopped) return;
   extern __shared__ __align__(16) float smem[];
   __shared__ int64_t s_rows[kMaxB];
@@ -698,14 +708,16 @@ size_t hidden_smem_bytes(int H, int L, int cluster) {
   return hidden_fixed_floats(H, L, cluster) * sizeof(float) + (size_t)ns * H * (H / cluster) * sizeof(float);
 }
 
-typedef void (*hidden_fn)(HidArgs);
+typedef void (*hidden_fn)(HidGroupArgs);
 static hidden_fn hidden_kernel(int H, int cluster) {
   return (H == 256 && cluster == 16) ? k_hidden<256, 16> : k_hidden<0, 0>;
 }
 
-static int launch_hidden_cluster(const HidArgs& a, int cluster, cudaStream_t s, bool dry) {
+// One cluster of `cluster` CTAs per model of the group.  The clusters need not be co-resident: none waits on another.
+static int launch_hidden_cluster(const HidGroupArgs& g, int cluster, cudaStream_t s, bool dry) {
+  const HidArgs& a = g.a[0];
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)cluster);
+  cfg.gridDim = dim3((unsigned)(cluster * g.n));
   cfg.blockDim = dim3(kHidThreads);
   cfg.dynamicSmemBytes = hidden_smem_bytes(a.H, a.L, cluster);
   cfg.stream = s;
@@ -725,7 +737,7 @@ static int launch_hidden_cluster(const HidArgs& a, int cluster, cudaStream_t s, 
     }
     return n;
   }
-  LOC_CUDA(cudaLaunchKernelEx(&cfg, hidden_kernel(a.H, cluster), a));
+  LOC_CUDA(cudaLaunchKernelEx(&cfg, hidden_kernel(a.H, cluster), g));
   loc::g_launches.fetch_add(1);
   return 0;
 }
@@ -753,21 +765,34 @@ int hidden_max_cluster(int H, int L) {
       cudaGetLastError();
       continue;
     }
-    HidArgs dummy = {};
-    dummy.H = H;
-    dummy.L = L;
+    HidGroupArgs dummy = {};
+    dummy.n = 1;
+    dummy.a[0].H = H;
+    dummy.a[0].L = L;
     if (launch_hidden_cluster(dummy, c, 0, true) > 0) return c;
   }
   return 0;
 }
 
-int hidden_launch(const HidArgs& a, int cluster, cudaStream_t s) {
+int hidden_group_launch(const HidGroupArgs& g, int cluster, cudaStream_t s) {
+  LOC_CHECK(g.n >= 1 && g.n <= kMaxGroup, "hidden stack group: bad group size");
+  const HidArgs& a = g.a[0];
   LOC_CHECK(cluster > 0 && a.H % (4 * cluster) == 0, "hidden stack: width must be a multiple of 4 x cluster size");
   LOC_CHECK(a.H % 32 == 0, "hidden stack: width must be a multiple of 32");
   LOC_CHECK(a.n_slots >= 1, "hidden stack: shared memory budget exceeded for this width / nlayers");
+  for (int i = 1; i < g.n; ++i)  // one launch has one shared-memory size and one slice geometry
+    LOC_CHECK(g.a[i].H == a.H && g.a[i].L == a.L && g.a[i].n_slots == a.n_slots,
+              "hidden stack group: the models of one launch must share width, nlayers and cluster size");
   const size_t smem = hidden_smem_bytes(a.H, a.L, cluster);
   LOC_CUDA(cudaFuncSetAttribute(hidden_kernel(a.H, cluster), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  return launch_hidden_cluster(a, cluster, s, false);
+  return launch_hidden_cluster(g, cluster, s, false);
+}
+
+int hidden_launch(const HidArgs& a, int cluster, cudaStream_t s) {
+  HidGroupArgs g;
+  g.n = 1;
+  g.a[0] = a;
+  return hidden_group_launch(g, cluster, s);
 }
 
 int hidden_reslice(const float* small, float* fs, float* bs, int H, int L, int cluster, cudaStream_t s) {

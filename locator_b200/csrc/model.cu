@@ -390,6 +390,10 @@ static void begin_training_hidden(loc_model* m, HidArgs& h) {
 static int hidden_stack(const loc_model* m, const HidArgs& h, cudaStream_t s, bool overlap_previous = false) {
   return m->hid_tc ? hidden_tc_launch(h, s, overlap_previous) : hidden_launch(h, m->cluster, s);
 }
+// The hidden stacks of a replicate group in one launch, one cluster each, on the family of m (every model's).
+static int hidden_stacks(const loc_model* m, const HidGroupArgs& g, cudaStream_t s) {
+  return m->hid_tc ? hidden_tc_group_launch(g, s) : hidden_group_launch(g, m->cluster, s);
+}
 
 // First-layer backward + Adam; on the tcgen05 path also the host mirror of the counter its CTAs bump when they are
 // done (l1_backward_tc launches exactly n_bwd_blocks of them).
@@ -476,7 +480,8 @@ static BigArgs big_args(loc_model* m, const RowSrc& src, int gated) {
 //   batch statistics over all rows of every model's step (one launch for the group),
 //   first-layer forward with those statistics (one wide pass over W1 per model on the tcgen05 path),
 //   the step's 32-row chunks through the hidden stack -- tcgen05: side by side, one cluster per chunk, whole models
-//     per grouped launch (floor(8 / chunks) models each), then the step end of all models in one launch,
+//     per grouped launch (floor(8 / chunks) models each), then the step end of all models in one launch; CUDA cores:
+//     chunk by chunk, each after its first-layer forward, in a group chunk c of every model in one launch,
 //   one pass over W1 | m | v per model (dW1 over all rows + Adam), back to back,
 //   the small-layer update over the chunks: after the backward for a single model; in a group on the model's side
 //     stream, forked after the hidden launch that holds its chunks (it runs under the other models' backwards) and
@@ -508,40 +513,62 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
       if (l1_forward_wide_tc(a, m->n_partials, nb, m->wide, s)) return 1;
     }
   }
-  // tcgen05 hidden stack: the chunks run side by side, one cluster each (k_hidden_tc_group); their loss sums and the
-  // step's optimizer bookkeeping follow in k_bb_step_end.  LOC_BB_SERIAL=1 (tests): one launch per chunk.  A model's
-  // chunks never straddle two launches: each publishes DevState::hid_seq once all of the model's chunks are done.
-  const bool side_by_side = wide && nc > 1 && getenv("LOC_BB_SERIAL") == nullptr;
-  const int per_launch = side_by_side ? kMaxGroup / nc : 1;
+  // Chunk c of model g: its first-layer forward into the model's partial tiles (unless the wide pass left them), then
+  // the arguments of its hidden stack.
+  auto chunk = [&](int g, int c, HidArgs& h) -> int {
+    loc_model* m = ms[g];
+    const RowSrc sc = chunk_rows(srcs[g], c);
+    if (!wide) {
+      L1Args a = l1_args(m, m->train_packed, m->train_row_words, sc, 0, gated);
+      a.mmean = m->bb_mean;
+      a.mvar = m->bb_var;
+      if (forward_l1(m, a, s)) return 1;
+    }
+    h = hid_args(m, sc, 1, gated, m->train_locs, nullptr);
+    if (wide)
+      wide_chunk(m, h, nc, c);
+    else
+      h.outs = m->outs + c * 256;
+    const int64_t chunk_stride = (int64_t)m->L * kMaxB * m->H;
+    h.acts = m->acts + c * chunk_stride;
+    h.dzs = m->dzs + c * chunk_stride;
+    h.loss_rows = nb;
+    h.row_base = kMaxB * c;
+    h.mask_rows = kMaxB * m->cap_chunks;
+    h.chunk_flags = (c > 0 ? 1 : 0) | (c < nc - 1 ? 2 : 0);
+    begin_training_hidden(m, h);
+    return 0;
+  };
+  const bool serial = getenv("LOC_BB_SERIAL") != nullptr;  // tests: one hidden launch per chunk and model
   const bool fork = n > 1;
-  for (int g0 = 0; g0 < n; g0 += per_launch) {
+  // tcgen05 hidden stack: the chunks run side by side, one cluster each (k_hidden_tc_group); their loss sums and the
+  // step's optimizer bookkeeping follow in k_bb_step_end.  A model's chunks never straddle two launches: each
+  // publishes DevState::hid_seq once all of the model's chunks are done.
+  const bool side_by_side = wide && nc > 1 && !serial;
+  // CUDA-core hidden stack, a group: chunk by chunk, the forwards of every model, then chunk c of every model in one
+  // k_hidden launch (one cluster per model).  Loss and step bookkeeping stay inside the launch, as for one model.
+  const bool chunk_lockstep = !wide && fork && !ms[0]->hid_tc && !serial;
+  if (chunk_lockstep) {
+    for (int c = 0; c < nc; ++c) {
+      HidGroupArgs hg;
+      hg.n = n;
+      for (int g = 0; g < n; ++g)
+        if (chunk(g, c, hg.a[g])) return 1;
+      if (hidden_stacks(ms[0], hg, s)) return 1;
+    }
+    if (fork_updates(ms, n, s, [&](int i, cudaStream_t su) { return bb_hidden_update_launch(bg.a[i], su); })) return 1;
+  }
+  const int per_launch = side_by_side ? kMaxGroup / nc : 1;
+  for (int g0 = 0; !chunk_lockstep && g0 < n; g0 += per_launch) {
     const int g1 = g0 + per_launch < n ? g0 + per_launch : n;
     HidGroupArgs hg;
     hg.n = 0;
     for (int g = g0; g < g1; ++g) {
       loc_model* m = ms[g];
-      const int64_t chunk_stride = (int64_t)m->L * kMaxB * m->H;
       const int first = hg.n;
       for (int c = 0; c < nc; ++c) {
-        const RowSrc sc = chunk_rows(srcs[g], c);
-        if (!wide) {
-          L1Args a = l1_args(m, m->train_packed, m->train_row_words, sc, 0, gated);
-          a.mmean = m->bb_mean;
-          a.mvar = m->bb_var;
-          if (forward_l1(m, a, s)) return 1;
-        }
-        HidArgs h = hid_args(m, sc, 1, gated, m->train_locs, nullptr);
-        if (wide)
-          wide_chunk(m, h, nc, c);
-        else
-          h.outs = m->outs + c * 256;
-        h.acts = m->acts + c * chunk_stride;
-        h.dzs = m->dzs + c * chunk_stride;
-        h.loss_rows = nb;
-        h.row_base = kMaxB * c;
-        h.mask_rows = kMaxB * m->cap_chunks;
-        h.chunk_flags = (c > 0 ? 1 : 0) | (c < nc - 1 ? 2 : 0);
-        begin_training_hidden(m, h);
+        HidArgs h;
+        if (chunk(g, c, h)) return 1;
         if (side_by_side) {
           h.chunk_flags = 2;  // nobody bumps the step counters inside the launch
           h.val_slot = m->val_slots + 2 * c;
@@ -1224,10 +1251,16 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
     loc_model* m = models[g];
     LOC_CHECK(m != nullptr && d_perms[g] != nullptr && m->train_packed != nullptr && m->val_packed != nullptr,
               "loc_group_train_epochs: every model needs bound training / validation data and a batch order");
-    LOC_CHECK(m->hid_tc && m->use_tc, "loc_group_train_epochs: grouped replicates need the tcgen05 first layer and hidden stack (width 256, nlayers <= 14)");
+    LOC_CHECK(m->use_tc == m->hid_tc,
+              "loc_group_train_epochs: models whose first layer and hidden stack run on different kernel families (width 256 "
+              "with 15..21 layers: tcgen05 first layer, CUDA-core hidden stack) cannot be grouped");
+    LOC_CHECK(m->hid_tc == m0->hid_tc,
+              "loc_group_train_epochs: the models of a group must all run the tcgen05 kernels (width 256, nlayers <= 14) or all "
+              "the CUDA-core kernels");
     LOC_CHECK(m->exchange == nullptr && m->tp == nullptr, "loc_group_train_epochs: sharded models cannot be grouped");
-    LOC_CHECK(m->L == m0->L && m->B == m0->B && m->n_train == m0->n_train,
-              "loc_group_train_epochs: replicates of a group must share nlayers, batch size and training-set size");
+    LOC_CHECK(m->H == m0->H && m->L == m0->L && m->B == m0->B && m->n_train == m0->n_train && m->cluster == m0->cluster,
+              "loc_group_train_epochs: replicates of a group must share width, nlayers, batch size, training-set size and "
+              "hidden-stack cluster size");
   }
   cudaStream_t s = (cudaStream_t)stream;
   for (int g = 0; g < n_models; ++g) {
@@ -1247,12 +1280,16 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
   // max(B, H) instead of B + H / G -- a gain only when the weight stream outlasts the hidden stack, hence
   // K >= kRingMinK.  "lockstep" (small K, models on all SMs, or LOC_GROUP_SCHEDULE=lockstep): all hidden
   // stacks in one launch, then the backwards back to back, updates on side streams.
+  // CUDA-core models (widths other than 256) always run the lockstep, without fused forwards: the CUDA-core
+  // first-layer backward has none, and the ring pays only where the tcgen05 weight stream outlasts the stack
+  // (LOC_GROUP_SCHEDULE does not apply to them).
   // Models of more than 32 rows a step ("large batch", LOC_GROUP_SCHEDULE does not apply): train_step_big with the
-  // whole group, a lockstep of its own -- one statistics launch, hidden stacks packed whole models per launch, one
-  // step end, the backwards back to back, updates on side streams.
+  // whole group, a lockstep of its own -- one statistics launch, hidden stacks packed whole models per launch (tcgen05)
+  // or chunk c of every model per launch (CUDA cores), the backwards back to back, updates on side streams.
   const bool big = m0->B > kMaxB;
+  const bool fuse = m0->use_tc;  // the backward also runs the next step's forward
   const char* sched = getenv("LOC_GROUP_SCHEDULE");  // "ring" / "lockstep" override the choice by K (tests, A/B)
-  bool ring = !big && n_models >= 2 && (m0->K >= kRingMinK || (sched != nullptr && strcmp(sched, "ring") == 0));
+  bool ring = !big && m0->hid_tc && n_models >= 2 && (m0->K >= kRingMinK || (sched != nullptr && strcmp(sched, "ring") == 0));
   for (int g = 0; g < n_models; ++g) ring = ring && models[g]->n_bwd_blocks <= sm_count() - kHidTcCtas;
   if (sched != nullptr && strcmp(sched, "lockstep") == 0) ring = false;
   struct Pending {
@@ -1334,7 +1371,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
         begin_training_hidden(m, hg.a[g]);
       }
       // all hidden stacks in one launch: one cluster per replicate
-      if (hidden_tc_group_launch(hg, s)) return 1;
+      if (hidden_stacks(m0, hg, s)) return 1;
       // small-layer updates on the side streams, first-layer backward (+ next forward) back to back
       if (fork_updates(models, n_models, s, [&](int g, cudaStream_t su) {
             return update_launch(models[g], upd_args(models[g], hg.a[g].src.nb, 1), su);
@@ -1344,14 +1381,14 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
         loc_model* m = models[g];
         const RowSrc src = rows(g, off);
         L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 1);
-        if (has_next) {
+        if (fuse && has_next) {
           a.src_next = rows(g, off + m0->B);
           a.fuse_next = 1;
         }
         if (backward_l1(m, a, s)) return 1;
       }
       if (join_updates(models, n_models, s)) return 1;
-      have_fwd = has_next;
+      have_fwd = fuse && has_next;
     }
     for (int g = 0; g < n_models; ++g)
       if (end_epoch(models[g], s)) return 1;

@@ -157,6 +157,8 @@ struct UpdArgs {
 int l1_forward_simt(const L1Args& a, int n_partials, cudaStream_t s);
 int l1_backward_simt(const L1Args& a, int nblocks, cudaStream_t s);
 int hidden_launch(const HidArgs& a, int cluster, cudaStream_t s);
+// g.n models (same width, nlayers and cluster size) in one launch, one cluster each: replicate groups
+int hidden_group_launch(const HidGroupArgs& g, int cluster, cudaStream_t s);
 int hidden_update_launch(const UpdArgs& a, cudaStream_t s, bool overlap_previous = false);
 int hidden_update_blocks(int H, int L);  // blocks of one hidden_update_launch (each bumps DevState::upd_cnt once)
 int hidden_max_cluster(int H, int L);  // largest usable cluster size (16, 8, ...) for this device

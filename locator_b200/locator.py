@@ -103,7 +103,8 @@ def build_parser():
                         "with --jacknife a prediction-only sweep on the stored model. default: None")
     parser.add_argument("--replicates_per_gpu", default=4, type=int,
                         help="(locator_b200) bootstrap / window models trained side by side on each GPU (1-8; neither "
-                        "the indices nor the predictions depend on it). default: 4")
+                        "the indices nor the predictions depend on it; width 256 with more than 14 layers trains one "
+                        "model at a time). default: 4")
     return parser
 
 

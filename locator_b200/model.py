@@ -382,8 +382,10 @@ def fit_group(models, xs, ys, validation_datas, epochs=None, patience=100, verbo
     are issued in lockstep through ``loc_group_train_epochs`` so the models' latency-bound hidden
     stacks share launches.  Any batch size: above 32 rows the models' batch statistics and step ends
     share one launch each, and their 32-row chunks share hidden-stack launches.  Models must have the
-    same nlayers / batch size / number of training rows (replicates of one run do) and run the tcgen05 first layer
-    and hidden stack (width 256, nlayers up to 14: ``impl == hidden_impl == "tcgen05"``).
+    same width / nlayers / batch size / number of training rows (replicates of one run do) and run one kernel
+    family for the first layer and the hidden stack: all tcgen05 (width 256, nlayers up to 14) or all CUDA-core
+    (other widths), i.e. ``impl == hidden_impl`` and the same for every model.  Width 256 with 15..21 layers
+    (tcgen05 first layer, CUDA-core hidden stack) is refused; such models train one at a time.
     Returns the list of History objects.
     """
     G = len(models)

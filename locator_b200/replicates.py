@@ -115,11 +115,12 @@ def _run_items(L, items, base, reps=None):
         finally:
             args.out = original_out
     _tick(f"{len(models)} models created")
-    same = len({(r["traingen"].n, m.nlayers, m.batch_size) for r, m in zip(reps, models)}) == 1
-    # groups need the tcgen05 first layer AND hidden stack: width-256 models deeper than 14 layers run their hidden
-    # stack on CUDA cores and train one after the other
-    tc = all(m.impl == "tcgen05" and m.hidden_impl == "tcgen05" for m in models)
-    if len(reps) > 1 and same and tc:
+    same = len({(r["traingen"].n, m.width, m.nlayers, m.batch_size) for r, m in zip(reps, models)}) == 1
+    # groups need one kernel family for the first layer AND the hidden stack: tcgen05 (width 256, up to 14 layers)
+    # or CUDA cores (other widths).  Width-256 models deeper than 14 layers run a tcgen05 first layer in front of a
+    # CUDA-core hidden stack and train one after the other.
+    family = {(m.impl, m.hidden_impl) for m in models}
+    if len(reps) > 1 and same and family in ({("tcgen05", "tcgen05")}, {("simt", "simt")}):
         start = time.time()
         histories = fit_group(models, [r["traingen"] for r in reps], [r["trainlocs"] for r in reps],
                               [(r["testgen"], r["testlocs"]) for r in reps], epochs=args.max_epochs,
