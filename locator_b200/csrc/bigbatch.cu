@@ -514,12 +514,12 @@ __global__ void __launch_bounds__(1024) k_bb_hidden_update(BigArgs a) {
 // End of a large step whose chunks ran through the hidden stack side by side (grouped launches): per-chunk loss sums
 // added in chunk order (same bits as chunk-by-chunk launches), then the optimizer bookkeeping of the step.  One block
 // per model of a replicate group.
-__global__ void k_bb_step_end(BigEndArgs e, int nc, int loss_rows, int gated) {
+__global__ void k_bb_step_end(BigEndArgs e, int gated) {
   DevState* st = e.st[blockIdx.x];
   const float* slots = e.slots[blockIdx.x];
   if (gated && st->stopped) return;
   float acc = 0.f;
-  for (int c = 0; c < nc; ++c) {
+  for (int c = 0; c < e.nc[blockIdx.x]; ++c) {
     const float s = slots[2 * c], n = slots[2 * c + 1];
     const float mean = s / n;
     st->loss_total += mean * n;
@@ -528,7 +528,7 @@ __global__ void k_bb_step_end(BigEndArgs e, int nc, int loss_rows, int gated) {
     if (!isfinite(mean)) st->nonfinite = 1;
   }
   st->step_sum = acc;
-  st->last_loss = acc / (float)loss_rows;
+  st->last_loss = acc / (float)e.loss_rows[blockIdx.x];
   const int t = st->t + 1;
   st->t = t;
   st->step_id = st->step_id + 1;
@@ -536,9 +536,9 @@ __global__ void k_bb_step_end(BigEndArgs e, int nc, int loss_rows, int gated) {
   st->alpha = st->lr * sqrtf(1.f - b2p) / (1.f - b1p);
 }
 
-int bb_step_end_launch(const BigEndArgs& e, int nc, int loss_rows, int gated, cudaStream_t s) {
+int bb_step_end_launch(const BigEndArgs& e, int gated, cudaStream_t s) {
   LOC_CHECK(e.n >= 1 && e.n <= kMaxGroup, "step end (large batch): bad group size");
-  k_bb_step_end<<<(unsigned)e.n, 1, 0, s>>>(e, nc, loss_rows, gated);
+  k_bb_step_end<<<(unsigned)e.n, 1, 0, s>>>(e, gated);
   LOC_LAUNCHED();
   return 0;
 }

@@ -475,29 +475,32 @@ static BigArgs big_args(loc_model* m, const RowSrc& src, int gated) {
   return g;
 }
 
-// One optimizer step of n models created with batch_size > 32 (bigbatch.cu), the same number of rows each (a
-// single model, or a replicate group of loc_group_train_epochs):
+// One optimizer step of n models created with batch_size > 32 (bigbatch.cu), each over its own number of rows (a
+// single model, or the models of a replicate group of loc_group_train_epochs that have a step at this offset):
 //   batch statistics over all rows of every model's step (one launch for the group),
 //   first-layer forward with those statistics (one wide pass over W1 per model on the tcgen05 path),
 //   the step's 32-row chunks through the hidden stack -- tcgen05: side by side, one cluster per chunk, whole models
-//     per grouped launch (floor(8 / chunks) models each), then the step end of all models in one launch; CUDA cores:
-//     chunk by chunk, each after its first-layer forward, in a group chunk c of every model in one launch,
+//     packed into grouped launches by their own chunk counts (up to 8 chunks a launch), then the step end of those
+//     models in one launch; a model whose step fits in one chunk gets its own launch, as alone; CUDA cores: chunk by
+//     chunk, each after its first-layer forward, in a group chunk c of every model that has one in one launch,
 //   one pass over W1 | m | v per model (dW1 over all rows + Adam), back to back,
 //   the small-layer update over the chunks: after the backward for a single model; in a group on the model's side
 //     stream, forked after the hidden launch that holds its chunks (it runs under the other models' backwards) and
 //     joined before the next step.
 // Every model's launches are the ones it gets alone, with the same arguments, so the group gives the same bits.
 static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int gated, cudaStream_t s) {
-  const int nb = srcs[0].nb, nc = (nb + kMaxB - 1) / kMaxB;
   LOC_CHECK(n >= 1 && n <= kMaxGroup, "training step (large batch): bad group size");
+  int ncs[kMaxGroup], nc_max = 0;
   BigGroupArgs bg;
   bg.n = n;
   for (int g = 0; g < n; ++g) {
     loc_model* m = ms[g];
     m->chain_open = 0;
     m->span_perm = nullptr;
-    LOC_CHECK(srcs[g].nb == nb, "training step (large batch): the models of a group step the same number of rows");
-    LOC_CHECK(nb >= 1 && nc <= m->cap_chunks && m->bb_mean != nullptr, "training step: more rows than the model's batch_size");
+    ncs[g] = (srcs[g].nb + kMaxB - 1) / kMaxB;
+    if (ncs[g] > nc_max) nc_max = ncs[g];
+    LOC_CHECK(srcs[g].nb >= 1 && ncs[g] <= m->cap_chunks && m->bb_mean != nullptr,
+              "training step: more rows than the model's batch_size");
     LOC_CHECK(m->exchange == nullptr && m->tp == nullptr, "sharded models train with batch_size <= 32");
     bg.a[g] = big_args(m, srcs[g], gated);
   }
@@ -510,13 +513,14 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
       L1Args a = l1_args(m, m->train_packed, m->train_row_words, srcs[g], 0, gated);
       a.mmean = m->bb_mean;  // "inference" forward with the step's batch statistics
       a.mvar = m->bb_var;
-      if (l1_forward_wide_tc(a, m->n_partials, nb, m->wide, s)) return 1;
+      if (l1_forward_wide_tc(a, m->n_partials, srcs[g].nb, m->wide, s)) return 1;
     }
   }
   // Chunk c of model g: its first-layer forward into the model's partial tiles (unless the wide pass left them), then
   // the arguments of its hidden stack.
   auto chunk = [&](int g, int c, HidArgs& h) -> int {
     loc_model* m = ms[g];
+    const int nc = ncs[g];
     const RowSrc sc = chunk_rows(srcs[g], c);
     if (!wide) {
       L1Args a = l1_args(m, m->train_packed, m->train_row_words, sc, 0, gated);
@@ -532,7 +536,7 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
     const int64_t chunk_stride = (int64_t)m->L * kMaxB * m->H;
     h.acts = m->acts + c * chunk_stride;
     h.dzs = m->dzs + c * chunk_stride;
-    h.loss_rows = nb;
+    h.loss_rows = srcs[g].nb;
     h.row_base = kMaxB * c;
     h.mask_rows = kMaxB * m->cap_chunks;
     h.chunk_flags = (c > 0 ? 1 : 0) | (c < nc - 1 ? 2 : 0);
@@ -541,58 +545,67 @@ static int train_step_big(loc_model* const* ms, const RowSrc* srcs, int n, int g
   };
   const bool serial = getenv("LOC_BB_SERIAL") != nullptr;  // tests: one hidden launch per chunk and model
   const bool fork = n > 1;
-  // tcgen05 hidden stack: the chunks run side by side, one cluster each (k_hidden_tc_group); their loss sums and the
-  // step's optimizer bookkeeping follow in k_bb_step_end.  A model's chunks never straddle two launches: each
-  // publishes DevState::hid_seq once all of the model's chunks are done.
-  const bool side_by_side = wide && nc > 1 && !serial;
+  // tcgen05 hidden stack: the chunks of a model of more than one chunk run side by side, one cluster each
+  // (k_hidden_tc_group); their loss sums and the step's optimizer bookkeeping follow in k_bb_step_end.  A model's
+  // chunks never straddle two launches: each publishes DevState::hid_seq once all of the model's chunks are done.
+  auto side_by_side = [&](int g) { return wide && ncs[g] > 1 && !serial; };
   // CUDA-core hidden stack, a group: chunk by chunk, the forwards of every model, then chunk c of every model in one
   // k_hidden launch (one cluster per model).  Loss and step bookkeeping stay inside the launch, as for one model.
   const bool chunk_lockstep = !wide && fork && !ms[0]->hid_tc && !serial;
   if (chunk_lockstep) {
-    for (int c = 0; c < nc; ++c) {
+    for (int c = 0; c < nc_max; ++c) {
       HidGroupArgs hg;
-      hg.n = n;
+      hg.n = 0;
       for (int g = 0; g < n; ++g)
-        if (chunk(g, c, hg.a[g])) return 1;
+        if (c < ncs[g] && chunk(g, c, hg.a[hg.n++])) return 1;
       if (hidden_stacks(ms[0], hg, s)) return 1;
     }
     if (fork_updates(ms, n, s, [&](int i, cudaStream_t su) { return bb_hidden_update_launch(bg.a[i], su); })) return 1;
   }
-  const int per_launch = side_by_side ? kMaxGroup / nc : 1;
-  for (int g0 = 0; !chunk_lockstep && g0 < n; g0 += per_launch) {
-    const int g1 = g0 + per_launch < n ? g0 + per_launch : n;
-    HidGroupArgs hg;
+  // Models g0 .. g1 - 1 whose chunks are packed into hg: one grouped launch, then their updates forked.
+  HidGroupArgs hg;
+  hg.n = 0;
+  int g0 = 0;
+  auto flush = [&](int g1) -> int {
+    if (hg.n > 0 && hidden_tc_group_launch(hg, s)) return 1;
     hg.n = 0;
-    for (int g = g0; g < g1; ++g) {
-      loc_model* m = ms[g];
-      const int first = hg.n;
-      for (int c = 0; c < nc; ++c) {
-        HidArgs h;
-        if (chunk(g, c, h)) return 1;
-        if (side_by_side) {
-          h.chunk_flags = 2;  // nobody bumps the step counters inside the launch
-          h.val_slot = m->val_slots + 2 * c;
-          hg.a[hg.n++] = h;
-          continue;
-        }
-        if (hidden_stack(m, h, s)) return 1;
-      }
-      for (int i = first; i < hg.n; ++i) hg.a[i].hid_seq = m->h_hid_seq;  // published concurrently: the same (final) value
-    }
-    if (side_by_side && hidden_tc_group_launch(hg, s)) return 1;
-    if (fork && fork_updates(ms + g0, g1 - g0, s,
-                             [&](int i, cudaStream_t su) { return bb_hidden_update_launch(bg.a[g0 + i], su); }))
+    if (fork && g1 > g0 &&
+        fork_updates(ms + g0, g1 - g0, s, [&](int i, cudaStream_t su) { return bb_hidden_update_launch(bg.a[g0 + i], su); }))
       return 1;
-  }
-  if (side_by_side) {
-    BigEndArgs e;
-    e.n = n;
-    for (int g = 0; g < n; ++g) {
-      e.st[g] = ms[g]->st;
-      e.slots[g] = ms[g]->val_slots;
+    g0 = g1;
+    return 0;
+  };
+  BigEndArgs e;
+  e.n = 0;
+  for (int g = 0; !chunk_lockstep && g < n; ++g) {
+    loc_model* m = ms[g];
+    if (!side_by_side(g) || hg.n + ncs[g] > kMaxGroup)
+      if (flush(g)) return 1;
+    const int first = hg.n;
+    for (int c = 0; c < ncs[g]; ++c) {
+      HidArgs h;
+      if (chunk(g, c, h)) return 1;
+      if (side_by_side(g)) {
+        h.chunk_flags = 2;  // nobody bumps the step counters inside the launch
+        h.val_slot = m->val_slots + 2 * c;
+        hg.a[hg.n++] = h;
+        continue;
+      }
+      if (hidden_stack(m, h, s)) return 1;
     }
-    if (bb_step_end_launch(e, nc, nb, gated, s)) return 1;
+    for (int i = first; i < hg.n; ++i) hg.a[i].hid_seq = m->h_hid_seq;  // published concurrently: the same (final) value
+    if (side_by_side(g)) {
+      e.st[e.n] = m->st;
+      e.slots[e.n] = m->val_slots;
+      e.nc[e.n] = ncs[g];
+      e.loss_rows[e.n] = srcs[g].nb;
+      ++e.n;
+    } else if (flush(g + 1)) {
+      return 1;
+    }
   }
+  if (!chunk_lockstep && flush(n)) return 1;
+  if (e.n > 0 && bb_step_end_launch(e, gated, s)) return 1;
   for (int g = 0; g < n; ++g)
     if (bb_l1_backward_launch(bg.a[g], ms[g]->bb_pq, s)) return 1;
   if (!fork) return bb_hidden_update_launch(bg.a[0], s);
@@ -1247,6 +1260,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
   LOC_CHECK(models != nullptr && d_perms != nullptr && n_models >= 1 && n_models <= kMaxGroup && n_epochs >= 1,
             "loc_group_train_epochs: bad arguments");
   loc_model* m0 = models[0];
+  int64_t n_max = 0;  // rows of the largest training set: the epoch's last step offset is below it
   for (int g = 0; g < n_models; ++g) {
     loc_model* m = models[g];
     LOC_CHECK(m != nullptr && d_perms[g] != nullptr && m->train_packed != nullptr && m->val_packed != nullptr,
@@ -1258,9 +1272,10 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
               "loc_group_train_epochs: the models of a group must all run the tcgen05 kernels (width 256, nlayers <= 14) or all "
               "the CUDA-core kernels");
     LOC_CHECK(m->exchange == nullptr && m->tp == nullptr, "loc_group_train_epochs: sharded models cannot be grouped");
-    LOC_CHECK(m->H == m0->H && m->L == m0->L && m->B == m0->B && m->n_train == m0->n_train && m->cluster == m0->cluster,
-              "loc_group_train_epochs: replicates of a group must share width, nlayers, batch size, training-set size and "
-              "hidden-stack cluster size");
+    LOC_CHECK(m->H == m0->H && m->L == m0->L && m->B == m0->B && m->cluster == m0->cluster,
+              "loc_group_train_epochs: replicates of a group must share width, nlayers, batch size and hidden-stack cluster "
+              "size");
+    if (m->n_train > n_max) n_max = m->n_train;
   }
   cudaStream_t s = (cudaStream_t)stream;
   for (int g = 0; g < n_models; ++g) {
@@ -1269,7 +1284,11 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
     k_begin_call<<<1, 1, 0, s>>>(models[g]->st);
     LOC_LAUNCHED();
   }
-  auto rows = [&](int g, int64_t off) { return step_rows(models[g], d_perms[g], m0->n_train, off); };
+  // Training sets may differ in size: the step at offset `off` holds the models with off < n_train, each with its own
+  // rows, its own next step and its own epoch end -- the arguments it gets alone.
+  auto rows = [&](int g, int64_t off) { return step_rows(models[g], d_perms[g], models[g]->n_train, off); };
+  auto steps_at = [&](int g, int64_t off) { return off < models[g]->n_train; };
+  auto has_next = [&](int g, int64_t off) { return off + m0->B < models[g]->n_train; };
   // Schedule.  "ring" (default whenever every model's first-layer kernels leave one cluster's worth of SMs
   // free, loc_model_set_l1_ctas): one stream, per slot  H(g) -> B(g-1) -> U(g-1)  where H is the 16-CTA hidden
   // stack of model g (plain launch: starts when everything before it is complete), B the first-layer backward
@@ -1321,10 +1340,14 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
           if (backward_l1(pend.m, pend.a, s, overlap)) return 1;
           return update_launch(pend.m, pend.u, s, overlap);
         };
-        for (int64_t off = 0; off < m0->n_train; off += m0->B) {
-          const bool has_next = off + m0->B < m0->n_train;
+        for (int64_t off = 0; off < n_max; off += m0->B) {
           for (int g = g0; g < g1; ++g) {
+            if (!steps_at(g, off)) continue;  // this model's epoch has ended: its slot is skipped
             loc_model* m = models[g];
+            // the other models of the ring have ended their epoch: this model's own previous backward and update go
+            // first, and its hidden stack follows them as in a solo chained step
+            if (pend.m == m && launch_pending(true)) return 1;
+            if (pend.m == m) pend.m = nullptr;
             const RowSrc src = rows(g, off);
             L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 1);
             if (!have_fwd && forward_l1(m, a, s)) return 1;  // first step of the epoch: later ones are fused
@@ -1334,7 +1357,7 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
             if (h_overlaps) h.wait_bwd = m->h_bwd_cnt;
             if (hidden_stack(m, h, s, h_overlaps)) return 1;
             if (pend.m != nullptr && launch_pending(true)) return 1;
-            if (has_next) {
+            if (has_next(g, off)) {
               a.src_next = rows(g, off + m0->B);
               a.fuse_next = 1;
             }
@@ -1343,52 +1366,56 @@ int loc_group_train_epochs(loc_model** models, int32_t n_models, const int32_t* 
             pend.u = upd_args(m, src.nb, 1);
             pend.hid_seq = h.hid_seq;
           }
-          have_fwd = has_next;
+          have_fwd = true;  // every model with a step at the next offset fused its forward into this step's backward
         }
         if (pend.m != nullptr && launch_pending(false)) return 1;  // the ring's last backward and update of the epoch
         g0 = g1;
       }
     }
-    for (int64_t off = 0; big && off < m0->n_train; off += m0->B) {
+    for (int64_t off = 0; !ring && off < n_max; off += m0->B) {
+      // the models with a step at this offset
+      loc_model* ms[kMaxGroup];
       RowSrc srcs[kMaxGroup];
-      for (int g = 0; g < n_models; ++g) srcs[g] = rows(g, off);
-      if (train_step_big(models, srcs, n_models, 1, s)) return 1;
-    }
-    bool have_fwd = false;
-    for (int64_t off = 0; !ring && !big && off < m0->n_train; off += m0->B) {
-      const bool has_next = off + m0->B < m0->n_train;
+      int act[kMaxGroup], n = 0;
+      for (int g = 0; g < n_models; ++g)
+        if (steps_at(g, off)) {
+          ms[n] = models[g];
+          srcs[n] = rows(g, off);
+          act[n++] = g;
+        }
+      if (big) {
+        if (train_step_big(ms, srcs, n, 1, s)) return 1;
+        continue;
+      }
       HidGroupArgs hg;
-      hg.n = n_models;
+      hg.n = n;
       // first-layer forwards (first step of the epoch only: later ones are fused into the backward)
-      for (int g = 0; g < n_models; ++g) {
-        loc_model* m = models[g];
-        const RowSrc src = rows(g, off);
-        if (!have_fwd) {
-          L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 1);
+      for (int i = 0; i < n; ++i) {
+        loc_model* m = ms[i];
+        if (!(fuse && off > 0)) {
+          L1Args a = l1_args(m, m->train_packed, m->train_row_words, srcs[i], 1, 1);
           if (forward_l1(m, a, s)) return 1;
         }
-        hg.a[g] = hid_args(m, src, 1, 1, m->train_locs, nullptr);
-        begin_training_hidden(m, hg.a[g]);
+        hg.a[i] = hid_args(m, srcs[i], 1, 1, m->train_locs, nullptr);
+        begin_training_hidden(m, hg.a[i]);
       }
       // all hidden stacks in one launch: one cluster per replicate
       if (hidden_stacks(m0, hg, s)) return 1;
       // small-layer updates on the side streams, first-layer backward (+ next forward) back to back
-      if (fork_updates(models, n_models, s, [&](int g, cudaStream_t su) {
-            return update_launch(models[g], upd_args(models[g], hg.a[g].src.nb, 1), su);
+      if (fork_updates(ms, n, s, [&](int i, cudaStream_t su) {
+            return update_launch(ms[i], upd_args(ms[i], srcs[i].nb, 1), su);
           }))
         return 1;
-      for (int g = 0; g < n_models; ++g) {
-        loc_model* m = models[g];
-        const RowSrc src = rows(g, off);
-        L1Args a = l1_args(m, m->train_packed, m->train_row_words, src, 1, 1);
-        if (fuse && has_next) {
-          a.src_next = rows(g, off + m0->B);
+      for (int i = 0; i < n; ++i) {
+        loc_model* m = ms[i];
+        L1Args a = l1_args(m, m->train_packed, m->train_row_words, srcs[i], 1, 1);
+        if (fuse && has_next(act[i], off)) {
+          a.src_next = rows(act[i], off + m0->B);
           a.fuse_next = 1;
         }
         if (backward_l1(m, a, s)) return 1;
       }
-      if (join_updates(models, n_models, s)) return 1;
-      have_fwd = fuse && has_next;
+      if (join_updates(ms, n, s)) return 1;
     }
     for (int g = 0; g < n_models; ++g)
       if (end_epoch(models[g], s)) return 1;

@@ -370,7 +370,8 @@ def load_network(traingen, dropout_prop):
     # layer, hence the same setting for EVERY model of such a run whatever --replicates_per_gpu / --gpus say:
     # the outputs of a replicate run never depend on how it was scheduled.
     # (Only where the weight stream outlasts the hidden stack: RING_MIN_SNPS mirrors kRingMinK of the library.)
-    grouped = (args.bootstrap or args.windows) and K >= RING_MIN_SNPS
+    # The folds of a k-fold holdout run (locator_b200.holdout) are such replicates too.
+    grouped = (args.bootstrap or args.windows or getattr(args, "folds", None)) and K >= RING_MIN_SNPS
     return LocatorModel(K, width=args.width, nlayers=args.nlayers, dropout_prop=args.dropout_prop,
                         batch_size=args.batch_size, max_epochs=args.max_epochs, seed=_model_seed(),
                         l1_ctas=spare_cluster_l1_ctas() if grouped else None)
@@ -531,28 +532,33 @@ def _jacknife_draws(af, K, n_pred):
     t.join()
 
 
-def main(argv=None):
-    global args
-    parser = build_parser()
-    set_args(parser.parse_args(argv))
-
-    # set seed and gpu (locator.py:170-173), load stored parameters (:177-184), seed again in main() (:491-494):
-    # with --load_params it is the stored seed that decides the run's draws
+def start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights")):
+    """Install ``ns`` as ``args`` and set the run up as the reference does: seed and gpu (locator.py:170-173),
+    load stored parameters (:177-184), seed again in main() (:491-494) -- with --load_params it is the stored
+    seed that decides the run's draws.  ``extensions``: flags of this build, kept from the command line (a
+    params file does not hold them)."""
+    set_args(ns)
     if args.seed is not None:
         np.random.seed(args.seed)
     if args.gpu_number is not None:
         os.environ["CUDA_VISIBLE_DEVICES"] = args.gpu_number
     if args.load_params is not None:
-        gpus, rpg, lw = args.gpus, args.replicates_per_gpu, args.load_weights
+        kept = {k: getattr(args, k) for k in extensions}
         with open(args.load_params, "r") as f:
             args.__dict__ = json.load(f)
-        args.gpus, args.replicates_per_gpu, args.load_weights = gpus, rpg, lw
+        args.__dict__.update(kept)
     if args.seed is not None:
         np.random.seed(args.seed)
     if args.gpu_number is not None:
         os.environ["CUDA_VISIBLE_DEVICES"] = args.gpu_number
     if args.out is None:
         raise SystemExit("--out is required")
+    return args
+
+
+def main(argv=None):
+    parser = build_parser()
+    start_run(parser.parse_args(argv))
     validate_args(args)
     _write_params()
     from . import replicates

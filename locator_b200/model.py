@@ -381,8 +381,10 @@ def fit_group(models, xs, ys, validation_datas, epochs=None, patience=100, verbo
     callbacks state and history, and ends bit-identical to the same model trained alone); the steps
     are issued in lockstep through ``loc_group_train_epochs`` so the models' latency-bound hidden
     stacks share launches.  Any batch size: above 32 rows the models' batch statistics and step ends
-    share one launch each, and their 32-row chunks share hidden-stack launches.  Models must have the
-    same width / nlayers / batch size / number of training rows (replicates of one run do) and run one kernel
+    share one launch each, and their 32-row chunks share hidden-stack launches.  Training and validation
+    sets may differ in size (the folds of a k-fold holdout): each epoch's step at row offset ``off`` holds
+    the models that still have rows there, and every model ends its epoch after its own last step.  Models
+    must have the same width / nlayers / batch size and run one kernel
     family for the first layer and the hidden stack: all tcgen05 (width 256, nlayers up to 14) or all CUDA-core
     (other widths), i.e. ``impl == hidden_impl`` and the same for every model.  Width 256 with 15..21 layers
     (tcgen05 first layer, CUDA-core hidden stack) is refused; such models train one at a time.
@@ -399,7 +401,7 @@ def fit_group(models, xs, ys, validation_datas, epochs=None, patience=100, verbo
         m.set_schedule(patience=patience)
         rngs.append(np.random.default_rng(m.seed))
         m._keep["perms"] = []
-    n = models[0]._keep["train"][0].n
+    ns = [m._keep["train"][0].n for m in models]
     done = 0
     states = [m.state() for m in models]
     while done < epochs:
@@ -409,7 +411,7 @@ def fit_group(models, xs, ys, validation_datas, epochs=None, patience=100, verbo
         ne = min(epochs_per_call, epochs - done)
         perms = []
         for i in active:
-            p = _as_dev(np.stack([rngs[i].permutation(n) for _ in range(ne)]).astype(np.int32), torch.int32)
+            p = _as_dev(np.stack([rngs[i].permutation(ns[i]) for _ in range(ne)]).astype(np.int32), torch.int32)
             models[i]._keep["perms"] = [p]
             perms.append(p)
         handles = (C.c_void_p * len(active))(*[models[i]._h for i in active])

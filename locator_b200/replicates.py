@@ -28,6 +28,11 @@ def _tick(what):
 # ---------------------------------------------------------------------------------------------
 # (de)serialisation of packed device matrices for the worker processes
 # ---------------------------------------------------------------------------------------------
+# the packed device matrices a base dict or a work item may hold ("genotypes": the whole filtered matrix of a
+# k-fold holdout run, whose folds are row gathers of it)
+_MATRICES = ("traingen", "testgen", "predgen", "genotypes")
+
+
 def _to_host(g):
     return {"words": g.words.cpu().numpy(), "n": g.n, "K": g.K}
 
@@ -87,6 +92,14 @@ def _prepare(L, item, base):
                 "trainlocs": item["trainlocs"], "testlocs": item["testlocs"], "norm": item["norm"],
                 "pred": item["pred"], "samples": item["samples"], "boot": 0, "cb_boot": None,
                 "seed_tag": item["index"] + 1, "out": item["window_out"]}
+    if item["kind"] == "fold":
+        # k-fold holdout (locator_b200.holdout): row gathers of the filtered matrix; "pred" is the held-out fold
+        g, locs, f = base["genotypes"], base["locs"], item["fold"]
+        print("starting fold " + str(f))
+        return {"traingen": g.take_rows(item["train"]), "testgen": g.take_rows(item["val"]),
+                "predgen": g.take_rows(item["held"]), "trainlocs": locs[item["train"]], "testlocs": locs[item["val"]],
+                "norm": base["norm"], "pred": item["held"], "samples": base["samples"], "boot": f, "cb_boot": f,
+                "seed_tag": f + 1, "out": item["fold_out"], "fold": f}
     raise ValueError(item["kind"])
 
 
@@ -94,9 +107,10 @@ def _run_items(L, items, base, reps=None):
     """Train + predict a list of replicates inside the current process / on the current device.
 
     One replicate: the reference's sequence (load_network, train_network, predict_locs).  Several:
-    the models are trained side by side as one lockstep group (model.fit_group, at any batch size;
-    results are bit-identical to training them one after the other), then predicted one by one.
-    ``reps``: the items' matrices when a Prefetcher has already prepared them.
+    the models are trained side by side as one lockstep group (model.fit_group, at any batch size and
+    training-set size; results are bit-identical to training them one after the other), then predicted
+    one by one.  ``reps``: the items' matrices when a Prefetcher has already prepared them.
+    Returns one result per item: (fold, held-out rows, de-normalised predictions) for a holdout fold, else None.
     """
     from .model import fit_group
 
@@ -115,7 +129,7 @@ def _run_items(L, items, base, reps=None):
         finally:
             args.out = original_out
     _tick(f"{len(models)} models created")
-    same = len({(r["traingen"].n, m.width, m.nlayers, m.batch_size) for r, m in zip(reps, models)}) == 1
+    same = len({(m.width, m.nlayers, m.batch_size) for m in models}) == 1  # training-set sizes may differ
     # groups need one kernel family for the first layer AND the hidden stack: tcgen05 (width 256, up to 14 layers)
     # or CUDA cores (other widths).  Width-256 models deeper than 14 layers run a tcgen05 first layer in front of a
     # CUDA-core hidden stack and train one after the other.
@@ -136,8 +150,15 @@ def _run_items(L, items, base, reps=None):
         for m, cb, rep in zip(models, callbacks, reps):
             h, _ = L.train_network(m, rep["traingen"], rep["testgen"], rep["trainlocs"], rep["testlocs"], cb, rep["boot"])
             histories.append(h)
+    results = []
     for m, h, rep in zip(models, histories, reps):
         meanlong, sdlong, meanlat, sdlat = rep["norm"]
+        if "fold" in rep:
+            from .holdout import predict_fold
+
+            results.append(predict_fold(m, h, rep))
+            continue
+        results.append(None)
         original_out = args.out
         args.out = rep["out"]
         try:
@@ -150,6 +171,7 @@ def _run_items(L, items, base, reps=None):
     _tick("group predicted, files written")
     if items and items[0]["kind"] == "window":
         print(f"Window run time {(time.time() - t1) / 60:.2f} minutes")
+    return results
 
 
 class Prefetcher:
@@ -194,19 +216,22 @@ class Prefetcher:
 
 
 def _run_pipelined(L, groups, base):
-    """groups: iterable of work-item lists.  Group i+1 is prepared while group i trains."""
+    """groups: iterable of work-item lists.  Group i+1 is prepared while group i trains.  Returns the items'
+    results (_run_items) in order."""
     pf = Prefetcher(L, base)
+    results = []
     try:
         cur = None
         for items in groups:
             nxt = (items, pf.submit(items))
             if cur is not None:
-                _run_items(L, cur[0], base, Prefetcher.collect(cur[1]))
+                results += _run_items(L, cur[0], base, Prefetcher.collect(cur[1]))
             cur = nxt
         if cur is not None:
-            _run_items(L, cur[0], base, Prefetcher.collect(cur[1]))
+            results += _run_items(L, cur[0], base, Prefetcher.collect(cur[1]))
     finally:
         pf.close()
+    return results
 
 
 def _group_size(args):
@@ -226,7 +251,7 @@ def serve(L, base, take_group, queue_is_deep, done, who="worker"):
     and predict it; while the queue is deep the NEXT group is taken and prepared meanwhile.
 
     take_group(block) -> list of items, or None when there is nothing (block=False) / the queue has ended;
-    queue_is_deep() -> prefetching cannot starve another GPU; done(items) reports completion.
+    queue_is_deep() -> prefetching cannot starve another GPU; done(items, results) reports completion.
     Shared by the worker processes of ``locator --gpus N`` (ReplicatePool) and by the ranks of a
     torch.distributed job (RankQueue)."""
     pf = Prefetcher(L, base)
@@ -248,9 +273,9 @@ def serve(L, base, take_group, queue_is_deep, done, who="worker"):
             _tick(f"{who}: group of {len(items)} taken")
             reps = Prefetcher.collect(fut)
             _tick(f"{who}: group prepared")
-            _run_items(L, items, base, reps)
+            results = _run_items(L, items, base, reps)
             _tick(f"{who}: group done")
-            done(items)
+            done(items, results)
     finally:
         pf.close()
 
@@ -304,8 +329,12 @@ def run_items_ranked(L, base, items, world=1, store=None, key="loc_queue"):
     """Rank mode of the replicate drivers: this process (one GPU) serves `items` together with the other
     ranks of the job.  Returns the indices this rank ran, in groups."""
     q = RankQueue(items, world, store, key, _group_size(L.args))
-    serve(L, base, q.take_group, q.queue_is_deep, lambda its: None, who=f"rank {os.environ.get('RANK', '0')}")
+    serve(L, base, q.take_group, q.queue_is_deep, lambda its, res: None, who=f"rank {os.environ.get('RANK', '0')}")
     return q.taken
+
+
+def _item_id(item):
+    return item.get("boot", item.get("index", item.get("fold")))
 
 
 def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q=None):
@@ -317,7 +346,7 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
                 if item is None:
                     break
                 run(rank, args, item)
-                result_q.put(("done", rank, item.get("boot", item.get("index"))))
+                result_q.put(("done", rank, (_item_id(item), None)))
             result_q.put(("exit", rank, None))
             return
         _tick(f"worker {rank}: process up")
@@ -338,8 +367,9 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
             _tick(f"worker {rank}: base matrices received")
         if base_host is not None:
             base = dict(base_host)
-            for k in ("traingen", "testgen", "predgen"):
-                base[k] = _to_dev(base_host[k])
+            for k in _MATRICES:
+                if k in base_host:
+                    base[k] = _to_dev(base_host[k])
         import queue as _queue
 
         G = _group_size(args)
@@ -381,9 +411,9 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
             except NotImplementedError:
                 return False
 
-        def done(items):
-            for it in items:
-                result_q.put(("done", rank, it.get("boot", it.get("index"))))
+        def done(items, results):
+            for it, res in zip(items, results):
+                result_q.put(("done", rank, (_item_id(it), res)))
 
         serve(L, base, take_group, queue_is_deep, done, who=f"worker {rank}")
         _tick(f"worker {rank}: exiting")
@@ -394,7 +424,8 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
 
 
 class ReplicatePool:
-    """One worker process per GPU pulling work items from a shared queue."""
+    """One worker process per GPU pulling work items from a shared queue.  After close(), ``results`` holds
+    (item id, result) per item in order of completion (result: see _run_items)."""
 
     def __init__(self, n_gpus, args, base=None, runner=None, deferred_base=False):
         """deferred_base: the workers are started now and wait for the run's matrices (``send_base``)."""
@@ -414,14 +445,16 @@ class ReplicatePool:
             p.start()
         self.submitted = 0
         self.closed = False
+        self.results = []
 
     @staticmethod
     def _host(base):
         if base is None:
             return None
         base_host = dict(base)
-        for k in ("traingen", "testgen", "predgen"):
-            base_host[k] = _to_host(base[k])
+        for k in _MATRICES:
+            if k in base:
+                base_host[k] = _to_host(base[k])
         return base_host
 
     def send_base(self, base):
@@ -469,6 +502,7 @@ class ReplicatePool:
                 continue
             if kind == "done":
                 done += 1
+                self.results.append(payload)
             elif kind == "exit":
                 exited += 1
                 exited_ranks.add(rank)
