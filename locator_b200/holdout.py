@@ -24,6 +24,7 @@ import sys
 import numpy as np
 
 from . import locator as L
+from . import replicates
 
 
 def build_parser():
@@ -84,26 +85,11 @@ def predict_fold(model, history, rep):
 
 def run(ac, locs, norm, samples, folds):
     """Train and predict every fold through the replicate queue; returns the fold results in fold order."""
-    from . import replicates
-
     args = L.args
     base = {"genotypes": ac.packed, "locs": locs, "norm": norm, "samples": samples}
     items = [{"kind": "fold", "fold": f, "held": held, "train": train, "val": val, "fold_out": f"{args.out}_holdout{f}"}
              for f, (held, train, val) in enumerate(folds)]
-    n_gpus = max(1, int(getattr(args, "gpus", 1) or 1))
-    if n_gpus == 1:
-        G = replicates._group_size(args)
-        results = replicates._run_pipelined(L, (items[i:i + G] for i in range(0, len(items), G)), base)
-    else:
-        pool = replicates.ReplicatePool(n_gpus, args, base)
-        try:
-            for it in items:
-                pool.submit(it)
-            pool.close()
-        finally:
-            pool.abort()
-        results = [res for _, res in pool.results]
-    return sorted(results, key=lambda r: r[0])
+    return replicates.run_work(L, items, base)
 
 
 def write_predictions(results, locs, norm, samples):
@@ -142,13 +128,17 @@ def main(argv=None):
     check_args(args)  # a --load_params file may ask for one of them
     L.validate_args(args)
     L._write_params()
-    genotypes, samples = L.load_genotypes()
-    sample_data, locs = L.sort_samples(samples, genotypes)
-    meanlong, sdlong, meanlat, sdlat, locs = L.normalize_locs(locs)
-    norm = (meanlong, sdlong, meanlat, sdlat)
-    ac = L.filter_snps(genotypes)
-    folds = draw_folds(locs, int(args.folds), float(args.train_split))
-    results = run(ac, locs, norm, samples, folds)
+    replicates.start_pool_early(args)  # several GPUs: the workers boot while this process reads and draws
+    try:
+        genotypes, samples = L.load_genotypes()
+        sample_data, locs = L.sort_samples(samples, genotypes)
+        meanlong, sdlong, meanlat, sdlat, locs = L.normalize_locs(locs)
+        norm = (meanlong, sdlong, meanlat, sdlat)
+        ac = L.filter_snps(genotypes)
+        folds = draw_folds(locs, int(args.folds), float(args.train_split))
+        results = run(ac, locs, norm, samples, folds)
+    finally:
+        replicates.abort_early_pool()  # only still there if the run failed before handing it over
     write_predictions(results, locs, norm, samples)
     return 0
 

@@ -21,9 +21,10 @@ Differences that are deliberate and documented in DESIGN.md:
     reference) come from Philox streams keyed by ``--seed``;
   * weights files are ``.weights.npz`` (no HDF5 on this image) and only exist with --keep_weights
     (the best-epoch checkpoint lives in device memory, not on disk);
-  * ``--gpus N`` and ``--replicates_per_gpu G`` (extensions, not written to params.json): --bootstrap /
-    --windows replicates are spread over N GPUs of the box with a work queue, G models trained side
-    by side on each GPU (locator_b200.replicates); results do not depend on either.
+  * ``--gpus N`` and ``--replicates_per_gpu G`` (extensions, not written to params.json): --bootstrap
+    replicates (the FULL model included), --windows replicates and the folds of a k-fold holdout run
+    (locator_b200.holdout) are work items of one queue at every GPU count, spread over N GPUs of the box,
+    G models trained side by side on each GPU (locator_b200.replicates); results do not depend on either.
 """
 from __future__ import annotations
 
@@ -100,7 +101,8 @@ def build_parser():
     parser.add_argument("--load_weights", default=None,
                         help="(locator_b200) predict from a weights file written by --keep_weights (.weights.npz, Keras "
                         "weight order; see python -m locator_b200.keras_weights for .weights.h5) instead of training: "
-                        "with --jacknife a prediction-only sweep on the stored model. default: None")
+                        "with --jacknife a prediction-only sweep on the stored model; not with --bootstrap or --windows, "
+                        "which train every model they predict from. default: None")
     parser.add_argument("--replicates_per_gpu", default=4, type=int,
                         help="(locator_b200) bootstrap / window models trained side by side on each GPU (1-8; neither "
                         "the indices nor the predictions depend on it; width 256 with more than 14 layers trains one "
@@ -147,6 +149,9 @@ def validate_args(ns):
         problems.append(f"--patience {ns.patience}: must be >= 0")
     if not 1 <= int(getattr(ns, "replicates_per_gpu", 4) or 1) <= 8:
         problems.append(f"--replicates_per_gpu {ns.replicates_per_gpu}: must be in [1, 8]")
+    if getattr(ns, "load_weights", None) and (ns.bootstrap or ns.windows):
+        problems.append(f"--load_weights with --{'bootstrap' if ns.bootstrap else 'windows'}: replicate runs train every "
+                        "model they predict from")
     if ns.windows:
         # the reference takes int(args.window_start / _stop / _size) inside its loop (locator.py:524-531): a value
         # such as "2e5" only fails there, after the genome has been read; here it fails now

@@ -1,7 +1,8 @@
 """Replicate drivers: --bootstrap and --windows runs of the reference are loops over independent
 models (/root/reference/locator/locator.py:519-583 windows, :609-681 bootstrap).  Here the
-independent models are work items of a dynamic queue served by one worker process per GPU
-(``--gpus N``); there is no collective on the training path.  Everything that consumes numpy's
+independent models (and the folds of locator_b200.holdout) are work items handed to run_work, which
+serves them in this process with one GPU and from one worker process per GPU with ``--gpus N``;
+there is no collective on the training path.  Everything that consumes numpy's
 global random stream (bootstrap reseeds + site orders, per-window imputation / subsample / split)
 is drawn serially in the parent, in the reference's order, and shipped with the work item, so the
 indices do not depend on the number of GPUs.
@@ -9,6 +10,7 @@ indices do not depend on the number of GPUs.
 from __future__ import annotations
 
 import copy
+import itertools
 import os
 import time
 import traceback
@@ -42,6 +44,11 @@ def _to_dev(h):
     from .genotypes import PackedGenotypes
 
     return PackedGenotypes(torch.as_tensor(h["words"]).cuda(), h["n"], h["K"])
+
+
+def _convert(d, fn):
+    """Copy of a base dict or work item (or None) with its packed matrices converted by fn (_to_host / _to_dev)."""
+    return None if d is None else {k: fn(v) if k in _MATRICES else v for k, v in d.items()}
 
 
 def draw_bootstrap_orders(nsites, nboots):
@@ -103,21 +110,19 @@ def _prepare(L, item, base):
     raise ValueError(item["kind"])
 
 
-def _run_items(L, items, base, reps=None):
+def _run_items(L, items, reps):
     """Train + predict a list of replicates inside the current process / on the current device.
 
     One replicate: the reference's sequence (load_network, train_network, predict_locs).  Several:
     the models are trained side by side as one lockstep group (model.fit_group, at any batch size and
     training-set size; results are bit-identical to training them one after the other), then predicted
-    one by one.  ``reps``: the items' matrices when a Prefetcher has already prepared them.
+    one by one.  ``reps``: the items prepared by _prepare (a Prefetcher).
     Returns one result per item: (fold, held-out rows, de-normalised predictions) for a holdout fold, else None.
     """
     from .model import fit_group
 
     args = L.args
     t1 = time.time()
-    if reps is None:
-        reps = [_prepare(L, it, base) for it in items]
     models, callbacks = [], []
     for rep in reps:
         L._seed_tag[0] = rep["seed_tag"]
@@ -215,27 +220,12 @@ class Prefetcher:
         self.pool.shutdown(wait=True)
 
 
-def _run_pipelined(L, groups, base):
-    """groups: iterable of work-item lists.  Group i+1 is prepared while group i trains.  Returns the items'
-    results (_run_items) in order."""
-    pf = Prefetcher(L, base)
-    results = []
-    try:
-        cur = None
-        for items in groups:
-            nxt = (items, pf.submit(items))
-            if cur is not None:
-                results += _run_items(L, cur[0], base, Prefetcher.collect(cur[1]))
-            cur = nxt
-        if cur is not None:
-            results += _run_items(L, cur[0], base, Prefetcher.collect(cur[1]))
-    finally:
-        pf.close()
-    return results
-
-
 def _group_size(args):
     return max(1, min(8, int(getattr(args, "replicates_per_gpu", 1) or 1)))
+
+
+def _n_gpus(args):
+    return max(1, int(getattr(args, "gpus", 1) or 1))
 
 
 def _resolve(runner):
@@ -252,7 +242,7 @@ def serve(L, base, take_group, queue_is_deep, done, who="worker"):
 
     take_group(block) -> list of items, or None when there is nothing (block=False) / the queue has ended;
     queue_is_deep() -> prefetching cannot starve another GPU; done(items, results) reports completion.
-    Shared by the worker processes of ``locator --gpus N`` (ReplicatePool) and by the ranks of a
+    Shared by one-GPU runs (run_work), the worker processes of ``--gpus N`` (ReplicatePool) and the ranks of a
     torch.distributed job (RankQueue)."""
     pf = Prefetcher(L, base)
     try:
@@ -273,7 +263,7 @@ def serve(L, base, take_group, queue_is_deep, done, who="worker"):
             _tick(f"{who}: group of {len(items)} taken")
             reps = Prefetcher.collect(fut)
             _tick(f"{who}: group prepared")
-            results = _run_items(L, items, base, reps)
+            results = _run_items(L, items, reps)
             _tick(f"{who}: group done")
             done(items, results)
     finally:
@@ -333,20 +323,12 @@ def run_items_ranked(L, base, items, world=1, store=None, key="loc_queue"):
     return q.taken
 
 
-def _item_id(item):
-    return item.get("boot", item.get("index", item.get("fold")))
-
-
-def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q=None):
+def _worker(rank, n_gpus, args, init_q, task_q, result_q, runner=None):
     try:
-        if runner is not None:  # host-logic tests: no CUDA, the runner consumes the raw item
+        if runner is not None:  # host-logic tests: no CUDA, no base; the runner consumes the raw item
             run = _resolve(runner)
-            while True:
-                item = task_q.get()
-                if item is None:
-                    break
-                run(rank, args, item)
-                result_q.put(("done", rank, (_item_id(item), None)))
+            for item in iter(task_q.get, None):
+                result_q.put(("done", rank, (item["seq"], run(rank, args, item))))
             result_q.put(("exit", rank, None))
             return
         _tick(f"worker {rank}: process up")
@@ -359,27 +341,14 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
         _tick(f"worker {rank}: torch + CUDA context ready")
 
         L.set_args(copy.copy(args))
-        base = None
-        if init_q is not None:
-            # the pool was started before the parent had the run's matrices (so that this start-up -- import
-            # torch, CUDA context: seconds -- overlaps the parent's own): they arrive here, once
-            base_host = init_q.get()
-            _tick(f"worker {rank}: base matrices received")
-        if base_host is not None:
-            base = dict(base_host)
-            for k in _MATRICES:
-                if k in base_host:
-                    base[k] = _to_dev(base_host[k])
+        # the pool is started before the parent has the run's matrices (so that this start-up -- import torch, CUDA
+        # context: seconds -- overlaps the parent's own): they arrive here, once
+        base = _convert(init_q.get(), _to_dev)
+        _tick(f"worker {rank}: base matrices received")
         import queue as _queue
 
         G = _group_size(args)
         state = {"finished": False}
-
-        def to_dev(it):
-            for k in ("traingen", "testgen", "predgen"):
-                if k in it and isinstance(it[k], dict):
-                    it[k] = _to_dev(it[k])
-            return it
 
         def take_group(block):
             """Up to G queued items; None when there is nothing (block=False) or the queue has ended."""
@@ -402,7 +371,7 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
                     state["finished"] = True
                     break
                 items.append(nxt)
-            return [to_dev(it) for it in items]
+            return [_convert(it, _to_dev) for it in items]
 
         def queue_is_deep():
             """Prefetch only while every worker could still fill a group of its own (no starving at the tail)."""
@@ -413,7 +382,7 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
 
         def done(items, results):
             for it, res in zip(items, results):
-                result_q.put(("done", rank, (_item_id(it), res)))
+                result_q.put(("done", rank, (it["seq"], res)))
 
         serve(L, base, take_group, queue_is_deep, done, who=f"worker {rank}")
         _tick(f"worker {rank}: exiting")
@@ -424,41 +393,27 @@ def _worker(rank, n_gpus, args, base_host, task_q, result_q, runner=None, init_q
 
 
 class ReplicatePool:
-    """One worker process per GPU pulling work items from a shared queue.  After close(), ``results`` holds
-    (item id, result) per item in order of completion (result: see _run_items)."""
+    """One worker process per GPU pulling work items from a shared queue.  The workers start at once and wait for
+    the run's base matrices (send_base); close() returns the items' results (see _run_items) in submission order."""
 
-    def __init__(self, n_gpus, args, base=None, runner=None, deferred_base=False):
-        """deferred_base: the workers are started now and wait for the run's matrices (``send_base``)."""
+    def __init__(self, n_gpus, args, runner=None):
         import multiprocessing as mp
 
         ctx = mp.get_context("spawn")
         self.n = n_gpus
         self.task_q = ctx.Queue()
         self.result_q = ctx.Queue()
-        self.init_qs = [ctx.Queue() for _ in range(n_gpus)] if deferred_base else None
-        base_host = self._host(base)
+        self.init_qs = [ctx.Queue() for _ in range(n_gpus)]
         self.procs = [ctx.Process(target=_worker,
-                                  args=(r, n_gpus, args, base_host, self.task_q, self.result_q, runner,
-                                        self.init_qs[r] if deferred_base else None))
+                                  args=(r, n_gpus, args, self.init_qs[r], self.task_q, self.result_q, runner))
                       for r in range(n_gpus)]
         for p in self.procs:
             p.start()
         self.submitted = 0
         self.closed = False
-        self.results = []
-
-    @staticmethod
-    def _host(base):
-        if base is None:
-            return None
-        base_host = dict(base)
-        for k in _MATRICES:
-            if k in base:
-                base_host[k] = _to_host(base[k])
-        return base_host
 
     def send_base(self, base):
-        base_host = self._host(base)
+        base_host = _convert(base, _to_host)
         for q in self.init_qs:
             q.put(base_host)
 
@@ -472,11 +427,7 @@ class ReplicatePool:
                 p.join()
 
     def submit(self, item):
-        item = dict(item)
-        for k in ("traingen", "testgen", "predgen"):
-            if k in item and not isinstance(item[k], dict):
-                item[k] = _to_host(item[k])
-        self.task_q.put(item)
+        self.task_q.put(dict(_convert(item, _to_host), seq=self.submitted))
         self.submitted += 1
 
     def close(self):
@@ -486,7 +437,8 @@ class ReplicatePool:
             self.task_q.put(None)
         import queue as _queue
 
-        done = exited = 0
+        results = {}
+        exited = 0
         errors = []
         exited_ranks = set()
         while exited < self.n and not errors:
@@ -501,8 +453,8 @@ class ReplicatePool:
                         break
                 continue
             if kind == "done":
-                done += 1
-                self.results.append(payload)
+                seq, res = payload
+                results[seq] = res
             elif kind == "exit":
                 exited += 1
                 exited_ranks.add(rank)
@@ -515,70 +467,70 @@ class ReplicatePool:
         _tick("parent: workers joined")
         if errors:
             raise RuntimeError(f"replicate worker {errors[0][0]} failed:\n{errors[0][1]}")
-        if done != self.submitted:
-            raise RuntimeError(f"{self.submitted - done} replicates were not completed")
+        if len(results) != self.submitted:
+            raise RuntimeError(f"{self.submitted - len(results)} replicates were not completed")
+        return [results[seq] for seq in range(self.submitted)]
 
 
 # ---------------------------------------------------------------------------------------------
-# drivers called from locator.main()
+# drivers called from locator.main() and holdout.main()
 # ---------------------------------------------------------------------------------------------
-_early = {"pool": None, "taken": None}
+_early = {"pool": None}
 
 
 def start_pool_early(args):
     """Called by main() right after the arguments are known: with several GPUs the worker processes of a
-    --windows / --bootstrap run boot (import torch, create their CUDA context) while the parent is still
-    importing, reading metadata and drawing indices."""
-    n_gpus = max(1, int(getattr(args, "gpus", 1) or 1))
-    if n_gpus > 1 and (args.windows or args.bootstrap) and _early["pool"] is None:
+    --windows / --bootstrap / k-fold holdout run boot (import torch, create their CUDA context) while the parent is
+    still importing, reading metadata and drawing indices."""
+    n_gpus = _n_gpus(args)
+    if n_gpus > 1 and (args.windows or args.bootstrap or getattr(args, "folds", None)) and _early["pool"] is None:
         _tick("parent: starting the worker pool")
-        _early["pool"] = ReplicatePool(n_gpus, args, deferred_base=bool(args.bootstrap) and not args.windows)
+        _early["pool"] = ReplicatePool(n_gpus, args)
     return _early["pool"]
 
 
 def abort_early_pool():
-    """End of main(): a pool that was never handed over, or whose driver failed before close(), is torn down."""
-    for key in ("pool", "taken"):
-        pool, _early[key] = _early[key], None
-        if pool is not None:
-            pool.abort()
+    """End of main(): a pool that was never handed over (the run failed before its driver started) is torn down."""
+    pool, _early["pool"] = _early["pool"], None
+    if pool is not None:
+        pool.abort()
 
 
-def _take_pool(n_gpus, args, base=None):
+def run_work(L, items, base=None):
+    """Train and predict every work item; returns one result per item (see _run_items), in item order.
+
+    ``items`` is consumed lazily, in order and in this thread, so whatever draws from numpy's global stream while
+    producing them keeps the reference's order.  One GPU: this process serves the items in groups of
+    --replicates_per_gpu, the next group prepared while one trains.  Several: the worker pool (started early by
+    start_pool_early, or now) receives ``base`` and then every item as it is produced."""
+    args = L.args
+    n_gpus = _n_gpus(args)
+    if n_gpus == 1:
+        items, G, results = iter(items), _group_size(args), []
+        serve(L, base, lambda block: list(itertools.islice(items, G)) or None, lambda: True,
+              lambda its, res: results.extend(res), who="parent")
+        return results
     pool, _early["pool"] = _early["pool"], None
     if pool is None:
-        pool = ReplicatePool(n_gpus, args, base)
-    elif pool.init_qs is not None:
+        pool = ReplicatePool(n_gpus, args)
+    try:
         _tick("parent: sending the base matrices")
         pool.send_base(base)
-    _early["taken"] = pool
-    return pool
+        for item in items:
+            pool.submit(item)
+        return pool.close()
+    finally:
+        pool.abort()
 
 
 def run_bootstrap(L, traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples):
-    args = L.args
+    """The un-resampled FULL model (locator.py:611-632) and every replicate, all work items.  Training draws nothing
+    from numpy's global stream, so every replicate's draws are taken first (full groups form at once)."""
     base = {"traingen": traingen, "testgen": testgen, "predgen": predgen, "trainlocs": trainlocs,
             "testlocs": testlocs, "norm": norm, "pred": pred, "samples": samples}
-    n_gpus = max(1, int(getattr(args, "gpus", 1) or 1))
-    if n_gpus == 1:
-        # 1. initial full run (locator.py:611-632)
-        L._seed_tag[0] = 0
-        L._run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, "FULL", "FULL")
-        # 2. every replicate's draws, serially, as the reference's loop would take them
-        orders = draw_bootstrap_orders(traingen.K, args.nboots)
-        G = _group_size(args)
-        items = [{"kind": "boot", "boot": boot, "site_order": order} for boot, order in enumerate(orders)]
-        _run_pipelined(L, (items[i:i + G] for i in range(0, len(items), G)), base)
-        return
-    # Several GPUs: the full model is one more independent work item (training draws nothing from numpy's
-    # global stream, so the replicates' draws do not have to wait for it), and the workers start up while
-    # the parent draws: no GPU idles through the full run.
-    orders = draw_bootstrap_orders(traingen.K, args.nboots)  # before the first submit: full groups form at once
-    pool = _take_pool(n_gpus, args, base)
-    pool.submit({"kind": "full", "boot": "FULL"})
-    for boot, order in enumerate(orders):
-        pool.submit({"kind": "boot", "boot": boot, "site_order": order})
-    pool.close()
+    orders = draw_bootstrap_orders(traingen.K, L.args.nboots)
+    boots = [{"kind": "boot", "boot": boot, "site_order": order} for boot, order in enumerate(orders)]
+    run_work(L, [{"kind": "full", "boot": "FULL"}] + boots, base)
 
 
 def window_bounds(positions, start, stop, size):
@@ -596,44 +548,27 @@ def run_windows(L, genotypes, samples):
     start = int(args.window_start)
     stop = np.max(positions) if args.window_stop == None else int(args.window_stop)  # noqa: E711
     size = int(args.window_size)  # validate_args: int() accepts it, as the reference requires
-    n_gpus = max(1, int(getattr(args, "gpus", 1) or 1))
-    pool = _take_pool(n_gpus, args) if n_gpus > 1 else None
     # Recipes instead of matrices whenever no draw depends on the genotypes: whoever runs the window (a
     # worker process, or this process's prefetch thread) reads, filters and packs it.
     # LOC_WINDOWS_PARENT_INGEST=1 keeps the serial reference order of work (parity tests compare the two).
     recipes_ok = L.windows_are_data_independent() and not os.environ.get("LOC_WINDOWS_PARENT_INGEST")
-    pending, recipes = [], []
-    for index, (i, a, b) in enumerate(window_bounds(positions, start, stop, size)):
-        print(f"\nProcessing window {i}-{i+size}")
-        print(f"SNPs {a}-{b}")
-        sub = genotypes[a:b]
-        sample_data, locs = L.sort_samples(samples, sub)
-        meanlong, sdlong, meanlat, sdlat, locs = L.normalize_locs(locs)
-        if sub.lazy is not None and recipes_ok:
-            item = {"kind": "window_lazy", "index": index, "window_out": f"{args.out}_{i}-{i+size-1}",
-                    "where": sub.lazy, "locs": locs, "drawn": L.draw_split(locs),
-                    "norm": (meanlong, sdlong, meanlat, sdlat), "samples": samples}
-            if pool is not None:
-                pool.submit(item)
-            else:
-                recipes.append(item)
-            continue
-        ac = L.filter_snps(sub)
-        train, test, traingen, testgen, trainlocs, testlocs, pred, predgen = L.split_train_test(ac, locs)
-        item = {"kind": "window", "index": index, "window_out": f"{args.out}_{i}-{i+size-1}", "traingen": traingen,
-                "testgen": testgen, "predgen": predgen, "trainlocs": trainlocs, "testlocs": testlocs,
-                "norm": (meanlong, sdlong, meanlat, sdlat), "pred": pred, "samples": samples}
-        if pool is None:
-            pending.append(item)
-            if len(pending) >= _group_size(args):
-                _run_items(L, pending, None)
-                pending = []
-        else:
-            pool.submit(item)
-    if pending:
-        _run_items(L, pending, None)
-    if recipes:
-        G = _group_size(args)
-        _run_pipelined(L, (recipes[j:j + G] for j in range(0, len(recipes), G)), None)
-    if pool is not None:
-        pool.close()
+
+    def items():
+        for index, (i, a, b) in enumerate(window_bounds(positions, start, stop, size)):
+            print(f"\nProcessing window {i}-{i+size}")
+            print(f"SNPs {a}-{b}")
+            sub = genotypes[a:b]
+            sample_data, locs = L.sort_samples(samples, sub)
+            meanlong, sdlong, meanlat, sdlat, locs = L.normalize_locs(locs)
+            if sub.lazy is not None and recipes_ok:
+                yield {"kind": "window_lazy", "index": index, "window_out": f"{args.out}_{i}-{i+size-1}",
+                       "where": sub.lazy, "locs": locs, "drawn": L.draw_split(locs),
+                       "norm": (meanlong, sdlong, meanlat, sdlat), "samples": samples}
+                continue
+            ac = L.filter_snps(sub)
+            train, test, traingen, testgen, trainlocs, testlocs, pred, predgen = L.split_train_test(ac, locs)
+            yield {"kind": "window", "index": index, "window_out": f"{args.out}_{i}-{i+size-1}", "traingen": traingen,
+                   "testgen": testgen, "predgen": predgen, "trainlocs": trainlocs, "testlocs": testlocs,
+                   "norm": (meanlong, sdlong, meanlat, sdlat), "pred": pred, "samples": samples}
+
+    run_work(L, items())

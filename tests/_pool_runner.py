@@ -1,4 +1,5 @@
-"""CPU stand-in for a replicate: records which worker ran which item (used by test_host.py)."""
+"""CPU stand-in for a replicate: records which worker ran which item and returns the item's boot (used by
+test_host.py)."""
 import os
 import time
 
@@ -9,3 +10,4 @@ def run(rank, args, item):
     time.sleep(0.01 * item.get("cost", 1))
     with open(os.path.join(args.out, f"item_{item['boot']}.txt"), "w") as fh:
         fh.write(f"{rank} {int(item['site_order'].sum())}\n")
+    return item["boot"]

@@ -121,7 +121,8 @@ def test_vcf_reader_matches_oracle_reader_and_zarr_round_trip(tmp_path, fixture_
 
 def test_replicate_pool_two_workers(tmp_path):
     """The N > 1 replicate path without GPUs: two worker processes drain the shared queue, every item
-    runs exactly once, a failing item surfaces as an error in the parent."""
+    runs exactly once, its result comes back in submission order although items of uneven cost finish out of
+    order, a failing item surfaces as an error in the parent."""
     from locator_b200 import replicates
 
     sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
@@ -133,8 +134,10 @@ def test_replicate_pool_two_workers(tmp_path):
     args = argparse.Namespace(out=str(tmp_path))
     pool = replicates.ReplicatePool(2, args, runner="_pool_runner:run")
     for b, o in enumerate(orders):
-        pool.submit({"kind": "boot", "boot": b, "site_order": o, "cost": 1 + (b % 3)})
-    pool.close()
+        pool.submit({"kind": "boot", "boot": b, "site_order": o, "cost": 100 if b == 0 else 1})
+    assert pool.close() == list(range(7))
+    finished = sorted(range(7), key=lambda b: os.path.getmtime(tmp_path / f"item_{b}.txt"))
+    assert finished[-1] == 0  # item 0 (100x the cost) finished last, its result still comes first
     ranks = set()
     for b, o in enumerate(orders):
         rank, s = open(tmp_path / f"item_{b}.txt").read().split()
@@ -596,13 +599,17 @@ def test_validate_args_limits_of_this_build():
         return L.build_parser().parse_args(["--vcf", "x.vcf", "--sample_data", "s.txt", "--out", "o"] + list(extra))
 
     for ok in ([], ["--batch_size", "1"], ["--batch_size", "64"], ["--batch_size", "256"], ["--width", "96"],
-               ["--nlayers", "2"], ["--dropout_prop", "0"], ["--nlayers", "21"], ["--width", "320", "--nlayers", "13"]):
+               ["--nlayers", "2"], ["--dropout_prop", "0"], ["--nlayers", "21"], ["--width", "320", "--nlayers", "13"],
+               ["--jacknife", "--load_weights", "f"]):
         L.validate_args(ns(*ok))
     for bad, word in ((["--batch_size", "0"], "batch_size"), (["--batch_size", "257"], "batch_size"),
                       (["--width", "100"], "width"), (["--nlayers", "1"], "nlayers"), (["--dropout_prop", "1.0"], "dropout_prop"),
                       (["--max_epochs", "0"], "max_epochs"), (["--windows", "--window_size", "2e5"], "window_size"),
                       # deepest stack per width: the CUDA-core hidden stack's shared-memory layout (loc_hidden_max_nlayers)
                       (["--nlayers", "22"], "at most 21"), (["--width", "512"], "width 512"),
-                      (["--width", "224", "--nlayers", "11"], "at most 10")):
+                      (["--width", "224", "--nlayers", "11"], "at most 10"),
+                      # replicate runs train every model they predict from
+                      (["--bootstrap", "--load_weights", "f"], "load_weights"),
+                      (["--windows", "--window_size", "100", "--load_weights", "f"], "load_weights")):
         with pytest.raises(SystemExit, match=word):
             L.validate_args(ns(*bad))
