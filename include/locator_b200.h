@@ -108,6 +108,24 @@ int loc_site_sums(const uint32_t* d_packed, int64_t n, int64_t K, int64_t row_wo
 int loc_pack_sites(const int8_t* d_gt, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx,
                    int64_t K, uint32_t* d_packed, int64_t row_words, void* stream);
 
+/* The same three steps straight from a PLINK 1 .bed file (SNP-major, mode byte 0x01) in device memory.  d_bed is
+ * the record area without the 3-byte header: record v is ceil(nsamp/4) bytes at d_bed + v * ceil(nsamp/4) (any
+ * alignment), sample i the 2-bit field at bits 2*(i%4) of its byte i/4; the pad fields of a record's last byte are
+ * ignored.  A record stands for the GT rows 0 -> (1, 1) homozygous A1, 1 -> (-1, -1) missing, 2 -> (0, 1),
+ * 3 -> (0, 0) homozygous A2 (A1, .bim column 5, is allele index 1), and every output equals that of the int8 entry
+ * point on that cube:
+ *   loc_bed_site_stats    = loc_site_stats    (filter_snps :265-273: count_alleles / is_biallelic / min_mac);
+ *   loc_bed_pack_sites    = loc_pack_sites    (to_allele_counts()[:, :, 1], :277): packed value = copies of A1,
+ *                           missing -> 0; any K;
+ *   loc_bed_missing_calls = loc_missing_calls (replace_md :255-261), same two phases.
+ * loc_compact_sites and loc_patch_calls apply unchanged. */
+int loc_bed_site_stats(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, int32_t min_mac, int32_t* d_n_alleles,
+                       int32_t* d_alt_count, int32_t* d_n_missing, uint8_t* d_keep, void* stream);
+int loc_bed_pack_sites(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
+                       uint32_t* d_packed, int64_t row_words, void* stream);
+int loc_bed_missing_calls(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
+                          const int32_t* d_n_missing, int64_t* d_offsets, int64_t* d_k, int64_t* d_samp, void* stream);
+
 /* Overwrite individual genotypes (imputation results of replace_md, :258-261):
  * packed[d_samp[i]][d_k[i]] = d_val[i], i < n.  (k indexes packed columns.) */
 int loc_patch_calls(uint32_t* d_packed, int64_t row_words, const int64_t* d_k,

@@ -1,5 +1,5 @@
-// K1/K2: genotype filter, 2-bit pack, row/column gathers, jacknife column replacement.
-// Integer, HBM-bound, bit-exact against oracle/ingest_ref.py.
+// K1/K2: genotype filter, 2-bit pack, row/column gathers, jacknife column replacement; the filter and pack also
+// straight from PLINK 1 .bed records.  Integer, HBM-bound, bit-exact against oracle/ingest_ref.py.
 //
 // Reference semantics (locator/locator.py): filter_snps :265-281 (allel count_alleles /
 // is_biallelic / to_allele_counts()[:, :, 1]), split_train_test :303-307, bootstrap gather
@@ -465,6 +465,187 @@ __global__ void __launch_bounds__(256) k_missing_calls(const int8_t* __restrict_
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// PLINK 1 .bed records (SNP-major, mode byte 0x01), without the 3-byte header: record v is rb = ceil(N/4) bytes at
+// bed + v * rb, sample i the 2-bit field at bits 2 * (i % 4) of its byte i / 4.  Codes and the GT rows they stand
+// for (A1 plays allele index 1): 0 = homozygous A1 (1, 1), 1 = missing (-1, -1), 2 = heterozygous (0, 1),
+// 3 = homozygous A2 (0, 0).  The pad fields of a record's last byte are 0 (= homozygous A1): every kernel masks
+// them.  Records are byte-aligned (rb may be odd): the kernels read the aligned 32-bit words that hold a record's
+// bytes -- a CUDA allocation starts 256-byte aligned, so such a word never leaves the allocation -- and drop the
+// fields that lie outside the record.
+// ---------------------------------------------------------------------------------------------
+
+// 0x55555555-style mask of the fields, inside [0, nsamp), of the word whose first byte is record byte wb (< 0: the
+// word starts before the record)
+__device__ __forceinline__ uint32_t bed_field_mask(int64_t wb, int64_t nsamp) {
+  const int64_t f0 = wb * 4;  // sample of the word's first field
+  const int64_t lo = f0 < 0 ? -f0 : 0;
+  const int64_t hi = nsamp - f0 < 16 ? nsamp - f0 : 16;
+  if (hi <= lo) return 0u;
+  const uint32_t top = hi >= 16 ? 0xFFFFFFFFu : (1u << (2 * hi)) - 1u;
+  return top & ~((1u << (2 * lo)) - 1u) & 0x55555555u;
+}
+
+constexpr int kBedLoads = 8;  // 32-bit loads in flight per lane: a 1 KB record (4,096 samples) in one round
+
+// Site statistics: one warp per record.  Per word, the four codes are counted with masks and popc.
+__global__ void __launch_bounds__(256) k_bed_site_stats(const uint8_t* __restrict__ bed, int64_t nvar, int64_t nsamp,
+                                                        int min_mac, int32_t* __restrict__ n_alleles,
+                                                        int32_t* __restrict__ alt_count, int32_t* __restrict__ n_missing,
+                                                        uint8_t* __restrict__ keep) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  const int64_t rb = (nsamp + 3) >> 2;
+  for (int64_t v = warp; v < nvar; v += nwarps) {
+    const uintptr_t addr = reinterpret_cast<uintptr_t>(bed + v * rb);
+    const uint32_t* words = reinterpret_cast<const uint32_t*>(addr & ~(uintptr_t)3);
+    const int64_t head = (int64_t)(addr & 3);  // bytes of the first word before the record
+    const int64_t nw = (head + rb + 3) >> 2;
+    int hom1 = 0, miss = 0, het = 0, hom2 = 0;
+    for (int64_t i = lane; i < nw; i += 32 * kBedLoads) {
+      uint32_t x[kBedLoads];
+#pragma unroll
+      for (int u = 0; u < kBedLoads; ++u) x[u] = i + 32 * u < nw ? __ldcs(words + i + 32 * u) : 0u;
+#pragma unroll
+      for (int u = 0; u < kBedLoads; ++u) {
+        const int64_t wb = 4 * (i + 32 * u) - head;  // record byte of the word's first byte
+        const uint32_t m = i + 32 * u >= nw ? 0u : (wb >= 0 && 4 * wb + 16 <= nsamp) ? 0x55555555u
+                                                                                     : bed_field_mask(wb, nsamp);
+        const uint32_t lo = x[u], hi = x[u] >> 1;  // low / high bit of every field at the field's even bit
+        hom1 += __popc(~(lo | hi) & m);
+        miss += __popc(lo & ~hi & m);
+        het += __popc(~lo & hi & m);
+        hom2 += __popc(lo & hi & m);
+      }
+    }
+    hom1 = __reduce_add_sync(0xffffffffu, hom1);
+    miss = __reduce_add_sync(0xffffffffu, miss);
+    het = __reduce_add_sync(0xffffffffu, het);
+    hom2 = __reduce_add_sync(0xffffffffu, hom2);
+    if (lane == 0) {
+      const int na = (hom1 + het > 0) + (het + hom2 > 0);  // allele 1 (A1) seen, allele 0 (A2) seen
+      const int alt = 2 * hom1 + het;
+      if (n_alleles) n_alleles[v] = na;
+      if (alt_count) alt_count[v] = alt;
+      if (n_missing) n_missing[v] = miss;
+      if (keep) keep[v] = (na == 2 && (min_mac == 1 || alt >= min_mac)) ? 1 : 0;
+    }
+  }
+}
+
+// codes of 16 fields -> copies of A1 (the packed value): {0 -> 2, 1 -> 0, 2 -> 1, 3 -> 0}
+__device__ __forceinline__ uint32_t bed_counts(uint32_t x) {
+  const uint32_t lo = x & 0x55555555u, hi = (x >> 1) & 0x55555555u;
+  return ((~(lo | hi) & 0x55555555u) << 1) | (hi & ~lo);
+}
+
+// the 4 record bytes at p (any alignment) as one word, from the aligned words that hold them; the word after the
+// record area (end) is not read
+__device__ __forceinline__ uint32_t bed_word(const uint8_t* p, uintptr_t end) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(p);
+  const uint32_t* w = reinterpret_cast<const uint32_t*>(a & ~(uintptr_t)3);
+  const uint32_t sh = (uint32_t)(a & 3) * 8u;
+  const uint32_t lo = __ldg(w);
+  const uint32_t hi = (sh != 0u && reinterpret_cast<uintptr_t>(w + 1) < end) ? __ldg(w + 1) : 0u;
+  return __funnelshift_r(lo, hi, sh);
+}
+
+// 16 x 16 matrix of 2-bit elements, row q in r[q] (element j at bits 2j) -> its transpose in place.  Stage B swaps
+// bit B of the row and the column index: the off-diagonal B x B blocks trade places.
+template <int B, uint32_t M>
+__device__ __forceinline__ void transpose_stage(uint32_t (&r)[16]) {
+#pragma unroll
+  for (int q = 0; q < 16; ++q)
+    if ((q & B) == 0) {
+      const uint32_t t = ((r[q] >> (2 * B)) ^ r[q + B]) & M;
+      r[q + B] ^= t;
+      r[q] ^= t << (2 * B);
+    }
+}
+
+__device__ __forceinline__ void transpose16x2(uint32_t (&r)[16]) {
+  transpose_stage<8, 0x0000FFFFu>(r);
+  transpose_stage<4, 0x00FF00FFu>(r);
+  transpose_stage<2, 0x0F0F0F0Fu>(r);
+  transpose_stage<1, 0x33333333u>(r);
+}
+
+// Pack: SNP-major records -> the sample-major 2-bit matrix of the kept sites.  A block covers 512 samples (16 per
+// lane: one 4-byte piece of a record) and 16 packed words (256 kept sites) at a time; a warp builds two words: per
+// word a lane loads the piece of each of the 16 records, maps the codes, and transposes the 16 x 16 block in
+// registers, which gives its 16 samples' words.  A padded shared-memory tile turns them into 64 contiguous bytes
+// per sample for the write (the layout of k_pack_sites).  The blocks of one grid row loop over the word groups, so
+// any K fits one launch.
+constexpr int kBedPackSamples = 512;
+
+__global__ void __launch_bounds__(256) k_bed_pack_sites(const uint8_t* __restrict__ bed, int64_t nvar, int64_t nsamp,
+                                                        const int64_t* __restrict__ site_idx, int64_t K,
+                                                        uint32_t* __restrict__ packed, int64_t row_words) {
+  __shared__ uint32_t tile[kBedPackSamples * kPackPitch];  // [sample j of the lane][lane][word], pitch 17
+  const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
+  const int64_t rb = (nsamp + 3) >> 2;
+  const uintptr_t end = reinterpret_cast<uintptr_t>(bed + nvar * rb);
+  const int64_t s0 = (int64_t)blockIdx.x * kBedPackSamples;
+  const int64_t byte0 = s0 / 4 + 4 * lane;  // record byte of this lane's first sample
+  const int64_t wgroups = (row_words + kPackWords - 1) / kPackWords;
+  for (int64_t wg = blockIdx.y; wg < wgroups; wg += gridDim.y) {
+    const int64_t w0 = wg * kPackWords;
+#pragma unroll
+    for (int jw = 0; jw < 2; ++jw) {
+      const int wl = 2 * wi + jw;
+      const int64_t k0 = (w0 + wl) * 16;
+      uint32_t r[16];
+#pragma unroll
+      for (int q = 0; q < 16; ++q)
+        r[q] = (k0 + q < K && byte0 < rb) ? bed_counts(bed_word(bed + __ldg(site_idx + k0 + q) * rb + byte0, end)) : 0u;
+      transpose16x2(r);  // r[j] = the word of sample s0 + 16 * lane + j
+#pragma unroll
+      for (int j = 0; j < 16; ++j) tile[(j * 32 + lane) * kPackPitch + wl] = r[j];
+    }
+    __syncthreads();
+    const int quarter = threadIdx.x & 3;
+    const int64_t w = w0 + 4 * quarter;
+    if (w < row_words) {
+      for (int sl = threadIdx.x >> 2; sl < kBedPackSamples; sl += 64) {
+        const int64_t ss = s0 + sl;
+        if (ss >= nsamp) break;  // samples past N (the pad fields among them) are not written
+        const uint32_t* t = tile + ((sl % 16) * 32 + sl / 16) * kPackPitch + 4 * quarter;
+        *reinterpret_cast<uint4*>(packed + ss * row_words + w) = make_uint4(t[0], t[1], t[2], t[3]);
+      }
+    }
+    __syncthreads();  // the tile is read before the next word group overwrites it
+  }
+}
+
+// k_missing_calls on .bed records: one warp per kept site with missing calls (code 1), ascending sample order.
+__global__ void __launch_bounds__(256) k_bed_missing_calls(const uint8_t* __restrict__ bed, int64_t nsamp,
+                                                           const int64_t* __restrict__ site_idx, int64_t K,
+                                                           const int64_t* __restrict__ offsets,
+                                                           int64_t* __restrict__ out_k, int64_t* __restrict__ out_samp) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  const int64_t rb = (nsamp + 3) >> 2;
+  for (int64_t k = warp; k < K; k += nwarps) {
+    const int64_t beg = offsets[k], end = offsets[k + 1];
+    if (beg == end) continue;
+    const uint8_t* rec = bed + site_idx[k] * rb;
+    int64_t pos = beg;
+    for (int64_t s0 = 0; s0 < nsamp && pos < end; s0 += 32) {
+      const int64_t sidx = s0 + lane;
+      const bool miss = sidx < nsamp && ((rec[sidx >> 2] >> (2 * (sidx & 3))) & 3) == 1;
+      const unsigned m = __ballot_sync(0xffffffffu, miss);
+      if (miss) {
+        const int64_t o = pos + __popc(m & ((1u << lane) - 1u));
+        out_k[o] = k;
+        out_samp[o] = sidx;
+      }
+      pos += __popc(m);
+    }
+  }
+}
+
 // sums[k] = sum over all n rows of the packed counts of SNP k (jacknife allele frequencies, locator.py:714-717,
 // with wide integers: the reference's pinned numpy promotes the uint8 row sums).  One thread per packed word
 // (16 SNPs), rows in the loop: a warp reads 128 contiguous bytes per row.
@@ -548,23 +729,27 @@ int loc_compact_sites(const uint8_t* d_keep, int64_t nvar, int64_t* d_site_idx, 
   return 0;
 }
 
+// phase 1 of loc_missing_calls / loc_bed_missing_calls: offsets[0..K] (offsets[K] = number of missing calls)
+static int missing_offsets(const int64_t* d_site_idx, int64_t K, const int32_t* d_n_missing, int64_t* d_offsets,
+                           cudaStream_t st) {
+  ScanSrc src = {nullptr, d_n_missing, d_site_idx};
+  long long* block_off = nullptr;
+  if (scan_launch(src, K, d_offsets + K, &block_off, st)) return 1;
+  if (K > 0) {
+    k_scan_offsets<<<(unsigned)cdiv(K, kScanBlock), kScanThreads, 0, st>>>(src, K, block_off, d_offsets);
+    LOC_LAUNCHED();
+  }
+  LOC_CUDA(cudaFreeAsync(block_off, st));
+  return 0;
+}
+
 int loc_missing_calls(const int8_t* d_gt, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
                       const int32_t* d_n_missing, int64_t* d_offsets, int64_t* d_k, int64_t* d_samp, void* stream) {
   (void)nvar;
   LOC_CHECK(K >= 0 && nsamp > 0 && d_offsets != nullptr, "loc_missing_calls: bad arguments");
   LOC_CHECK(K == 0 || (d_gt != nullptr && d_site_idx != nullptr && d_n_missing != nullptr), "loc_missing_calls: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  ScanSrc src = {nullptr, d_n_missing, d_site_idx};
-  if (d_k == nullptr) {  // phase 1: offsets[0..K] (offsets[K] = number of missing calls)
-    long long* block_off = nullptr;
-    if (scan_launch(src, K, d_offsets + K, &block_off, st)) return 1;
-    if (K > 0) {
-      k_scan_offsets<<<(unsigned)cdiv(K, kScanBlock), kScanThreads, 0, st>>>(src, K, block_off, d_offsets);
-      LOC_LAUNCHED();
-    }
-    LOC_CUDA(cudaFreeAsync(block_off, st));
-    return 0;
-  }
+  if (d_k == nullptr) return missing_offsets(d_site_idx, K, d_n_missing, d_offsets, st);
   LOC_CHECK(d_samp != nullptr, "loc_missing_calls: null output pointer");
   if (K == 0) return 0;
   int64_t blocks = cdiv(K, 8);
@@ -614,6 +799,59 @@ int loc_pack_sites(const int8_t* d_gt, int64_t nvar, int64_t nsamp, const int64_
     case 4: k_pack_sites<4><<<grid, 256, 0, st>>>(d_gt, nsamp, d_site_idx, K, d_packed, row_words); break;
     default: k_pack_sites<2><<<grid, 256, 0, st>>>(d_gt, nsamp, d_site_idx, K, d_packed, row_words); break;
   }
+  LOC_LAUNCHED();
+  return 0;
+}
+
+int loc_bed_site_stats(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, int32_t min_mac, int32_t* d_n_alleles,
+                       int32_t* d_alt_count, int32_t* d_n_missing, uint8_t* d_keep, void* stream) {
+  LOC_CHECK(nvar >= 0 && nsamp > 0, "loc_bed_site_stats: bad shape");
+  if (nvar == 0) return 0;
+  LOC_CHECK(d_bed != nullptr, "loc_bed_site_stats: null record pointer");
+  int64_t blocks = cdiv(nvar, 8);
+  static int wave = 0;  // one resident wave of blocks; the warps loop over the records
+  if (wave == 0) {
+    int per_sm = 8;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bed_site_stats, 256, 0);
+    wave = sm_count() * (per_sm > 0 ? per_sm : 1);
+  }
+  if (blocks > wave) blocks = wave;
+  k_bed_site_stats<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(d_bed, nvar, nsamp, min_mac, d_n_alleles,
+                                                                     d_alt_count, d_n_missing, d_keep);
+  LOC_LAUNCHED();
+  return 0;
+}
+
+int loc_bed_pack_sites(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
+                       uint32_t* d_packed, int64_t row_words, void* stream) {
+  LOC_CHECK(nvar >= 0 && nsamp > 0 && K >= 0, "loc_bed_pack_sites: bad shape");
+  LOC_CHECK(row_words >= cdiv(K, 16) && row_words % 4 == 0,
+            "loc_bed_pack_sites: row_words must be >= ceil(K/16) and a multiple of 4");
+  if (row_words == 0) return 0;
+  LOC_CHECK(d_packed != nullptr && (K == 0 || (d_bed != nullptr && d_site_idx != nullptr)),
+            "loc_bed_pack_sites: null pointer");
+  LOC_CHECK(reinterpret_cast<uintptr_t>(d_packed) % 16 == 0, "loc_bed_pack_sites: packed rows must be 16-byte aligned");
+  LOC_CHECK(cdiv(nsamp, kBedPackSamples) <= 0x7fffffff, "loc_bed_pack_sites: too many samples");
+  const int64_t wgroups = cdiv(row_words, kPackWords);
+  dim3 grid((unsigned)cdiv(nsamp, kBedPackSamples), (unsigned)(wgroups < 65535 ? wgroups : 65535));
+  k_bed_pack_sites<<<grid, 256, 0, (cudaStream_t)stream>>>(d_bed, nvar, nsamp, d_site_idx, K, d_packed, row_words);
+  LOC_LAUNCHED();
+  return 0;
+}
+
+int loc_bed_missing_calls(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
+                          const int32_t* d_n_missing, int64_t* d_offsets, int64_t* d_k, int64_t* d_samp, void* stream) {
+  (void)nvar;
+  LOC_CHECK(K >= 0 && nsamp > 0 && d_offsets != nullptr, "loc_bed_missing_calls: bad arguments");
+  LOC_CHECK(K == 0 || (d_bed != nullptr && d_site_idx != nullptr && d_n_missing != nullptr),
+            "loc_bed_missing_calls: null pointer");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (d_k == nullptr) return missing_offsets(d_site_idx, K, d_n_missing, d_offsets, st);
+  LOC_CHECK(d_samp != nullptr, "loc_bed_missing_calls: null output pointer");
+  if (K == 0) return 0;
+  int64_t blocks = cdiv(K, 8);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  k_bed_missing_calls<<<(unsigned)blocks, 256, 0, st>>>(d_bed, nsamp, d_site_idx, K, d_offsets, d_k, d_samp);
   LOC_LAUNCHED();
   return 0;
 }

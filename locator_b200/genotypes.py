@@ -154,7 +154,7 @@ class PackedGenotypes:
 
 
 class _Staging(threading.local):
-    """Per-thread pair of pinned host buffers the zarr chunks are decoded into (reused across windows)."""
+    """Per-thread pair of pinned host buffers the genotype rows are read into (reused across windows)."""
     bufs = None
     events = None
 
@@ -176,19 +176,24 @@ def _staging_buffers(nbytes):
     return st
 
 
-def upload_rows(rows) -> torch.Tensor:
-    """io.ZarrRows (GT int8 [nvar, N, 2] on disk) -> device tensor, without an intermediate pageable copy.
+_TORCH_DTYPES = {np.dtype(np.int8): torch.int8, np.dtype(np.uint8): torch.uint8}
 
-    Blocks of rows are decoded (thread pool, io._zarr_array) straight into one of two pinned staging
-    buffers and copied to the device asynchronously: block i+1 is decoded while block i is in flight.
+
+def upload_rows(rows) -> torch.Tensor:
+    """Rows of a genotype file on disk -> device tensor of ``rows.stored_shape``, without an intermediate pageable
+    copy: io.ZarrRows (GT int8 [nvar, N, 2]) or io.BedRows (.bed records uint8 [nvar, ceil(N/4)]).
+
+    Blocks of rows are read (zarr: chunks decoded by a thread pool, io._zarr_array; .bed: positioned reads) straight
+    into one of two pinned staging buffers and copied to the device asynchronously: block i+1 is read while block i
+    is in flight.
     """
-    nvar, N, ploidy = rows.shape
-    assert ploidy == 2 and rows.dtype == np.int8
+    shape, dtype = tuple(rows.stored_shape), _TORCH_DTYPES[np.dtype(rows.stored_dtype)]
+    nvar = shape[0]
     dev = _dev()
-    out = torch.empty((nvar, N, 2), dtype=torch.int8, device=dev)
+    out = torch.empty(shape, dtype=dtype, device=dev)
     if nvar == 0:
         return out
-    row_bytes = N * 2
+    row_bytes = int(np.prod(shape[1:], dtype=np.int64)) * out.element_size()
     block = max(1, min(nvar, UPLOAD_BLOCK_BYTES // row_bytes))
     st = _staging_buffers(block * row_bytes)
     stream = torch.cuda.current_stream()
@@ -197,7 +202,7 @@ def upload_rows(rows) -> torch.Tensor:
         slot = i & 1
         if st.events[slot] is not None:
             st.events[slot].synchronize()  # the previous copy out of this buffer has finished
-        host = st.bufs[slot][:(b - a) * row_bytes].view(torch.int8).view(b - a, N, 2)
+        host = st.bufs[slot][:(b - a) * row_bytes].view(dtype).view((b - a,) + shape[1:])
         rows.rows(a, b).read(out=host.numpy())
         out[a:b].copy_(host, non_blocking=True)
         ev = torch.cuda.Event()
@@ -262,3 +267,71 @@ def pack_sites(g: torch.Tensor, site_idx) -> PackedGenotypes:
         check(lib.loc_pack_sites(g.data_ptr(), nvar, N, idx.data_ptr(), K, out.ptr, out.row_words, _stream()),
               "loc_pack_sites")
     return out
+
+
+# ---- PLINK 1 .bed records on the device (the GT cube they stand for is never built) ----
+class BedRecords:
+    """SNP-major .bed records uint8 [nvar, ceil(N/4)] in device memory (header stripped); ``shape`` is that of
+    the GT cube [nvar, N, 2] they stand for."""
+
+    def __init__(self, records: torch.Tensor, nsamp: int):
+        self.records = records
+        self.nvar, self.nsamp = int(records.shape[0]), int(nsamp)
+        assert records.dim() == 2 and records.shape[1] == (self.nsamp + 3) // 4
+
+    @property
+    def shape(self):
+        return (self.nvar, self.nsamp, 2)
+
+    @staticmethod
+    def upload(rows) -> "BedRecords":
+        """io.BedRows -> device (pinned double-buffered positioned reads, upload_rows)."""
+        return BedRecords(upload_rows(rows), rows.nsamp)
+
+    @staticmethod
+    def from_host(records, nsamp) -> "BedRecords":
+        return BedRecords(_as_dev(np.asarray(records, dtype=np.uint8), torch.uint8), nsamp)
+
+
+def bed_site_stats(bed: BedRecords, min_mac=2):
+    """site_stats on .bed records: (n_alleles, alt_count, n_missing, keep) device tensors of the cube they stand for
+    (loc_bed_site_stats)."""
+    dev = bed.records.device
+    na = torch.empty(bed.nvar, dtype=torch.int32, device=dev)
+    alt = torch.empty(bed.nvar, dtype=torch.int32, device=dev)
+    miss = torch.empty(bed.nvar, dtype=torch.int32, device=dev)
+    keep = torch.empty(bed.nvar, dtype=torch.uint8, device=dev)
+    check(lib.loc_bed_site_stats(bed.records.data_ptr(), bed.nvar, bed.nsamp, int(min_mac), na.data_ptr(),
+                                 alt.data_ptr(), miss.data_ptr(), keep.data_ptr(), _stream()), "loc_bed_site_stats")
+    return na, alt, miss, keep
+
+
+def bed_pack_sites(bed: BedRecords, site_idx) -> PackedGenotypes:
+    """pack_sites on .bed records: the listed sites -> PackedGenotypes [N, K] (loc_bed_pack_sites)."""
+    idx = _idx(site_idx)
+    K = int(idx.numel())
+    out = PackedGenotypes.empty(bed.nsamp, K)
+    if K:
+        check(lib.loc_bed_pack_sites(bed.records.data_ptr(), bed.nvar, bed.nsamp, idx.data_ptr(), K, out.ptr,
+                                     out.row_words, _stream()), "loc_bed_pack_sites")
+    return out
+
+
+def bed_missing_calls(bed: BedRecords, site_idx: torch.Tensor, n_missing: torch.Tensor):
+    """missing_calls on .bed records: (k, sample) of every missing call of the kept sites in row-major (site,
+    sample) order (loc_bed_missing_calls)."""
+    K = int(site_idx.numel())
+    dev = bed.records.device
+    offsets = torch.zeros(K + 1, dtype=torch.int64, device=dev)
+    null = None
+    check(lib.loc_bed_missing_calls(bed.records.data_ptr(), bed.nvar, bed.nsamp, site_idx.data_ptr(), K,
+                                    n_missing.data_ptr(), offsets.data_ptr(), null, null, _stream()),
+          "loc_bed_missing_calls")
+    total = int(offsets[K].item())
+    ks = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
+    samps = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
+    if total:
+        check(lib.loc_bed_missing_calls(bed.records.data_ptr(), bed.nvar, bed.nsamp, site_idx.data_ptr(), K,
+                                        n_missing.data_ptr(), offsets.data_ptr(), ks.data_ptr(), samps.data_ptr(),
+                                        _stream()), "loc_bed_missing_calls")
+    return ks[:total], samps[:total]

@@ -28,7 +28,7 @@ from . import replicates
 
 
 def build_parser():
-    parser = L.build_parser()
+    parser = L.command_parser()
     parser.prog = "python -m locator_b200.holdout"
     parser.add_argument("--folds", default=10, type=int,
                         help="number of folds k: every located sample is predicted by the model trained on the other "
@@ -124,7 +124,7 @@ def write_predictions(results, locs, norm, samples):
 def main(argv=None):
     ns = build_parser().parse_args(argv)
     check_args(ns)
-    args = L.start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights", "folds"))
+    args = L.start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights", "folds", "bed"))
     check_args(args)  # a --load_params file may ask for one of them
     L.validate_args(args)
     L._write_params()

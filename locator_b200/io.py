@@ -4,7 +4,8 @@ Reference: ``load_genotypes`` /root/reference/locator/locator.py:187-228 --
 ``allel.read_vcf`` (calldata/GT int8 [nvar, N, 2], missing = -1, samples),
 ``zarr.open_group`` (calldata/GT, samples, variants/POS) and the ``--matrix`` table.
 The readers only produce the int8 GT cube on the host; filtering, allele counting and
-packing happen on the GPU (locator_b200.genotypes).
+packing happen on the GPU (locator_b200.genotypes).  PLINK 1 .bed files (``--bed``, an extension of
+this build) are not turned into a cube at all: their 2-bit records go to the device as they are.
 """
 from __future__ import annotations
 
@@ -19,12 +20,13 @@ import numpy as np
 class Genotypes:
     """GT int8 [nvar, N, 2] (missing = -1) + sample IDs (+ positions), as allel.GenotypeArray is used.
 
-    ``gt`` may be a ZarrRows (chunked store on disk): nothing is decoded until ``.gt`` is read, and a
-    variant slice ``g[a:b]`` only decodes the chunks that overlap it (the windows driver, locator.py:538).
+    ``gt`` may be a ZarrRows (chunked store on disk) or a BedRows (PLINK 1 .bed records): nothing is decoded
+    until ``.gt`` is read, and a variant slice ``g[a:b]`` only reads the rows that overlap it (the windows
+    driver, locator.py:538).
     """
 
     def __init__(self, gt, samples=None, positions=None):
-        if isinstance(gt, ZarrRows):
+        if isinstance(gt, (ZarrRows, BedRows)):
             self._lazy, self._gt = gt, None
             assert len(gt.shape) == 3 and gt.shape[2] == 2
         else:
@@ -36,17 +38,20 @@ class Genotypes:
     @property
     def gt(self):
         if self._gt is None:
-            self._gt = np.ascontiguousarray(self._lazy.read(), dtype=np.int8)
+            lazy = self._lazy
+            cube = decode_bed(lazy.read(), lazy.nsamp) if isinstance(lazy, BedRows) else lazy.read()
+            self._gt = np.ascontiguousarray(cube, dtype=np.int8)
         return self._gt
 
     @property
     def rows_on_disk(self):
-        """The ZarrRows behind this object while nothing has been decoded on the host, else None."""
+        """The ZarrRows / BedRows behind this object while nothing has been decoded on the host, else None."""
         return self._lazy if self._gt is None else None
 
     @property
     def lazy(self):
-        """(store path, array name, first row, end row) while nothing has been decoded, else None."""
+        """While nothing has been decoded: where the rows are -- (store path, array name, first row, end row) of a
+        zarr store, (file prefix, first row, end row) of a .bed file; else None."""
         return None if self._gt is not None or self._lazy is None else self._lazy.where()
 
     @property
@@ -251,6 +256,7 @@ class ZarrRows:
         self.b = full[0] if b is None else int(b)
         self.shape = (self.b - self.a,) + full[1:]
         self.dtype = np.dtype(meta["dtype"])
+        self.stored_shape, self.stored_dtype = self.shape, self.dtype  # what read(out=) fills
 
     def rows(self, a, b):
         return ZarrRows(self.root, self.name, self.a + a, self.a + b)
@@ -399,3 +405,152 @@ def write_zarr(path, gt, samples, positions, chunk_variants=65536, compress=True
     put("samples", s, (max(1, s.shape[0]),))
     p = np.asarray(positions, dtype=np.int64)
     put("variants/POS", p, (min(chunk_variants, max(1, p.shape[0])),))
+
+
+# ---------------------------------------------------------------------------------------------
+# PLINK 1 binary fileset (PREFIX.bed / .bim / .fam), SNP-major
+# ---------------------------------------------------------------------------------------------
+BED_MAGIC = b"\x6c\x1b"
+BED_HEADER = 3  # magic bytes + mode byte (0x01: SNP-major)
+# 2-bit code -> GT row; A1 (.bim column 5) is allele index 1, A2 (column 6) allele index 0
+BED_CODE_GT = np.array([[1, 1], [-1, -1], [0, 1], [0, 0]], dtype=np.int8)
+
+
+def read_fam(path):
+    """Sample IDs of a .fam file: column 2 (IID); the family ID is ignored."""
+    with open(path) as fh:
+        return np.array([line.split()[1] for line in fh if line.strip()], dtype=str)
+
+
+def read_bim(path):
+    """(chromosome, position) per variant of a .bim file: columns 1 and 4."""
+    import pandas as pd
+
+    if os.path.getsize(path) == 0:
+        return np.array([], dtype=str), np.array([], dtype=np.int64)
+    t = pd.read_csv(path, sep=r"\s+", header=None, usecols=[0, 3], dtype={0: str, 3: np.int64})
+    return t[0].to_numpy(dtype=str), t[3].to_numpy(dtype=np.int64)
+
+
+def check_bed(path, nvar, nsamp):
+    """Refuse a .bed file this build cannot read for nvar variants and nsamp samples; reads only its header."""
+    with open(path, "rb") as fh:
+        head = fh.read(BED_HEADER)
+    if len(head) < BED_HEADER or head[:2] != BED_MAGIC:
+        raise ValueError(f"{path}: not a PLINK 1 .bed file (magic bytes 6c 1b expected, found {head[:2].hex(' ') or 'none'})")
+    if head[2] == 0:
+        raise ValueError(f"{path}: sample-major .bed (mode byte 0) is not supported; write it SNP-major (mode byte 1), "
+                         "as PLINK does by default")
+    if head[2] != 1:
+        raise ValueError(f"{path}: unknown .bed mode byte {head[2]:#04x} (1 = SNP-major expected)")
+    want = BED_HEADER + nvar * ((nsamp + 3) // 4)
+    size = os.path.getsize(path)
+    if size != want:
+        raise ValueError(f"{path}: {size} bytes, but the {nvar} variants of the .bim and {nsamp} samples of the .fam need "
+                         f"3 + {nvar} x ceil({nsamp}/4) = {want} bytes")
+
+
+class BedRows:
+    """Records [a, b) of a SNP-major .bed file; ``shape`` is that of the GT cube [b - a, N, 2] they stand for.
+    read() gives the raw records, uint8 [b - a, ceil(N/4)] (``stored_shape``); nothing is read before."""
+
+    def __init__(self, prefix, nvar, nsamp, a=None, b=None):
+        self.prefix, self.path = prefix, prefix + ".bed"
+        self.nvar, self.nsamp = int(nvar), int(nsamp)
+        self.record_bytes = (self.nsamp + 3) // 4
+        self.a = 0 if a is None else int(a)
+        self.b = self.nvar if b is None else int(b)
+        self.shape = (self.b - self.a, self.nsamp, 2)
+        self.dtype = np.dtype(np.int8)  # of the cube
+        self.stored_shape, self.stored_dtype = (self.b - self.a, self.record_bytes), np.dtype(np.uint8)
+
+    def rows(self, a, b):
+        return BedRows(self.prefix, self.nvar, self.nsamp, self.a + a, self.a + b)
+
+    def where(self):
+        return (self.prefix, self.a, self.b)
+
+    def read(self, out=None):
+        """The records; with ``out`` (C-contiguous uint8 array of ``stored_shape``, e.g. a view of pinned memory)
+        they are read straight into it, by positioned reads from a few threads."""
+        if out is None:
+            out = np.empty(self.stored_shape, dtype=np.uint8)
+        elif out.shape != self.stored_shape or out.dtype != np.uint8 or not out.flags.c_contiguous:
+            raise ValueError(f"{self.path}: destination must be a C-contiguous uint8 array of shape {self.stored_shape}")
+        nbytes = out.nbytes
+        if nbytes == 0:
+            return out
+        buf = memoryview(out).cast("B")
+        offset = BED_HEADER + self.a * self.record_bytes
+        fd = os.open(self.path, os.O_RDONLY)
+        try:
+            def load(span):
+                lo, hi = span
+                while lo < hi:
+                    n = os.preadv(fd, [buf[lo:hi]], offset + lo)
+                    if n <= 0:
+                        raise ValueError(f"{self.path}: truncated file")
+                    lo += n
+
+            piece = 1 << 26
+            spans = [(lo, min(nbytes, lo + piece)) for lo in range(0, nbytes, piece)]
+            nthreads = min(len(spans), _io_threads())
+            if nthreads > 1:
+                from concurrent.futures import ThreadPoolExecutor
+
+                with ThreadPoolExecutor(nthreads) as pool:  # os.preadv drops the GIL
+                    list(pool.map(load, spans))
+            else:
+                for span in spans:
+                    load(span)
+        finally:
+            os.close(fd)
+        return out
+
+
+def decode_bed(records, nsamp):
+    """uint8 records [nvar, ceil(N/4)] -> GT int8 [nvar, N, 2] (host; the GPU path never builds the cube)."""
+    records = np.asarray(records, dtype=np.uint8)
+    codes = (records[:, :, None] >> np.array([0, 2, 4, 6], dtype=np.uint8)) & 3
+    return BED_CODE_GT[codes.reshape(records.shape[0], -1)[:, :nsamp]]
+
+
+def read_bed(prefix):
+    """PLINK 1 fileset -> dict like read_zarr(lazy=True): 'calldata/GT' (a BedRows: no genotype byte is read
+    here), 'samples' (.fam IIDs), 'variants/POS' and 'variants/CHROM' (.bim).  The .bed header and size are
+    checked against the .bim / .fam."""
+    samples = read_fam(prefix + ".fam")
+    chrom, pos = read_bim(prefix + ".bim")
+    check_bed(prefix + ".bed", len(pos), len(samples))
+    return {"calldata/GT": BedRows(prefix, len(pos), len(samples)), "samples": samples, "variants/POS": pos,
+            "variants/CHROM": chrom}
+
+
+def write_bed(prefix, gt, samples, positions, chrom="1"):
+    """GT int8 [nvar, N, 2] -> PREFIX.bed (SNP-major) / .bim / .fam, the write_zarr of PLINK input.  Refuses what a
+    .bed cannot hold: allele indices >= 2 and calls with one allele missing.  Allele 1 is written as A1."""
+    gt = np.asarray(gt, dtype=np.int8)
+    if gt.ndim != 3 or gt.shape[2] != 2:
+        raise ValueError("write_bed: GT must be [nvar, N, 2]")
+    if (gt >= 2).any():
+        raise ValueError("write_bed: allele indices >= 2 do not fit a .bed (biallelic) file")
+    miss = gt < 0
+    if (miss[:, :, 0] != miss[:, :, 1]).any():
+        raise ValueError("write_bed: half-missing calls do not fit a .bed file")
+    nvar, n = gt.shape[:2]
+    alt = (gt == 1).sum(axis=2)
+    code = np.where(miss[:, :, 0], 1, np.where(alt == 2, 0, np.where(alt == 1, 2, 3))).astype(np.uint8)
+    rb = (n + 3) // 4
+    padded = np.zeros((nvar, rb * 4), dtype=np.uint8)  # pad fields 0
+    padded[:, :n] = code
+    q = padded.reshape(nvar, rb, 4)
+    records = q[:, :, 0] | (q[:, :, 1] << 2) | (q[:, :, 2] << 4) | (q[:, :, 3] << 6)
+    with open(prefix + ".bed", "wb") as fh:
+        fh.write(BED_MAGIC + b"\x01")
+        fh.write(np.ascontiguousarray(records).tobytes())
+    positions = np.asarray(positions, dtype=np.int64)
+    chroms = np.broadcast_to(np.asarray(chrom, dtype=str), positions.shape)
+    with open(prefix + ".bim", "w") as fh:
+        fh.writelines(f"{c}\t{c}:{p}\t0\t{p}\tT\tA\n" for c, p in zip(chroms, positions))
+    with open(prefix + ".fam", "w") as fh:
+        fh.writelines(f"{s}\t{s}\t0\t0\t0\t-9\n" for s in np.asarray(samples).astype(str))

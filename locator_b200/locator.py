@@ -21,6 +21,8 @@ Differences that are deliberate and documented in DESIGN.md:
     reference) come from Philox streams keyed by ``--seed``;
   * weights files are ``.weights.npz`` (no HDF5 on this image) and only exist with --keep_weights
     (the best-epoch checkpoint lives in device memory, not on disk);
+  * ``--bed PREFIX`` (extension, not written to params.json): PLINK 1 .bed input, filtered and packed on the
+    device straight from its 2-bit records (locator_b200.io.BedRows, loc_bed_* kernels);
   * ``--gpus N`` and ``--replicates_per_gpu G`` (extensions, not written to params.json): --bootstrap
     replicates (the FULL model included), --windows replicates and the folds of a k-fold holdout run
     (locator_b200.holdout) are work items of one queue at every GPU count, spread over N GPUs of the box,
@@ -56,7 +58,7 @@ def build_parser():
                         "exactly match those in the VCF. X and Y values for samples without known locations should be NA.")
     parser.add_argument("--train_split", default=0.9, type=float, help="0-1, proportion of samples to use for training. default: 0.9")
     parser.add_argument("--windows", default=False, action="store_true",
-                        help="Run windowed analysis over a single chromosome (requires zarr input).")
+                        help="Run windowed analysis over a single chromosome (requires zarr or --bed input).")
     parser.add_argument("--window_start", default=0, help="default: 0")
     parser.add_argument("--window_stop", default=None, help="default: max snp position")
     parser.add_argument("--window_size", default=5e5, help="default: 500000")
@@ -110,6 +112,17 @@ def build_parser():
     return parser
 
 
+def command_parser():
+    """The parser of the `locator` command: build_parser() plus the genotype input formats of this build (--bed), which
+    the reference's function surface does not have."""
+    parser = build_parser()
+    parser.add_argument("--bed", default=None, metavar="PREFIX",
+                        help="(locator_b200) PLINK 1 binary fileset PREFIX.bed / .bim / .fam (SNP-major) instead of --vcf / "
+                        "--zarr / --matrix: A1 (.bim column 5) is the counted allele, the role ALT plays in a VCF; sample "
+                        "IDs are the .fam IIDs, positions .bim column 4 (--windows: one chromosome). default: None")
+    return parser
+
+
 def set_args(namespace):
     """Install the module-level ``args`` (programmatic use / tests)."""
     global args
@@ -123,6 +136,10 @@ def validate_args(ns):
     from ._cabi import lib  # fails loudly here when the CUDA library is missing
 
     problems = []
+    if getattr(ns, "bed", None) is not None:
+        other = [f"--{k}" for k in ("vcf", "zarr", "matrix") if getattr(ns, k) is not None]
+        if other:
+            problems.append(f"--bed with {' / '.join(other)}: give one genotype input")
     if not 1 <= int(ns.batch_size) <= 256:
         problems.append(f"--batch_size {ns.batch_size}: must be in [1, 256] (up to 32, the reference's default, a step runs "
                         "on the fused tensor-core kernels; 33..256 rows go through the stack in 32-row chunks)")
@@ -231,8 +248,21 @@ def load_genotypes():
     elif args.matrix is not None:
         genotypes = io.read_matrix(args.matrix)
         samples = genotypes.samples
+    elif getattr(args, "bed", None) is not None:
+        print("reading PLINK .bed")
+        try:
+            callset = io.read_bed(args.bed)  # .bim / .fam parsed, .bed header and size checked; no genotype byte read
+        except ValueError as e:
+            raise SystemExit(f"locator: {e}")
+        chroms = np.unique(callset["variants/CHROM"])
+        if args.windows and len(chroms) > 1:
+            raise SystemExit(f"locator: --windows on {args.bed}.bim, which lists {len(chroms)} chromosomes "
+                             f"({', '.join(chroms[:5])}{', ...' if len(chroms) > 5 else ''}): windows are positional and "
+                             "run over a single chromosome")
+        genotypes = io.Genotypes(callset["calldata/GT"], callset["samples"], callset["variants/POS"])
+        samples = callset["samples"]
     else:
-        raise SystemExit("one of --vcf, --zarr or --matrix is required")
+        raise SystemExit("one of --vcf, --zarr, --matrix or --bed is required")
     return genotypes, samples
 
 
@@ -260,7 +290,8 @@ def replace_md(genotypes, stats=None):
     (by the library's restatement of numpy's sampler, nprandom.legacy_binomial); everything around them stays
     on the device: the per-site counts are the ones the site filter already produced (loc_site_stats), the
     list of missing calls comes from loc_missing_calls, the draws are patched into the packed matrix.
-    ``stats`` = (device GT cube, alt_count, n_missing, kept-site indices, packed matrix) from filter_snps;
+    ``stats`` = (device GT cube or .bed records, alt_count, n_missing, kept-site indices, packed matrix) from
+    filter_snps;
     called on its own (as the reference's function can be) it imputes every site of ``genotypes``.
     """
     import torch
@@ -278,7 +309,10 @@ def replace_md(genotypes, stats=None):
     ninds = N - miss[idx].cpu().numpy().astype(np.int64)  # samples with a called genotype
     with np.errstate(divide="ignore", invalid="ignore"):
         af = dc / (2 * ninds)
-    ks, samps = G.missing_calls(g, idx, miss)  # row-major (site, sample) order
+    if isinstance(g, G.BedRecords):
+        ks, samps = G.bed_missing_calls(g, idx, miss)  # row-major (site, sample) order
+    else:
+        ks, samps = G.missing_calls(g, idx, miss)
     if ks.numel():
         from .nprandom import legacy_binomial
 
@@ -289,16 +323,24 @@ def replace_md(genotypes, stats=None):
 
 def filter_snps(genotypes):
     from . import genotypes as G
+    from .io import BedRows
 
     print("filtering SNPs")
     on_disk = getattr(genotypes, "rows_on_disk", None)
-    if on_disk is not None and on_disk.dtype == np.int8:
-        gt = G.upload_rows(on_disk)  # zarr chunks -> pinned staging -> device; the host never holds the cube
+    if isinstance(on_disk, BedRows):
+        # .bed records -> pinned staging -> device as they are on disk (2 bits a call); no cube anywhere
+        g = G.BedRecords.upload(on_disk)
+        n_alleles, alt_count, n_missing, keep = G.bed_site_stats(g, min_mac=int(args.min_mac))
+        keep_idx = G.compact_sites(keep)
+        packed = G.bed_pack_sites(g, keep_idx)
     else:
-        gt = genotypes.gt
-    g, n_alleles, alt_count, n_missing, keep = G.site_stats(gt, min_mac=int(args.min_mac))
-    keep_idx = G.compact_sites(keep)  # device-side prefix sum: the mask never visits the host
-    packed = G.pack_sites(g, keep_idx)
+        if on_disk is not None and on_disk.dtype == np.int8:
+            gt = G.upload_rows(on_disk)  # zarr chunks -> pinned staging -> device; the host never holds the cube
+        else:
+            gt = genotypes.gt
+        g, n_alleles, alt_count, n_missing, keep = G.site_stats(gt, min_mac=int(args.min_mac))
+        keep_idx = G.compact_sites(keep)  # device-side prefix sum: the mask never visits the host
+        packed = G.pack_sites(g, keep_idx)
     if args.impute_missing:
         ac = replace_md(genotypes, (g, alt_count, n_missing, keep_idx, packed))
     else:
@@ -537,7 +579,7 @@ def _jacknife_draws(af, K, n_pred):
     t.join()
 
 
-def start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights")):
+def start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights", "bed")):
     """Install ``ns`` as ``args`` and set the run up as the reference does: seed and gpu (locator.py:170-173),
     load stored parameters (:177-184), seed again in main() (:491-494) -- with --load_params it is the stored
     seed that decides the run's draws.  ``extensions``: flags of this build, kept from the command line (a
@@ -548,7 +590,7 @@ def start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights")):
     if args.gpu_number is not None:
         os.environ["CUDA_VISIBLE_DEVICES"] = args.gpu_number
     if args.load_params is not None:
-        kept = {k: getattr(args, k) for k in extensions}
+        kept = {k: getattr(args, k) for k in extensions if hasattr(args, k)}
         with open(args.load_params, "r") as f:
             args.__dict__ = json.load(f)
         args.__dict__.update(kept)
@@ -562,7 +604,7 @@ def start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights")):
 
 
 def main(argv=None):
-    parser = build_parser()
+    parser = command_parser()
     start_run(parser.parse_args(argv))
     validate_args(args)
     _write_params()
@@ -580,7 +622,7 @@ def _main_body():
     sample_data, locs = sort_samples(samples, genotypes)
     meanlong, sdlong, meanlat, sdlat, locs = normalize_locs(locs)
     norm = (meanlong, sdlong, meanlat, sdlat)
-    if args.windows and args.zarr is not None and windows_are_data_independent():
+    if args.windows and (args.zarr is not None or getattr(args, "bed", None) is not None) and windows_are_data_independent():
         # The reference filters and splits the whole genome before its window loop (main :500-517) and then
         # never uses the result; only the split's draws matter for what follows.  Take the draws, leave the
         # genome on disk: every window decodes just its own chunks (possibly inside a worker process).
@@ -594,8 +636,8 @@ def _main_body():
     if args.windows:
         from . import replicates
 
-        if args.zarr is None:
-            raise SystemExit("--windows requires --zarr input")
+        if args.zarr is None and getattr(args, "bed", None) is None:
+            raise SystemExit("--windows requires --zarr or --bed input")
         replicates.run_windows(sys.modules[__name__], genotypes, samples)
     elif not args.bootstrap and not args.jacknife:
         _run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, 0, None)

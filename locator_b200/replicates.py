@@ -78,16 +78,24 @@ def _prepare(L, item, base):
                 "pred": base["pred"], "samples": base["samples"], "boot": "FULL", "cb_boot": "FULL", "seed_tag": 0,
                 "out": args.out}
     if item["kind"] == "window_lazy":
-        # the window's genotypes are still on disk: decode its chunks, filter and gather here (on this
-        # worker's GPU); the random split was drawn by the parent in the reference's order
+        # the window's genotypes are still on disk: read its zarr chunks / .bed records, filter and gather here (on
+        # this worker's GPU); the random split was drawn by the parent in the reference's order
         from . import io
 
-        root, name, a, b = item["where"]
-        cache = _prepare.__dict__.setdefault("stores", {})
-        if root not in cache:
-            cache[root] = io.read_zarr(root, lazy=True)
-        cs = cache[root]
-        sub = io.Genotypes(io.ZarrRows(root, name, a, b), cs["samples"], cs["variants/POS"][a:b])
+        cache = _prepare.__dict__.setdefault("stores", {})  # zarr metadata / parsed .bim + .fam, once per process
+        if item.get("format") == "bed":
+            prefix, a, b = item["where"]
+            if ("bed", prefix) not in cache:
+                cache[("bed", prefix)] = io.read_bed(prefix)
+            cs = cache[("bed", prefix)]
+            rows = cs["calldata/GT"].rows(a, b)
+        else:
+            root, name, a, b = item["where"]
+            if root not in cache:
+                cache[root] = io.read_zarr(root, lazy=True)
+            cs = cache[root]
+            rows = io.ZarrRows(root, name, a, b)
+        sub = io.Genotypes(rows, cs["samples"], cs["variants/POS"][a:b])
         ac = L.filter_snps(sub)
         locs = item["locs"]
         train, test, traingen, testgen, trainlocs, testlocs, pred, predgen = L.split_train_test(ac, locs, item["drawn"])
@@ -543,6 +551,8 @@ def window_bounds(positions, start, stop, size):
 
 
 def run_windows(L, genotypes, samples):
+    from . import io
+
     args = L.args
     positions = np.array(genotypes.positions)
     start = int(args.window_start)
@@ -562,7 +572,8 @@ def run_windows(L, genotypes, samples):
             meanlong, sdlong, meanlat, sdlat, locs = L.normalize_locs(locs)
             if sub.lazy is not None and recipes_ok:
                 yield {"kind": "window_lazy", "index": index, "window_out": f"{args.out}_{i}-{i+size-1}",
-                       "where": sub.lazy, "locs": locs, "drawn": L.draw_split(locs),
+                       "where": sub.lazy, "format": "bed" if isinstance(sub.rows_on_disk, io.BedRows) else "zarr",
+                       "locs": locs, "drawn": L.draw_split(locs),
                        "norm": (meanlong, sdlong, meanlat, sdlat), "samples": samples}
                 continue
             ac = L.filter_snps(sub)
