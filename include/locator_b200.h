@@ -34,7 +34,12 @@
  *   - packed genotype matrix: sample-major, 2 bits per genotype (alt-allele count
  *     0/1/2), 16 genotypes per little-endian uint32 (SNP k of a row lives in word
  *     k/16, bits 2*(k%16)..+1), row pitch `row_words` uint32 (>= ceil(K/16),
- *     multiple of 4 so rows are 16-byte aligned); pad bits are zero.
+ *     multiple of 4 so rows are 16-byte aligned); pad bits are zero.  Code 3
+ *     never occurs in a matrix a model trains on: the mapped packs of a query
+ *     (loc_pack_sites_mapped / loc_bed_pack_sites_mapped) write it for a missing
+ *     call or a site the query lacks, and the inference forward
+ *     (loc_predict / loc_eval) gives it xhat = beta, BatchNorm's output at the
+ *     moving mean (mean imputation).
  *   - there is NO CPU fallback: every entry point fails if CUDA is unavailable.
  */
 #ifndef LOCATOR_B200_H
@@ -125,6 +130,17 @@ int loc_bed_pack_sites(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const 
                        uint32_t* d_packed, int64_t row_words, void* stream);
 int loc_bed_missing_calls(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
                           const int32_t* d_n_missing, int64_t* d_offsets, int64_t* d_k, int64_t* d_samp, void* stream);
+
+/* A query's genotypes in a stored model's site order (python -m locator_b200.predict): the layout of
+ * loc_pack_sites, where model site k takes query record d_src[k] (< nvar; -1 = the query lacks the site; duplicates
+ * allowed) and d_flip[k] != 0 swaps the roles of alleles 0 and 1 (the query's REF is the model's ALT).  A call with
+ * both alleles in {0, 1} packs its count of allele 1 (2 - that count when flipped); any other call (missing,
+ * half-missing, an allele index >= 2) and every call of an absent site packs 3.  The .bed variant reads records as
+ * loc_bed_pack_sites does (missing, code 1 -> 3; A2 counted when flipped). */
+int loc_pack_sites_mapped(const int8_t* d_gt, int64_t nvar, int64_t nsamp, const int64_t* d_src, const uint8_t* d_flip,
+                          int64_t K, uint32_t* d_packed, int64_t row_words, void* stream);
+int loc_bed_pack_sites_mapped(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_src,
+                              const uint8_t* d_flip, int64_t K, uint32_t* d_packed, int64_t row_words, void* stream);
 
 /* Overwrite individual genotypes (imputation results of replace_md, :258-261):
  * packed[d_samp[i]][d_k[i]] = d_val[i], i < n.  (k indexes packed columns.) */

@@ -51,6 +51,8 @@ SIGNATURES = {
     "loc_bed_site_stats": (C.c_int, [P, I64, I64, I32, P, P, P, P, P]),
     "loc_bed_pack_sites": (C.c_int, [P, I64, I64, P, I64, P, I64, P]),
     "loc_bed_missing_calls": (C.c_int, [P, I64, I64, P, I64, P, P, P, P, P]),
+    "loc_pack_sites_mapped": (C.c_int, [P, I64, I64, P, P, I64, P, I64, P]),
+    "loc_bed_pack_sites_mapped": (C.c_int, [P, I64, I64, P, P, I64, P, I64, P]),
     "loc_site_sums": (C.c_int, [P, I64, I64, I64, P, P]),
     "loc_patch_calls": (C.c_int, [P, I64, P, P, P, I64, P]),
     "loc_pack_counts": (C.c_int, [P, I64, I64, P, I64, P]),

@@ -175,6 +175,9 @@ __global__ void __launch_bounds__(256, 4) k_site_stats(const int8_t* __restrict_
 // into 64 contiguous bytes per sample for the write.  Blocks that are adjacent in x cover one set of
 // sites across all samples, so concurrently running blocks read whole rows.
 // The host picks the widest VB for which every load is aligned (VB | 2N and the base pointer).
+// MAPPED (loc_pack_sites_mapped): site_idx[k] is the query record of model site k or -1 (absent), and flip[k] swaps
+// the roles of alleles 0 and 1; a call with both alleles in {0, 1} packs its count of allele 1 (of allele 0 when
+// flipped), any other call -- and every call of an absent site -- packs 3.
 // ---------------------------------------------------------------------------------------------
 template <int VB>
 __device__ __forceinline__ void load_calls(const int8_t* p, uint32_t (&w)[(VB + 3) / 4]) {
@@ -194,9 +197,10 @@ __device__ __forceinline__ void load_calls(const int8_t* p, uint32_t (&w)[(VB + 
 constexpr int kPackWords = 16;  // packed words (of 16 sites) per block
 constexpr int kPackPitch = kPackWords + 1;
 
-template <int VB>
+template <int VB, bool MAPPED>
 __global__ void __launch_bounds__(256) k_pack_sites(const int8_t* __restrict__ gt, int64_t nsamp,
-                                                    const int64_t* __restrict__ site_idx, int64_t K,
+                                                    const int64_t* __restrict__ site_idx,
+                                                    const uint8_t* __restrict__ flip, int64_t K,
                                                     uint32_t* __restrict__ packed, int64_t row_words) {
   constexpr int CALLS = VB / 2;
   constexpr int S = 32 * CALLS;
@@ -211,11 +215,23 @@ __global__ void __launch_bounds__(256) k_pack_sites(const int8_t* __restrict__ g
     const int wl = 2 * wi + jw;
     const int64_t k0 = (w0 + wl) * 16;
     uint32_t raw[16][NW];
+    uint32_t flips = 0u;  // MAPPED: bit q = site k0 + q is flipped
 #pragma unroll
     for (int q = 0; q < 16; ++q) {
 #pragma unroll
       for (int e = 0; e < NW; ++e) raw[q][e] = 0u;
-      if (k0 + q < K && sb < nsamp) load_calls<VB>(gt + (__ldg(site_idx + k0 + q) * nsamp + sb) * 2, raw[q]);
+      if (k0 + q < K && sb < nsamp) {
+        const int64_t src = __ldg(site_idx + k0 + q);
+        if constexpr (MAPPED) {
+          flips |= (__ldg(flip + k0 + q) != 0 ? 1u : 0u) << q;
+          if (src < 0) {
+#pragma unroll
+            for (int e = 0; e < NW; ++e) raw[q][e] = 0xFFFFFFFFu;  // absent: every allele missing
+            continue;
+          }
+        }
+        load_calls<VB>(gt + (src * nsamp + sb) * 2, raw[q]);
+      }
     }
     uint32_t acc[CALLS];
 #pragma unroll
@@ -225,7 +241,14 @@ __global__ void __launch_bounds__(256) k_pack_sites(const int8_t* __restrict__ g
 #pragma unroll
       for (int e = 0; e < NW; ++e) {
         const uint32_t e1 = zero_bytes(raw[q][e] ^ 0x01010101u) >> 7;         // 1 where the allele is 1
-        const uint32_t g2 = (e1 + (e1 >> 8)) & 0x00030003u;                   // count of call A | call B << 16
+        uint32_t g2 = (e1 + (e1 >> 8)) & 0x00030003u;                         // count of call A | call B << 16
+        if constexpr (MAPPED) {
+          const uint32_t e0 = zero_bytes(raw[q][e]) >> 7;                     // 1 where the allele is 0
+          const uint32_t ok = e0 | e1;
+          const uint32_t bad = (ok & (ok >> 8) & 0x00010001u) ^ 0x00010001u;  // call with an allele outside {0, 1}
+          if ((flips >> q) & 1u) g2 = (e0 + (e0 >> 8)) & 0x00030003u;
+          g2 |= bad * 3u;
+        }
         acc[2 * e] |= (g2 & 3u) << (2 * q);
         if constexpr (CALLS > 1) acc[2 * e + 1] |= (g2 >> 16) << (2 * q);
       }
@@ -540,6 +563,13 @@ __device__ __forceinline__ uint32_t bed_counts(uint32_t x) {
   return ((~(lo | hi) & 0x55555555u) << 1) | (hi & ~lo);
 }
 
+// codes of 16 fields -> the packed value of the mapped pack: copies of A1 {0 -> 2, 2 -> 1, 3 -> 0}, or of A2 when
+// flipped {0 -> 0, 2 -> 1, 3 -> 2}; missing (code 1) -> 3
+__device__ __forceinline__ uint32_t bed_counts_mapped(uint32_t x, bool flip) {
+  const uint32_t lo = x & 0x55555555u, hi = (x >> 1) & 0x55555555u;
+  return ((flip ? lo : ~hi & 0x55555555u) << 1) | (lo ^ hi);
+}
+
 // the 4 record bytes at p (any alignment) as one word, from the aligned words that hold them; the word after the
 // record area (end) is not read
 __device__ __forceinline__ uint32_t bed_word(const uint8_t* p, uintptr_t end) {
@@ -576,11 +606,13 @@ __device__ __forceinline__ void transpose16x2(uint32_t (&r)[16]) {
 // word a lane loads the piece of each of the 16 records, maps the codes, and transposes the 16 x 16 block in
 // registers, which gives its 16 samples' words.  A padded shared-memory tile turns them into 64 contiguous bytes
 // per sample for the write (the layout of k_pack_sites).  The blocks of one grid row loop over the word groups, so
-// any K fits one launch.
+// any K fits one launch.  MAPPED (loc_bed_pack_sites_mapped): site_idx / flip as in k_pack_sites.
 constexpr int kBedPackSamples = 512;
 
+template <bool MAPPED>
 __global__ void __launch_bounds__(256) k_bed_pack_sites(const uint8_t* __restrict__ bed, int64_t nvar, int64_t nsamp,
-                                                        const int64_t* __restrict__ site_idx, int64_t K,
+                                                        const int64_t* __restrict__ site_idx,
+                                                        const uint8_t* __restrict__ flip, int64_t K,
                                                         uint32_t* __restrict__ packed, int64_t row_words) {
   __shared__ uint32_t tile[kBedPackSamples * kPackPitch];  // [sample j of the lane][lane][word], pitch 17
   const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
@@ -597,8 +629,18 @@ __global__ void __launch_bounds__(256) k_bed_pack_sites(const uint8_t* __restric
       const int64_t k0 = (w0 + wl) * 16;
       uint32_t r[16];
 #pragma unroll
-      for (int q = 0; q < 16; ++q)
-        r[q] = (k0 + q < K && byte0 < rb) ? bed_counts(bed_word(bed + __ldg(site_idx + k0 + q) * rb + byte0, end)) : 0u;
+      for (int q = 0; q < 16; ++q) {
+        if constexpr (MAPPED) {
+          r[q] = 0u;
+          if (k0 + q < K && byte0 < rb) {
+            const int64_t src = __ldg(site_idx + k0 + q);
+            r[q] = src < 0 ? 0xFFFFFFFFu  // absent: code 3 for every sample
+                           : bed_counts_mapped(bed_word(bed + src * rb + byte0, end), __ldg(flip + k0 + q) != 0);
+          }
+        } else {
+          r[q] = (k0 + q < K && byte0 < rb) ? bed_counts(bed_word(bed + __ldg(site_idx + k0 + q) * rb + byte0, end)) : 0u;
+        }
+      }
       transpose16x2(r);  // r[j] = the word of sample s0 + 16 * lane + j
 #pragma unroll
       for (int j = 0; j < 16; ++j) tile[(j * 32 + lane) * kPackPitch + wl] = r[j];
@@ -671,6 +713,55 @@ __global__ void __launch_bounds__(128) k_site_sums(const uint32_t* __restrict__ 
 }  // namespace loc
 
 using namespace loc;
+
+// launchers of the plain and the mapped variant of the two pack kernels
+template <bool MAPPED>
+static int pack_sites_launch(const char* what, const int8_t* d_gt, int64_t nsamp, const int64_t* d_idx,
+                             const uint8_t* d_flip, int64_t K, uint32_t* d_packed, int64_t row_words, void* stream) {
+  LOC_CHECK(nsamp > 0 && K >= 0, (std::string(what) + ": bad shape").c_str());
+  LOC_CHECK(row_words >= cdiv(K, 16) && row_words % 4 == 0, (std::string(what) + ": row_words must be >= ceil(K/16) and a multiple of 4").c_str());
+  if (row_words == 0) return 0;
+  LOC_CHECK(d_gt != nullptr && d_packed != nullptr, (std::string(what) + ": null pointer").c_str());
+  LOC_CHECK(!MAPPED || K == 0 || (d_idx != nullptr && d_flip != nullptr), (std::string(what) + ": null pointer").c_str());
+  LOC_CHECK(reinterpret_cast<uintptr_t>(d_packed) % 16 == 0, (std::string(what) + ": packed rows must be 16-byte aligned").c_str());
+  // widest aligned load: VB bytes = VB / 2 calls per lane
+  const uintptr_t base = reinterpret_cast<uintptr_t>(d_gt);
+  int vb = 16;
+  while (vb > 2 && ((nsamp * 2) % vb != 0 || base % vb != 0)) vb >>= 1;
+  LOC_CHECK(base % 2 == 0, (std::string(what) + ": genotype pointer must be 2-byte aligned").c_str());
+  const int S = 32 * (vb / 2);
+  const int64_t wgroups = cdiv(row_words, kPackWords);
+  const int64_t gy = wgroups < 32768 ? wgroups : 32768;
+  dim3 grid((unsigned)cdiv(nsamp, S), (unsigned)gy, (unsigned)cdiv(wgroups, gy));  // blocks past row_words write nothing
+  LOC_CHECK(grid.z <= 65535, (std::string(what) + ": K too large for one launch").c_str());
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (vb) {
+    case 16: k_pack_sites<16, MAPPED><<<grid, 256, 0, st>>>(d_gt, nsamp, d_idx, d_flip, K, d_packed, row_words); break;
+    case 8: k_pack_sites<8, MAPPED><<<grid, 256, 0, st>>>(d_gt, nsamp, d_idx, d_flip, K, d_packed, row_words); break;
+    case 4: k_pack_sites<4, MAPPED><<<grid, 256, 0, st>>>(d_gt, nsamp, d_idx, d_flip, K, d_packed, row_words); break;
+    default: k_pack_sites<2, MAPPED><<<grid, 256, 0, st>>>(d_gt, nsamp, d_idx, d_flip, K, d_packed, row_words); break;
+  }
+  LOC_LAUNCHED();
+  return 0;
+}
+
+template <bool MAPPED>
+static int bed_pack_launch(const char* what, const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_idx,
+                           const uint8_t* d_flip, int64_t K, uint32_t* d_packed, int64_t row_words, void* stream) {
+  LOC_CHECK(nvar >= 0 && nsamp > 0 && K >= 0, (std::string(what) + ": bad shape").c_str());
+  LOC_CHECK(row_words >= cdiv(K, 16) && row_words % 4 == 0, (std::string(what) + ": row_words must be >= ceil(K/16) and a multiple of 4").c_str());
+  if (row_words == 0) return 0;
+  LOC_CHECK(d_packed != nullptr && (K == 0 || (d_bed != nullptr && d_idx != nullptr && (!MAPPED || d_flip != nullptr))),
+            (std::string(what) + ": null pointer").c_str());
+  LOC_CHECK(reinterpret_cast<uintptr_t>(d_packed) % 16 == 0, (std::string(what) + ": packed rows must be 16-byte aligned").c_str());
+  LOC_CHECK(cdiv(nsamp, kBedPackSamples) <= 0x7fffffff, (std::string(what) + ": too many samples").c_str());
+  const int64_t wgroups = cdiv(row_words, kPackWords);
+  dim3 grid((unsigned)cdiv(nsamp, kBedPackSamples), (unsigned)(wgroups < 65535 ? wgroups : 65535));
+  k_bed_pack_sites<MAPPED><<<grid, 256, 0, (cudaStream_t)stream>>>(d_bed, nvar, nsamp, d_idx, d_flip, K, d_packed,
+                                                                    row_words);
+  LOC_LAUNCHED();
+  return 0;
+}
 
 extern "C" {
 
@@ -777,30 +868,13 @@ int loc_site_sums(const uint32_t* d_packed, int64_t n, int64_t K, int64_t row_wo
 int loc_pack_sites(const int8_t* d_gt, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
                    uint32_t* d_packed, int64_t row_words, void* stream) {
   (void)nvar;
-  LOC_CHECK(nsamp > 0 && K >= 0, "loc_pack_sites: bad shape");
-  LOC_CHECK(row_words >= cdiv(K, 16) && row_words % 4 == 0, "loc_pack_sites: row_words must be >= ceil(K/16) and a multiple of 4");
-  if (row_words == 0) return 0;
-  LOC_CHECK(d_gt != nullptr && d_packed != nullptr, "loc_pack_sites: null pointer");
-  LOC_CHECK(reinterpret_cast<uintptr_t>(d_packed) % 16 == 0, "loc_pack_sites: packed rows must be 16-byte aligned");
-  // widest aligned load: VB bytes = VB / 2 calls per lane
-  const uintptr_t base = reinterpret_cast<uintptr_t>(d_gt);
-  int vb = 16;
-  while (vb > 2 && ((nsamp * 2) % vb != 0 || base % vb != 0)) vb >>= 1;
-  LOC_CHECK(base % 2 == 0, "loc_pack_sites: genotype pointer must be 2-byte aligned");
-  const int S = 32 * (vb / 2);
-  const int64_t wgroups = cdiv(row_words, kPackWords);
-  const int64_t gy = wgroups < 32768 ? wgroups : 32768;
-  dim3 grid((unsigned)cdiv(nsamp, S), (unsigned)gy, (unsigned)cdiv(wgroups, gy));  // blocks past row_words write nothing
-  LOC_CHECK(grid.z <= 65535, "loc_pack_sites: K too large for one launch");
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (vb) {
-    case 16: k_pack_sites<16><<<grid, 256, 0, st>>>(d_gt, nsamp, d_site_idx, K, d_packed, row_words); break;
-    case 8: k_pack_sites<8><<<grid, 256, 0, st>>>(d_gt, nsamp, d_site_idx, K, d_packed, row_words); break;
-    case 4: k_pack_sites<4><<<grid, 256, 0, st>>>(d_gt, nsamp, d_site_idx, K, d_packed, row_words); break;
-    default: k_pack_sites<2><<<grid, 256, 0, st>>>(d_gt, nsamp, d_site_idx, K, d_packed, row_words); break;
-  }
-  LOC_LAUNCHED();
-  return 0;
+  return pack_sites_launch<false>("loc_pack_sites", d_gt, nsamp, d_site_idx, nullptr, K, d_packed, row_words, stream);
+}
+
+int loc_pack_sites_mapped(const int8_t* d_gt, int64_t nvar, int64_t nsamp, const int64_t* d_src, const uint8_t* d_flip,
+                          int64_t K, uint32_t* d_packed, int64_t row_words, void* stream) {
+  (void)nvar;
+  return pack_sites_launch<true>("loc_pack_sites_mapped", d_gt, nsamp, d_src, d_flip, K, d_packed, row_words, stream);
 }
 
 int loc_bed_site_stats(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, int32_t min_mac, int32_t* d_n_alleles,
@@ -824,19 +898,14 @@ int loc_bed_site_stats(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, int32_
 
 int loc_bed_pack_sites(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,
                        uint32_t* d_packed, int64_t row_words, void* stream) {
-  LOC_CHECK(nvar >= 0 && nsamp > 0 && K >= 0, "loc_bed_pack_sites: bad shape");
-  LOC_CHECK(row_words >= cdiv(K, 16) && row_words % 4 == 0,
-            "loc_bed_pack_sites: row_words must be >= ceil(K/16) and a multiple of 4");
-  if (row_words == 0) return 0;
-  LOC_CHECK(d_packed != nullptr && (K == 0 || (d_bed != nullptr && d_site_idx != nullptr)),
-            "loc_bed_pack_sites: null pointer");
-  LOC_CHECK(reinterpret_cast<uintptr_t>(d_packed) % 16 == 0, "loc_bed_pack_sites: packed rows must be 16-byte aligned");
-  LOC_CHECK(cdiv(nsamp, kBedPackSamples) <= 0x7fffffff, "loc_bed_pack_sites: too many samples");
-  const int64_t wgroups = cdiv(row_words, kPackWords);
-  dim3 grid((unsigned)cdiv(nsamp, kBedPackSamples), (unsigned)(wgroups < 65535 ? wgroups : 65535));
-  k_bed_pack_sites<<<grid, 256, 0, (cudaStream_t)stream>>>(d_bed, nvar, nsamp, d_site_idx, K, d_packed, row_words);
-  LOC_LAUNCHED();
-  return 0;
+  return bed_pack_launch<false>("loc_bed_pack_sites", d_bed, nvar, nsamp, d_site_idx, nullptr, K, d_packed, row_words,
+                                stream);
+}
+
+int loc_bed_pack_sites_mapped(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_src,
+                              const uint8_t* d_flip, int64_t K, uint32_t* d_packed, int64_t row_words, void* stream) {
+  return bed_pack_launch<true>("loc_bed_pack_sites_mapped", d_bed, nvar, nsamp, d_src, d_flip, K, d_packed, row_words,
+                               stream);
 }
 
 int loc_bed_missing_calls(const uint8_t* d_bed, int64_t nvar, int64_t nsamp, const int64_t* d_site_idx, int64_t K,

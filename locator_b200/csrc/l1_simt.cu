@@ -88,10 +88,16 @@ __global__ void __launch_bounds__(1024) k_l1_fwd_simt(L1Args a, int n_partials) 
         }
         const float inv = rsqrtf(var + kBnEps) * a.gamma[k];
         const float shift = a.beta[k] - mean * inv;
+        const unsigned long long miss = sb.bits & (sb.bits >> 1) & 0x5555555555555555ull;  // x = 3 at bit 2b
         for (int b = 0; b < kMaxB; ++b) {
           const float x = (float)((sb.bits >> (2 * b)) & 3ull);
           row[b] = (b < nb) ? x * inv + shift : 0.f;
         }
+        // x = 3 (missing call or absent site of a query, never in training): xhat = beta, BatchNorm's output at the
+        // moving mean
+        if (miss != 0ull)
+          for (int b = 0; b < nb; ++b)
+            if ((miss >> (2 * b)) & 1ull) row[b] = a.beta[k];
       } else {
         for (int b = 0; b < kMaxB; ++b) row[b] = 0.f;
       }

@@ -324,6 +324,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) k_l1_fwd_tc(L1Args a, int64_t nt
       }
       __syncwarp();
       float mean, var;
+      float miss = 0.f;  // x = 3 (missing call or absent site of a query, never in training): xhat = beta
       if (a.training) {
         moments_from_counts(n1, n2, nb, mean, var);
         if (valid) {
@@ -333,6 +334,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) k_l1_fwd_tc(L1Args a, int64_t nt
       } else {
         mean = mm;
         var = mv;
+        miss = valid ? to_tf32(beta) : 0.f;
       }
       const float inv = rsqrtf(var + kBnEps) * gamma;
       const float shift = beta - mean * inv;
@@ -349,9 +351,8 @@ __global__ void __launch_bounds__(F_THREADS, 1) k_l1_fwd_tc(L1Args a, int64_t nt
         for (int e = 0; e < 4; ++e) {
           const int b = 4 * c + e;
           const unsigned x = (unsigned)((g >> (2 * b)) & 3ull);
-          float val = lut[0];  // branch-free select (the lanes of a warp hold different genotypes)
-          val = x == 1u ? lut[1] : val;
-          val = x == 2u ? lut[2] : val;
+          // branch-free select (the lanes of a warp hold different genotypes)
+          const float val = (x & 2u) ? ((x & 1u) ? miss : lut[2]) : ((x & 1u) ? lut[1] : lut[0]);
           v[e] = b < nb ? val : 0.f;
         }
         *reinterpret_cast<float4*>(xrow + swz32(lane, c)) = make_float4(v[0], v[1], v[2], v[3]);
@@ -523,10 +524,13 @@ __global__ void __launch_bounds__(W_THREADS, 1) k_l1_fwd_wide(L1Args a, int64_t 
         // version transposed the genotypes through shared memory instead, 32 loads + ~130 integer instructions per
         // lane and stage: 23 % of the kernel's samples.)
         const float inv = rsqrtf(mv + kBnEps) * gamma;  // inference: moving statistics
-        const float shift = beta - mm * inv;
+        // fused as it always was: beta's use in the code-3 slot below would otherwise leave it a multiply and a
+        // subtraction, and move the tf32 images of the three genotype values
+        const float shift = fmaf(-mm, inv, beta);
         __syncwarp();  // the previous stage's table has been read by every lane
+        // x = 3 (missing call or absent site of a query): xhat = beta, BatchNorm's output at the moving mean
         lutw[lane] = make_float4(valid ? to_tf32(shift) : 0.f, valid ? to_tf32(inv + shift) : 0.f,
-                                 valid ? to_tf32(2.f * inv + shift) : 0.f, 0.f);
+                                 valid ? to_tf32(2.f * inv + shift) : 0.f, valid ? to_tf32(beta) : 0.f);
         __syncwarp();
         mbar_wait(&empty[s], ph ^ 1u);
         uint8_t* xrow = sX + s * W_XBYTES + wi * F_CHUNK + (lane & 3) * 4;

@@ -335,3 +335,24 @@ def bed_missing_calls(bed: BedRecords, site_idx: torch.Tensor, n_missing: torch.
                                         n_missing.data_ptr(), offsets.data_ptr(), ks.data_ptr(), samps.data_ptr(),
                                         _stream()), "loc_bed_missing_calls")
     return ks[:total], samps[:total]
+
+
+def pack_sites_mapped(g, src, flip) -> PackedGenotypes:
+    """A query in a stored model's site order: PackedGenotypes [N, K] where column k is query record src[k] (-1:
+    absent) of device GT int8 [nvar, N, 2] (GT cube) or BedRecords, allele roles swapped where flip[k]; missing
+    calls, calls with an allele index >= 2 and absent sites are 3 (loc_pack_sites_mapped / loc_bed_pack_sites_mapped)."""
+    s = _idx(src)
+    f = _as_dev(flip, torch.uint8)
+    K = int(s.numel())
+    if isinstance(g, BedRecords):
+        out = PackedGenotypes.empty(g.nsamp, K)
+        if K:
+            check(lib.loc_bed_pack_sites_mapped(g.records.data_ptr(), g.nvar, g.nsamp, s.data_ptr(), f.data_ptr(), K,
+                                                out.ptr, out.row_words, _stream()), "loc_bed_pack_sites_mapped")
+        return out
+    nvar, N, _ = g.shape
+    out = PackedGenotypes.empty(N, K)
+    if K:
+        check(lib.loc_pack_sites_mapped(g.data_ptr(), nvar, N, s.data_ptr(), f.data_ptr(), K, out.ptr, out.row_words,
+                                        _stream()), "loc_pack_sites_mapped")
+    return out

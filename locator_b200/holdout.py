@@ -15,6 +15,7 @@ Every numpy draw is taken serially in this process, so the outputs do not depend
   {out}_holdout_predlocs.txt     x,y,sampleID,fold -- one row per located sample, ascending sample index
   {out}_holdout{f}_history.txt   per fold
   {out}_holdout{f}.weights.npz   per fold, with --keep_weights
+  {out}_holdout{f}.sites.tsv     per fold, with --keep_weights --keep_sites (python -m locator_b200.predict)
   {out}_params.json              as a plain locator run writes it
 """
 from __future__ import annotations
@@ -86,7 +87,7 @@ def predict_fold(model, history, rep):
 def run(ac, locs, norm, samples, folds):
     """Train and predict every fold through the replicate queue; returns the fold results in fold order."""
     args = L.args
-    base = {"genotypes": ac.packed, "locs": locs, "norm": norm, "samples": samples}
+    base = {"genotypes": ac.packed, "locs": locs, "norm": norm, "samples": samples, "sites": ac.sites}
     items = [{"kind": "fold", "fold": f, "held": held, "train": train, "val": val, "fold_out": f"{args.out}_holdout{f}"}
              for f, (held, train, val) in enumerate(folds)]
     return replicates.run_work(L, items, base)
@@ -124,7 +125,7 @@ def write_predictions(results, locs, norm, samples):
 def main(argv=None):
     ns = build_parser().parse_args(argv)
     check_args(ns)
-    args = L.start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights", "folds", "bed"))
+    args = L.start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights", "folds", "bed", "keep_sites"))
     check_args(args)  # a --load_params file may ask for one of them
     L.validate_args(args)
     L._write_params()

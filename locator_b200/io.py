@@ -12,6 +12,7 @@ from __future__ import annotations
 import gzip
 import json
 import os
+import re
 import zlib
 
 import numpy as np
@@ -22,10 +23,11 @@ class Genotypes:
 
     ``gt`` may be a ZarrRows (chunked store on disk) or a BedRows (PLINK 1 .bed records): nothing is decoded
     until ``.gt`` is read, and a variant slice ``g[a:b]`` only reads the rows that overlap it (the windows
-    driver, locator.py:538).
+    driver, locator.py:538).  ``ids``: optional {"chrom", "ref", "alt"} string arrays per variant (site identity:
+    REF is allele index 0, ALT allele index 1), needed to record or match a model's sites (locator_b200.sites).
     """
 
-    def __init__(self, gt, samples=None, positions=None):
+    def __init__(self, gt, samples=None, positions=None, ids=None):
         if isinstance(gt, (ZarrRows, BedRows)):
             self._lazy, self._gt = gt, None
             assert len(gt.shape) == 3 and gt.shape[2] == 2
@@ -34,6 +36,7 @@ class Genotypes:
             assert self._gt.ndim == 3 and self._gt.shape[2] == 2
         self.samples = None if samples is None else np.asarray(samples)
         self.positions = None if positions is None else np.asarray(positions)
+        self.ids = ids
 
     @property
     def gt(self):
@@ -66,10 +69,20 @@ class Genotypes:
         if isinstance(key, tuple):
             key = key[0]
         pos = None if self.positions is None else self.positions[key]
+        ids = None if self.ids is None else {k: v[key] for k, v in self.ids.items()}
         if self._gt is None and isinstance(key, slice) and key.step in (None, 1):
             a, b, _ = key.indices(self._lazy.shape[0])
-            return Genotypes(self._lazy.rows(a, max(a, b)), self.samples, pos)
-        return Genotypes(self.gt[key], self.samples, pos)
+            return Genotypes(self._lazy.rows(a, max(a, b)), self.samples, pos, ids)
+        return Genotypes(self.gt[key], self.samples, pos, ids)
+
+
+def variant_ids(callset):
+    """{"chrom", "ref", "alt"} of a reader's dict (read_vcf(sites=True) / read_zarr / read_bed), or None when the
+    input does not name its alleles."""
+    keys = ("variants/CHROM", "variants/REF", "variants/ALT")
+    if not all(k in callset for k in keys):
+        return None
+    return {n: np.asarray(callset[k]) for n, k in zip(("chrom", "ref", "alt"), keys)}
 
 
 def _open_bytes(path):
@@ -108,14 +121,35 @@ def _read_vcf_native(data):
     return {"calldata/GT": gt, "samples": samples, "variants/POS": pos}
 
 
-def read_vcf(path):
-    """VCF / VCF.gz -> dict like allel.read_vcf: 'calldata/GT', 'samples', 'variants/POS'.
+_VCF_IDS = re.compile(rb"^([^#\n][^\t\n]*)\t[^\t\n]*\t[^\t\n]*\t([^\t\n]*)\t([^\t\n,]*)", re.M)
+
+
+def _vcf_ids(data, nvar, path):
+    """CHROM, REF and the first ALT allele (allele index 1) of every data line."""
+    rows = _VCF_IDS.findall(data)
+    if len(rows) != nvar:
+        raise ValueError(f"{path}: {len(rows)} data lines with CHROM / REF / ALT columns for {nvar} variants")
+    cols = list(zip(*rows)) if rows else [(), (), ()]
+    return {k: np.array([x.decode() for x in c], dtype=str) for k, c in
+            zip(("variants/CHROM", "variants/REF", "variants/ALT"), cols)}
+
+
+def read_vcf(path, sites=False):
+    """VCF / VCF.gz -> dict like allel.read_vcf: 'calldata/GT', 'samples', 'variants/POS'; with sites=True also
+    'variants/CHROM', 'variants/REF' and 'variants/ALT' (the first ALT allele: the one GT index 1 names).
 
     Fast path: FORMAT is exactly GT and every call is 3 bytes (``0|1``, ``./.``) -- one numpy view
     per line.  Anything else goes through a per-field parser (multi-digit alleles, extra FORMAT
     keys, haploid calls -> second allele -1).
     """
     data = _open_bytes(path)
+    out = _read_vcf(data, path)
+    if sites:
+        out.update(_vcf_ids(data, len(out["variants/POS"]), path))
+    return out
+
+
+def _read_vcf(data, path):
     if not os.environ.get("LOC_PY_VCF"):
         fast = _read_vcf_native(data)
         if fast is not None:
@@ -361,18 +395,32 @@ def _zarr_array(root, name, rows=None, out=None):
     return out
 
 
-def read_zarr(path, lazy=False):
+def _zarr_strings(path, name):
+    """A string array of the store as str (fixed-width bytes or vlen-utf8); 2-D (allel's variants/ALT): column 0."""
+    a = _zarr_array(path, name)
+    if a.ndim == 2:
+        a = a[:, 0]
+    return np.array([x.decode() if isinstance(x, bytes) else str(x) for x in a], dtype=str)
+
+
+def read_zarr(path, lazy=False, sites=False):
     """zarr v2 group with calldata/GT, samples, variants/POS -> dict (arrays fully loaded, like gt[:]; with
-    lazy=True calldata/GT is a ZarrRows that decodes row ranges on demand)."""
-    return {
+    lazy=True calldata/GT is a ZarrRows that decodes row ranges on demand).  sites=True: variants/CHROM, REF and
+    ALT (its first column: allele index 1) too, as str arrays, when the store has them."""
+    out = {
         "calldata/GT": ZarrRows(path, "calldata/GT") if lazy else _zarr_array(path, "calldata/GT"),
         "samples": _zarr_array(path, "samples"),
         "variants/POS": _zarr_array(path, "variants/POS"),
     }
+    for name in ("variants/CHROM", "variants/REF", "variants/ALT") if sites else ():
+        if os.path.exists(os.path.join(path, name, ".zarray")):
+            out[name] = _zarr_strings(path, name)
+    return out
 
 
-def write_zarr(path, gt, samples, positions, chunk_variants=65536, compress=True):
-    """Minimal zarr v2 writer (the vcf_to_zarr equivalent of this build): zlib-compressed chunks."""
+def write_zarr(path, gt, samples, positions, chunk_variants=65536, compress=True, chrom=None, ref=None, alt=None):
+    """Minimal zarr v2 writer (the vcf_to_zarr equivalent of this build): zlib-compressed chunks.  chrom / ref /
+    alt: optional per-variant strings, written as variants/CHROM, REF and ALT."""
     os.makedirs(path, exist_ok=True)
     with open(os.path.join(path, ".zgroup"), "w") as fh:
         json.dump({"zarr_format": 2}, fh)
@@ -405,6 +453,11 @@ def write_zarr(path, gt, samples, positions, chunk_variants=65536, compress=True
     put("samples", s, (max(1, s.shape[0]),))
     p = np.asarray(positions, dtype=np.int64)
     put("variants/POS", p, (min(chunk_variants, max(1, p.shape[0])),))
+    for name, v in (("CHROM", chrom), ("REF", ref), ("ALT", alt)):
+        if v is not None:
+            v = np.broadcast_to(np.asarray(v, dtype=str), p.shape)
+            b = v.astype("S" + str(max(1, max((len(x.encode()) for x in v), default=1))))
+            put("variants/" + name, b, (min(chunk_variants, max(1, b.shape[0])),))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -430,6 +483,16 @@ def read_bim(path):
         return np.array([], dtype=str), np.array([], dtype=np.int64)
     t = pd.read_csv(path, sep=r"\s+", header=None, usecols=[0, 3], dtype={0: str, 3: np.int64})
     return t[0].to_numpy(dtype=str), t[3].to_numpy(dtype=np.int64)
+
+
+def read_bim_alleles(path):
+    """(A1, A2) per variant of a .bim file: columns 5 and 6."""
+    import pandas as pd
+
+    if os.path.getsize(path) == 0:
+        return np.array([], dtype=str), np.array([], dtype=str)
+    t = pd.read_csv(path, sep=r"\s+", header=None, usecols=[4, 5], dtype=str, keep_default_na=False)
+    return t[4].to_numpy(dtype=str), t[5].to_numpy(dtype=str)
 
 
 def check_bed(path, nvar, nsamp):
@@ -515,15 +578,18 @@ def decode_bed(records, nsamp):
     return BED_CODE_GT[codes.reshape(records.shape[0], -1)[:, :nsamp]]
 
 
-def read_bed(prefix):
+def read_bed(prefix, sites=False):
     """PLINK 1 fileset -> dict like read_zarr(lazy=True): 'calldata/GT' (a BedRows: no genotype byte is read
-    here), 'samples' (.fam IIDs), 'variants/POS' and 'variants/CHROM' (.bim).  The .bed header and size are
-    checked against the .bim / .fam."""
+    here), 'samples' (.fam IIDs), 'variants/POS' and 'variants/CHROM' (.bim); sites=True: 'variants/REF' = A2 and
+    'variants/ALT' = A1 too (allele indices 0 and 1).  The .bed header and size are checked against the .bim / .fam."""
     samples = read_fam(prefix + ".fam")
     chrom, pos = read_bim(prefix + ".bim")
     check_bed(prefix + ".bed", len(pos), len(samples))
-    return {"calldata/GT": BedRows(prefix, len(pos), len(samples)), "samples": samples, "variants/POS": pos,
-            "variants/CHROM": chrom}
+    out = {"calldata/GT": BedRows(prefix, len(pos), len(samples)), "samples": samples, "variants/POS": pos,
+           "variants/CHROM": chrom}
+    if sites:
+        out["variants/ALT"], out["variants/REF"] = read_bim_alleles(prefix + ".bim")
+    return out
 
 
 def write_bed(prefix, gt, samples, positions, chrom="1"):

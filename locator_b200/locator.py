@@ -23,6 +23,8 @@ Differences that are deliberate and documented in DESIGN.md:
     (the best-epoch checkpoint lives in device memory, not on disk);
   * ``--bed PREFIX`` (extension, not written to params.json): PLINK 1 .bed input, filtered and packed on the
     device straight from its 2-bit records (locator_b200.io.BedRows, loc_bed_* kernels);
+  * ``--keep_sites`` (extension, not written to params.json): next to every weights file, X.sites.tsv with the
+    model's sites and location normalisation (locator_b200.sites), which python -m locator_b200.predict reads;
   * ``--gpus N`` and ``--replicates_per_gpu G`` (extensions, not written to params.json): --bootstrap
     replicates (the FULL model included), --windows replicates and the folds of a k-fold holdout run
     (locator_b200.holdout) are work items of one queue at every GPU count, spread over N GPUs of the box,
@@ -120,6 +122,10 @@ def command_parser():
                         help="(locator_b200) PLINK 1 binary fileset PREFIX.bed / .bim / .fam (SNP-major) instead of --vcf / "
                         "--zarr / --matrix: A1 (.bim column 5) is the counted allele, the role ALT plays in a VCF; sample "
                         "IDs are the .fam IIDs, positions .bim column 4 (--windows: one chromosome). default: None")
+    parser.add_argument("--keep_sites", default=False, action="store_true",
+                        help="(locator_b200) with --keep_weights: next to every X.weights.npz write X.sites.tsv -- the "
+                        "model's sites (CHROM POS REF ALT, one row per first-layer weight row) and the location mean / sd "
+                        "-- so that python -m locator_b200.predict can locate samples of another file. default: False")
     return parser
 
 
@@ -140,6 +146,11 @@ def validate_args(ns):
         other = [f"--{k}" for k in ("vcf", "zarr", "matrix") if getattr(ns, k) is not None]
         if other:
             problems.append(f"--bed with {' / '.join(other)}: give one genotype input")
+    if getattr(ns, "keep_sites", False):
+        if not ns.keep_weights:
+            problems.append("--keep_sites without --keep_weights: the sites file describes a weights file")
+        if ns.matrix is not None:
+            problems.append("--keep_sites with --matrix: a matrix has no site identity (CHROM / POS / REF / ALT)")
     if not 1 <= int(ns.batch_size) <= 256:
         problems.append(f"--batch_size {ns.batch_size}: must be in [1, 256] (up to 32, the reference's default, a step runs "
                         "on the fused tensor-core kernels; 33..256 rows go through the stack in 32-row chunks)")
@@ -203,8 +214,9 @@ class AlleleCounts:
     """``ac``: derived-allele counts [K sites, N samples] (reference orientation), stored packed
     sample-major on the device."""
 
-    def __init__(self, packed):
+    def __init__(self, packed, sites=None):
         self.packed = packed  # PackedGenotypes [N, K]
+        self.sites = sites  # --keep_sites: site table of the K columns (locator_b200.sites)
 
     @property
     def shape(self):
@@ -235,15 +247,18 @@ def _matrix_shape(g):
 def load_genotypes():
     from . import io
 
+    keep_sites = bool(getattr(args, "keep_sites", False))
     if args.zarr is not None:
         print("reading zarr")
-        callset = io.read_zarr(args.zarr, lazy=True)  # calldata/GT is decoded on first use (row ranges for --windows)
-        genotypes = io.Genotypes(callset["calldata/GT"], callset["samples"], callset["variants/POS"])
+        # calldata/GT is decoded on first use (row ranges for --windows)
+        callset = io.read_zarr(args.zarr, lazy=True, sites=keep_sites)
+        genotypes = io.Genotypes(callset["calldata/GT"], callset["samples"], callset["variants/POS"],
+                                 io.variant_ids(callset))
         samples = callset["samples"]
     elif args.vcf is not None:
         print("reading VCF")
-        vcf = io.read_vcf(args.vcf)
-        genotypes = io.Genotypes(vcf["calldata/GT"], vcf["samples"], vcf["variants/POS"])
+        vcf = io.read_vcf(args.vcf, sites=keep_sites)
+        genotypes = io.Genotypes(vcf["calldata/GT"], vcf["samples"], vcf["variants/POS"], io.variant_ids(vcf))
         samples = vcf["samples"]
     elif args.matrix is not None:
         genotypes = io.read_matrix(args.matrix)
@@ -251,7 +266,8 @@ def load_genotypes():
     elif getattr(args, "bed", None) is not None:
         print("reading PLINK .bed")
         try:
-            callset = io.read_bed(args.bed)  # .bim / .fam parsed, .bed header and size checked; no genotype byte read
+            # .bim / .fam parsed, .bed header and size checked; no genotype byte read
+            callset = io.read_bed(args.bed, sites=keep_sites)
         except ValueError as e:
             raise SystemExit(f"locator: {e}")
         chroms = np.unique(callset["variants/CHROM"])
@@ -259,10 +275,14 @@ def load_genotypes():
             raise SystemExit(f"locator: --windows on {args.bed}.bim, which lists {len(chroms)} chromosomes "
                              f"({', '.join(chroms[:5])}{', ...' if len(chroms) > 5 else ''}): windows are positional and "
                              "run over a single chromosome")
-        genotypes = io.Genotypes(callset["calldata/GT"], callset["samples"], callset["variants/POS"])
+        genotypes = io.Genotypes(callset["calldata/GT"], callset["samples"], callset["variants/POS"],
+                                 io.variant_ids(callset))
         samples = callset["samples"]
     else:
         raise SystemExit("one of --vcf, --zarr, --matrix or --bed is required")
+    if keep_sites and genotypes.ids is None:
+        raise SystemExit(f"locator: --keep_sites: {args.zarr} has no variants/CHROM, variants/REF and variants/ALT "
+                         "arrays, so the sites of a model cannot be named")
     return genotypes, samples
 
 
@@ -323,6 +343,7 @@ def replace_md(genotypes, stats=None):
 
 def filter_snps(genotypes):
     from . import genotypes as G
+    from . import sites
     from .io import BedRows
 
     print("filtering SNPs")
@@ -345,9 +366,11 @@ def filter_snps(genotypes):
         ac = replace_md(genotypes, (g, alt_count, n_missing, keep_idx, packed))
     else:
         ac = AlleleCounts(packed)
+    if getattr(args, "keep_sites", False):
+        ac.sites = sites.table(genotypes.ids, genotypes.positions, keep_idx.cpu().numpy())
     if not args.max_SNPs == None:  # noqa: E711  (as in the reference)
         sel = np.random.choice(range(ac.shape[0]), args.max_SNPs, replace=False)
-        ac = AlleleCounts(ac.packed.take_cols(sel))
+        ac = AlleleCounts(ac.packed.take_cols(sel), None if ac.sites is None else sites.take(ac.sites, sel))
     print("running on " + str(len(ac)) + " genotypes after filtering\n\n\n")
     return ac
 
@@ -459,6 +482,14 @@ def train_network(model, traingen, testgen, trainlocs, testlocs, callbacks, boot
     return history, model
 
 
+def save_sites(weights_path, site_table, norm):
+    """--keep_sites: the sidecar of a weights file just written (locator_b200.sites)."""
+    if args.keep_weights and getattr(args, "keep_sites", False):
+        from . import sites
+
+        sites.write(sites.sidecar_path(weights_path), site_table, args.width, args.nlayers, norm)
+
+
 def predict_locs(model, predgen, sdlong, meanlong, sdlat, meanlat, testlocs, pred, samples, testgen, history, boot=0,
                  verbose=True):
     import pandas as pd
@@ -521,7 +552,7 @@ def plot_history(history, dists):
 # ---------------------------------------------------------------------------------------------
 # drivers
 # ---------------------------------------------------------------------------------------------
-def _run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, boot, cb_boot):
+def _run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, boot, cb_boot, sites=None):
     meanlong, sdlong, meanlat, sdlat = norm
     model = load_network(traingen, args.dropout_prop)
     callbacks = load_callbacks(cb_boot)
@@ -535,6 +566,7 @@ def _run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, sample
         history = History()
     else:
         history, model = train_network(model, traingen, testgen, trainlocs, testlocs, callbacks, boot)
+        save_sites(callbacks[0].filepath, sites, norm)
     dists = predict_locs(model, predgen, sdlong, meanlong, sdlat, meanlat, testlocs, pred, samples, testgen, history,
                          boot)
     if args.plot_history and history.history["loss"]:
@@ -579,7 +611,7 @@ def _jacknife_draws(af, K, n_pred):
     t.join()
 
 
-def start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights", "bed")):
+def start_run(ns, extensions=("gpus", "replicates_per_gpu", "load_weights", "bed", "keep_sites")):
     """Install ``ns`` as ``args`` and set the run up as the reference does: seed and gpu (locator.py:170-173),
     load stored parameters (:177-184), seed again in main() (:491-494) -- with --load_params it is the stored
     seed that decides the run's draws.  ``extensions``: flags of this build, kept from the command line (a
@@ -640,17 +672,17 @@ def _main_body():
             raise SystemExit("--windows requires --zarr or --bed input")
         replicates.run_windows(sys.modules[__name__], genotypes, samples)
     elif not args.bootstrap and not args.jacknife:
-        _run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, 0, None)
+        _run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, 0, None, ac.sites)
     elif args.bootstrap:
         from . import replicates
 
         replicates.run_bootstrap(sys.modules[__name__], traingen, testgen, trainlocs, testlocs, predgen, norm, pred,
-                                 samples)
+                                 samples, ac.sites)
     elif args.jacknife:
         boot = "FULL"
         start = time.time()
         model, history, dists = _run_one(traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, boot,
-                                         boot)
+                                         boot, ac.sites)
         print("run time " + str((time.time() - start) / 60) + " minutes")
         print("starting jacknife resampling")
         af = ac.site_sums() / (ac.shape[1] * 2)  # wide integer sums (numpy >= 2 would wrap uint8 in the reference)

@@ -17,6 +17,7 @@ import traceback
 
 import numpy as np
 
+from . import sites
 
 def _tick(what):
     """LOC_TIMING=1: wall-clock milestones of the replicate drivers on stderr (seconds since the epoch, so the
@@ -70,43 +71,47 @@ def _prepare(L, item, base):
         return {"traingen": base["traingen"].take_cols(order), "testgen": base["testgen"].take_cols(order),
                 "predgen": base["predgen"].take_cols(order), "trainlocs": base["trainlocs"],
                 "testlocs": base["testlocs"], "norm": base["norm"], "pred": base["pred"], "samples": base["samples"],
-                "boot": item["boot"], "cb_boot": item["boot"], "seed_tag": item["boot"] + 1, "out": args.out}
+                "boot": item["boot"], "cb_boot": item["boot"], "seed_tag": item["boot"] + 1, "out": args.out,
+                "sites": None if base.get("sites") is None else sites.take(base["sites"], order)}
     if item["kind"] == "full":
         # the un-resampled model of a bootstrap run (locator.py:611-632), as a work item of its own
         return {"traingen": base["traingen"], "testgen": base["testgen"], "predgen": base["predgen"],
                 "trainlocs": base["trainlocs"], "testlocs": base["testlocs"], "norm": base["norm"],
                 "pred": base["pred"], "samples": base["samples"], "boot": "FULL", "cb_boot": "FULL", "seed_tag": 0,
-                "out": args.out}
+                "out": args.out, "sites": base.get("sites")}
     if item["kind"] == "window_lazy":
         # the window's genotypes are still on disk: read its zarr chunks / .bed records, filter and gather here (on
         # this worker's GPU); the random split was drawn by the parent in the reference's order
         from . import io
 
         cache = _prepare.__dict__.setdefault("stores", {})  # zarr metadata / parsed .bim + .fam, once per process
+        keep_sites = bool(getattr(args, "keep_sites", False))
         if item.get("format") == "bed":
             prefix, a, b = item["where"]
-            if ("bed", prefix) not in cache:
-                cache[("bed", prefix)] = io.read_bed(prefix)
-            cs = cache[("bed", prefix)]
+            if ("bed", prefix, keep_sites) not in cache:
+                cache[("bed", prefix, keep_sites)] = io.read_bed(prefix, sites=keep_sites)
+            cs = cache[("bed", prefix, keep_sites)]
             rows = cs["calldata/GT"].rows(a, b)
         else:
             root, name, a, b = item["where"]
-            if root not in cache:
-                cache[root] = io.read_zarr(root, lazy=True)
-            cs = cache[root]
+            if (root, keep_sites) not in cache:
+                cache[(root, keep_sites)] = io.read_zarr(root, lazy=True, sites=keep_sites)
+            cs = cache[(root, keep_sites)]
             rows = io.ZarrRows(root, name, a, b)
-        sub = io.Genotypes(rows, cs["samples"], cs["variants/POS"][a:b])
+        ids = io.variant_ids(cs)
+        sub = io.Genotypes(rows, cs["samples"], cs["variants/POS"][a:b],
+                           None if ids is None else {k: v[a:b] for k, v in ids.items()})
         ac = L.filter_snps(sub)
         locs = item["locs"]
         train, test, traingen, testgen, trainlocs, testlocs, pred, predgen = L.split_train_test(ac, locs, item["drawn"])
         return {"traingen": traingen, "testgen": testgen, "predgen": predgen, "trainlocs": trainlocs,
                 "testlocs": testlocs, "norm": item["norm"], "pred": pred, "samples": item["samples"], "boot": 0,
-                "cb_boot": None, "seed_tag": item["index"] + 1, "out": item["window_out"]}
+                "cb_boot": None, "seed_tag": item["index"] + 1, "out": item["window_out"], "sites": ac.sites}
     if item["kind"] == "window":
         return {"traingen": item["traingen"], "testgen": item["testgen"], "predgen": item["predgen"],
                 "trainlocs": item["trainlocs"], "testlocs": item["testlocs"], "norm": item["norm"],
                 "pred": item["pred"], "samples": item["samples"], "boot": 0, "cb_boot": None,
-                "seed_tag": item["index"] + 1, "out": item["window_out"]}
+                "seed_tag": item["index"] + 1, "out": item["window_out"], "sites": item["sites"]}
     if item["kind"] == "fold":
         # k-fold holdout (locator_b200.holdout): row gathers of the filtered matrix; "pred" is the held-out fold
         g, locs, f = base["genotypes"], base["locs"], item["fold"]
@@ -114,7 +119,7 @@ def _prepare(L, item, base):
         return {"traingen": g.take_rows(item["train"]), "testgen": g.take_rows(item["val"]),
                 "predgen": g.take_rows(item["held"]), "trainlocs": locs[item["train"]], "testlocs": locs[item["val"]],
                 "norm": base["norm"], "pred": item["held"], "samples": base["samples"], "boot": f, "cb_boot": f,
-                "seed_tag": f + 1, "out": item["fold_out"], "fold": f}
+                "seed_tag": f + 1, "out": item["fold_out"], "fold": f, "sites": base.get("sites")}
     raise ValueError(item["kind"])
 
 
@@ -163,6 +168,8 @@ def _run_items(L, items, reps):
         for m, cb, rep in zip(models, callbacks, reps):
             h, _ = L.train_network(m, rep["traingen"], rep["testgen"], rep["trainlocs"], rep["testlocs"], cb, rep["boot"])
             histories.append(h)
+    for cb, rep in zip(callbacks, reps):
+        L.save_sites(cb[0].filepath, rep["sites"], rep["norm"])
     results = []
     for m, h, rep in zip(models, histories, reps):
         meanlong, sdlong, meanlat, sdlat = rep["norm"]
@@ -531,11 +538,12 @@ def run_work(L, items, base=None):
         pool.abort()
 
 
-def run_bootstrap(L, traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples):
+def run_bootstrap(L, traingen, testgen, trainlocs, testlocs, predgen, norm, pred, samples, site_table=None):
     """The un-resampled FULL model (locator.py:611-632) and every replicate, all work items.  Training draws nothing
-    from numpy's global stream, so every replicate's draws are taken first (full groups form at once)."""
+    from numpy's global stream, so every replicate's draws are taken first (full groups form at once).
+    ``site_table``: --keep_sites, the sites of the filtered matrix (replicate b gets them in its site order)."""
     base = {"traingen": traingen, "testgen": testgen, "predgen": predgen, "trainlocs": trainlocs,
-            "testlocs": testlocs, "norm": norm, "pred": pred, "samples": samples}
+            "testlocs": testlocs, "norm": norm, "pred": pred, "samples": samples, "sites": site_table}
     orders = draw_bootstrap_orders(traingen.K, L.args.nboots)
     boots = [{"kind": "boot", "boot": boot, "site_order": order} for boot, order in enumerate(orders)]
     run_work(L, [{"kind": "full", "boot": "FULL"}] + boots, base)
@@ -580,6 +588,6 @@ def run_windows(L, genotypes, samples):
             train, test, traingen, testgen, trainlocs, testlocs, pred, predgen = L.split_train_test(ac, locs)
             yield {"kind": "window", "index": index, "window_out": f"{args.out}_{i}-{i+size-1}", "traingen": traingen,
                    "testgen": testgen, "predgen": predgen, "trainlocs": trainlocs, "testlocs": testlocs,
-                   "norm": (meanlong, sdlong, meanlat, sdlat), "pred": pred, "samples": samples}
+                   "norm": (meanlong, sdlong, meanlat, sdlat), "pred": pred, "samples": samples, "sites": ac.sites}
 
     run_work(L, items())
